@@ -21,7 +21,7 @@ LIB = os.path.join(HERE, "libpgmuvi_b200.so")
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--threads", "1",
-    # compressed device code: the library shrinks from 178 MB to ~30 MB (41 translation units with
+    # compressed device code: the library shrinks from 178 MB to ~30 MB (39 translation units with
     # -lineinfo); the driver inflates it when the module is loaded
     "-Xfatbin=-compress-all", "--compress-mode=size",
 ]

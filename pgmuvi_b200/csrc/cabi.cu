@@ -160,12 +160,7 @@ int check_common(int B, int n_max, int d, int Q, int kernel_kind) {
 
 // number of packed raw parameters of a model (layout in include/pgmuvi_b200.h)
 int host_param_count(int d, int Q, int kernel_kind, int flags) {
-  const bool sep = kernel_kind >= PGM_KIND_SEP_RBF;
-  const int ds = sep ? 1 : d;
-  const int nl = (kernel_kind >= PGM_KIND_STAT_BASE)
-                     ? pgm::stat_num_time(kernel_kind) + pgm::sep_num_lam(pgm::stat_wave_atom(kernel_kind))
-                     : pgm::sep_num_lam(kernel_kind);
-  return 1 + Q + 2 * Q * ds + ((flags & PGM_FLAG_LEARN_NOISE) ? 1 : 0) + nl;
+  return pgm::param_layout(kernel_kind, d, Q, (flags & PGM_FLAG_LEARN_NOISE) != 0).P;
 }
 
 size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }

@@ -22,6 +22,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <math.h>
+#include "../../include/pgmuvi_b200.h"   // PGM_KIND_* / PGM_CON_* / PGM_FLAG_*
 
 namespace pgm {
 
@@ -34,30 +35,6 @@ constexpr int OPBUF = TS * KC;  // elements per operand per stage (XOR-swizzled,
 constexpr int LD_S = 68;        // smem ld of the 64x64 work tile (diagonal blocks)
 constexpr int STAGE_ELEMS = NSTAGES * 2 * OPBUF;   // 8192 doubles = 64 KB
 constexpr int S_ELEMS = TS * LD_S;                 // 4352
-
-#define PGM_KIND_SM1D 0
-#define PGM_KIND_SM_ARD_PRODSUM 1
-#define PGM_KIND_SM_ARD_SUMPROD 2
-// separable 2-D models (gps.py:1327-1336): SM(time, Q mixtures) x wavelength kernel
-#define PGM_KIND_SEP_RBF 3        // ScaleKernel(RBFKernel)           gps.py:1045-1048, 1063
-#define PGM_KIND_SEP_MATERN15 4   // ScaleKernel(MaternKernel(1.5))   gps.py:1049-1052
-#define PGM_KIND_SEP_RQ 5         // ScaleKernel(RQKernel)            gps.py:1053-1056
-#define PGM_KIND_SEP_CONST 6      // ConstantKernel (achromatic)      gps.py:1414-1415
-// stationary (non-spectral-mixture) time kernels, N3: kind = 8 + 5 * TK + WK,
-//   TK: 0 ScaleKernel(RBFKernel), 1 ScaleKernel(MaternKernel(1.5))      gps.py:985-990
-//       2 quasi-periodic ScaleKernel(PeriodicKernel * RBFKernel)         gps.py:915-935
-//       3 quasi-periodic + ScaleKernel(RBFKernel) (WK = 0 only)          gps.py:1187-1236
-//       4 / 5 ScaleKernel(MaternKernel(0.5 | 2.5)) (WK = 0 only)         gps.py:1166-1179
-//   WK: 0 none (1-D model), 1 RBF, 2 Matern-1.5, 3 RQ, 4 Constant       gps.py:1045-1072
-// K = os_t f_T(tau_t) [x os_w f_W(tau_lambda)]; no mixtures (Q = 0 in the packed layout).
-#define PGM_KIND_STAT_BASE 8
-#define PGM_KIND_STAT(tk, wk) (PGM_KIND_STAT_BASE + 5 * (tk) + (wk))
-#define PGM_FLAG_GRAD 1
-#define PGM_FLAG_LEARN_NOISE 2
-#define PGM_FLAG_BOUNDS_PER_LC 4
-// psd_safe_cholesky's ladder starts at 1e-6 for float32 models (GPyTorch cholesky_jitter) instead
-// of 1e-8: set by the *_f32 entry points
-#define PGM_FLAG_JITTER_F32 8
 
 // ------------------------------------------------------------------------------------
 // small PTX wrappers
@@ -248,16 +225,24 @@ __host__ __device__ constexpr int sep_num_lam(int sep_kind) {
   return (sep_kind == PGM_KIND_SEP_RBF || sep_kind == PGM_KIND_SEP_MATERN15) ? 2
          : (sep_kind == PGM_KIND_SEP_RQ) ? 3 : (sep_kind == PGM_KIND_SEP_CONST) ? 1 : 0;
 }
+// dims the spectral mixture acts on: d for the plain spectral-mixture kinds, else time only
+__host__ __device__ constexpr int mix_dims(int kind, int d) {
+  return kind >= PGM_KIND_SEP_RBF ? 1 : d;
+}
+// kernel parameters behind the mixture: wavelength kernel (outputscale, lengthscale[, alpha])
+// or (constant); stationary kinds: time kernel (outputscale, lengthscale) + wavelength kernel
+__host__ __device__ constexpr int num_lam(int kind) {
+  return kind >= PGM_KIND_STAT_BASE ? stat_num_time(kind) + sep_num_lam(stat_wave_atom(kind))
+                                    : sep_num_lam(kind);
+}
 
 template <int KIND, int QT, int D>
 struct Cfg {
   static constexpr bool STAT = KIND >= PGM_KIND_STAT_BASE;
   static constexpr bool SEP = KIND >= PGM_KIND_SEP_RBF && !STAT;
-  static constexpr int DS = (SEP || STAT) ? 1 : D;      // dims the spectral mixture acts on
-  // kernel parameters behind the mixture: wavelength kernel (outputscale, lengthscale[, alpha])
-  // or (constant); stationary kinds: time kernel (outputscale, lengthscale) + wavelength kernel
-  static constexpr int NLT = STAT ? stat_num_time(KIND) : 0;
-  static constexpr int NL = STAT ? NLT + sep_num_lam(stat_wave_atom(KIND)) : sep_num_lam(KIND);
+  static constexpr int DS = mix_dims(KIND, D);
+  static constexpr int NLT = STAT ? stat_num_time(KIND) : 0;   // time-kernel parameters of NL
+  static constexpr int NL = num_lam(KIND);
   static_assert(!STAT || QT == 4, "stationary kinds carry the time-kernel constants in w[4]");
   static constexpr int NCS = DS * QT;         // (cos, sin) pairs per point
   static constexpr int NFB = D + 2 * NCS;     // per-point doubles: x[D], (cos,sin)[DS][QT]
@@ -1111,10 +1096,50 @@ __device__ __forceinline__ void block_reduce(double (&v)[NVAL], double* red, dou
 }
 
 // packed raw-parameter layout:  [ mean | w[Q] | mu[Q*DS] | sigma[Q*DS] | (noise) | lam[NL] ]
-template <int KIND, int QT, int D>
-__host__ __device__ __forceinline__ int param_count(int Q, bool learn_noise) {
-  using C = Cfg<KIND, QT, D>;
-  return 1 + Q + 2 * Q * C::DS + (learn_noise ? 1 : 0) + C::NL;
+// (mean at slot 0, w at slot 1): the first slot of each later group and the slot count P
+struct ParamLayout {
+  int o_mu, o_sigma, o_noise, o_lam, P;
+};
+__host__ __device__ constexpr ParamLayout param_layout(int kind, int d, int Q, bool learn_noise) {
+  const int ds = mix_dims(kind, d), o_noise = 1 + Q + 2 * Q * ds;
+  const int o_lam = o_noise + (learn_noise ? 1 : 0);
+  return ParamLayout{1 + Q, 1 + Q + Q * ds, o_noise, o_lam, o_lam + num_lam(kind)};
+}
+
+// constraint of one slot (gpytorch.constraints): *th = theta(raw) and, if jc is given,
+// *jc = d theta / d raw
+__device__ __forceinline__ void constrain(int kd, double raw, double lb, double ub, double* th,
+                                          double* jc) {
+  double t = raw, j = 1.0;
+  if (kd == PGM_CON_SOFTPLUS) {
+    t = softplus_d(raw) + lb;
+    j = sigmoid_d(raw);
+  } else if (kd == PGM_CON_INTERVAL) {
+    const double s = sigmoid_d(raw);
+    t = lb + (ub - lb) * s;
+    j = (ub - lb) * s * (1.0 - s);
+  } else if (kd == PGM_CON_RSOFTPLUS) {
+    const double v = softplus_d(raw) + lb;
+    t = ub / v;
+    j = -ub * sigmoid_d(raw) / (v * v);
+  }
+  *th = t;
+  if (jc) *jc = j;
+}
+// threads 0..P-1: slot tid of light curve b's raw parameters -> theta[tid] (and jac[tid] unless
+// jac is null), with the bounds of the light curve under PGM_FLAG_BOUNDS_PER_LC
+template <class Args>
+__device__ __forceinline__ void load_theta(const Args& A, int b, int P, const double* raw,
+                                           double* theta, double* jac) {
+  const int tid = threadIdx.x;
+  if (tid < P) {
+    const size_t bo = (A.flags & PGM_FLAG_BOUNDS_PER_LC) ? (size_t)b * P : 0;
+    double th, jc;   // locals: passing theta + tid, jac + tid costs the dense builder registers
+    constrain(A.con_kind[tid], raw[tid], A.con_lb[bo + tid], A.con_ub[bo + tid], &th,
+              jac ? &jc : nullptr);
+    theta[tid] = th;
+    if (jac) jac[tid] = jc;
+  }
 }
 
 // constants of the wavelength kernel from its constrained parameters (lam_factor above)
@@ -1189,6 +1214,90 @@ __device__ __forceinline__ double lam_grad_factor(int t, const double* wq, const
   }
 }
 
+// kernel constants from theta: mixture weights wq[QT] and aq = 2 pi^2 sigma^2 [QT*DS] (zero for
+// the padded mixtures), constants behind the mixture lamq[4]; the stationary kinds fill all three
+// in stat_setup.  Threads 0..QT*DS-1 and 32 of the block write.
+template <int KIND, int QT, int D>
+__device__ __forceinline__ void kernel_constants(const double* theta, int Q, const ParamLayout& L,
+                                                 double* wq, double* aq, double* lamq) {
+  using C = Cfg<KIND, QT, D>;
+  constexpr int DS = C::DS;
+  const int tid = threadIdx.x;
+  if (!C::STAT && tid < QT) wq[tid] = (tid < Q) ? theta[1 + tid] : 0.0;
+  if (!C::STAT && tid < QT * DS) {
+    const int q = tid / DS, dd = tid - q * DS;
+    const double sg = (q < Q) ? theta[L.o_sigma + q * DS + dd] : 0.0;
+    aq[q * DS + dd] = 2.0 * M_PI * M_PI * sg * sg;
+  }
+  if (tid == 32) {
+    if constexpr (C::STAT) stat_setup<KIND>(theta + L.o_lam, wq, aq, lamq);
+    else lam_setup<KIND>(theta + L.o_lam, lamq);
+  }
+}
+
+// per-point fields of point i of the light curve's inputs x[n][D], centred on its first input:
+// x_i - x_0 into fx[dd * stride + i], (cos, sin)(2 pi mu_qd (x_id - x_0d)) into
+// fcs[2 * ((dd * QT + q) * stride + i)] (0 and (1, 0) for an invalid point or a padded mixture).
+// mu = theta + o_mu.
+template <int KIND, int QT, int D>
+__device__ __forceinline__ void point_fields(const double* x, int i, bool valid, const double* mu,
+                                             int Q, double* fx, double* fcs, int stride) {
+  constexpr int DS = Cfg<KIND, QT, D>::DS;
+#pragma unroll
+  for (int dd = 0; dd < D; ++dd) {
+    const double xc = valid ? (x[(size_t)i * D + dd] - x[dd]) : 0.0;
+    fx[(size_t)dd * stride + i] = xc;
+    if (dd < DS) {
+#pragma unroll
+      for (int q = 0; q < QT; ++q) {
+        double sn = 0.0, cs = 1.0;
+        if (valid && q < Q) sincospi(2.0 * mu[q * DS + dd] * xc, &sn, &cs);
+        *reinterpret_cast<double2*>(fcs + ((size_t)(dd * QT + q) * stride + i) * 2) =
+            make_double2(cs, sn);
+      }
+    }
+  }
+}
+
+// per-datum exact marginal log-likelihood -(y^T K~^-1 y + log |K~| + n log 2 pi) / (2 n)
+__device__ __forceinline__ double mll_value(double inv_quad, double logdet, int n) {
+  return -0.5 * (inv_quad + logdet + (double)n * 1.8378770664093454836) / n;
+}
+
+// d mll / d theta of slot tid from the block-reduced carriers: fin[0..NG) the kernel-gradient
+// accumulators, fin[NG] tr W, fin[NV] sum alpha.  The caller applies d theta / d raw.
+template <int KIND, int QT, int D>
+__device__ __forceinline__ double grad_slot(int tid, int n, const ParamLayout& L, const double* fin,
+                                            const double* theta, const double* wq,
+                                            const double* lamq) {
+  using C = Cfg<KIND, QT, D>;
+  constexpr int DS = C::DS;
+  const double half = 0.5 / (double)n;
+  if (tid == 0) return fin[C::NV] / (double)n;
+  if (tid < L.o_mu) return half * fin[tid - 1];
+  if (tid < L.o_sigma) {
+    const int t = tid - L.o_mu, q = t / DS, dd = t - q * DS;
+    return half * (-2.0 * M_PI * wq[q]) * fin[QT + q * DS + dd];
+  }
+  if (tid < L.o_noise) {
+    const int t = tid - L.o_sigma, q = t / DS, dd = t - q * DS;
+    return half * (-4.0 * M_PI * M_PI * theta[tid] * wq[q]) * fin[QT + QT * DS + q * DS + dd];
+  }
+  if (tid < L.o_lam) return half * fin[C::NG];   // learned noise: tr W
+  // parameters behind the mixture: constant factors of lam_factor's derivative carriers
+  const int t = tid - L.o_lam;
+  return half * lam_grad_factor<KIND>(t, wq, lamq) * fin[QT + 2 * QT * DS + t];
+}
+
+// diagonal jitter of Cholesky attempt 0..3: psd_safe_cholesky's ladder 0, 1e-8, 1e-7, 1e-6
+// (1e-6, 1e-5, 1e-4 under PGM_FLAG_JITTER_F32, GPyTorch's float32 cholesky_jitter)
+__device__ __forceinline__ double chol_jitter(int attempt, int flags) {
+  if (attempt <= 0) return 0.0;
+  double j = (flags & PGM_FLAG_JITTER_F32) ? 1e-6 : 1e-8;
+  for (int t = 1; t < attempt; ++t) j *= 10.0;
+  return j;
+}
+
 // ------------------------------------------------------------------------------------
 // pipeline state carried by a block across light curves (mbarrier phases keep running)
 // ------------------------------------------------------------------------------------
@@ -1234,9 +1343,8 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   const bool learn_noise = (A.flags & PGM_FLAG_LEARN_NOISE) != 0;
   const bool want_grad = (A.flags & PGM_FLAG_GRAD) != 0;
   constexpr int DS = C::DS;
-  const int P = param_count<KIND, QT, D>(Q, learn_noise);
-  const int o_noise = 1 + Q + 2 * Q * DS;             // learned-noise slot (if any)
-  const int o_lam = o_noise + (learn_noise ? 1 : 0);  // wavelength-kernel slots
+  const ParamLayout L = param_layout(KIND, D, Q, learn_noise);
+  const int P = L.P;
   const int n = A.n_valid ? A.n_valid[b] : A.n_max;
   const int N = (n + TS - 1) / TS;
   const int npad = N * TS;
@@ -1269,61 +1377,19 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   PGM_PROF_START();
   __syncthreads();
   // ---- constraints: raw -> theta, d theta / d raw  (A.2) -----------------------------
-  if (tid < P) {
-    const double rv = raw[tid];
-    const int kd = A.con_kind[tid];
-    const size_t bo = (A.flags & PGM_FLAG_BOUNDS_PER_LC) ? (size_t)b * P : 0;
-    const double lb = A.con_lb[bo + tid], ub = A.con_ub[bo + tid];
-    double th = rv, jc = 1.0;
-    if (kd == 1) {
-      th = softplus_d(rv) + lb;
-      jc = sigmoid_d(rv);
-    } else if (kd == 2) {
-      const double s = sigmoid_d(rv);
-      th = lb + (ub - lb) * s;
-      jc = (ub - lb) * s * (1.0 - s);
-    } else if (kd == 3) {   // PGM_CON_RSOFTPLUS: ub / (softplus(raw) + lb)
-      const double v = softplus_d(rv) + lb;
-      th = ub / v;
-      jc = -ub * sigmoid_d(rv) / (v * v);
-    }
-    theta[tid] = th;
-    jac[tid] = jc;
-  }
+  load_theta(A, b, P, raw, theta, jac);
   load_exp_tab(tab);
   __syncthreads();
-  if (!C::STAT && tid < QT) wq[tid] = (tid < Q) ? theta[1 + tid] : 0.0;
-  if (!C::STAT && tid < QT * DS) {
-    const int q = tid / DS, dd = tid - q * DS;
-    const double sg = (q < Q) ? theta[1 + Q + Q * DS + q * DS + dd] : 0.0;
-    aq[q * DS + dd] = 2.0 * M_PI * M_PI * sg * sg;
-  }
-  if (tid == 32) {
-    if constexpr (C::STAT) stat_setup<KIND>(theta + o_lam, wq, aq, lamq);
-    else lam_setup<KIND>(theta + o_lam, lamq);
-  }
+  kernel_constants<KIND, QT, D>(theta, Q, L, wq, aq, lamq);
   const double mean = theta[0];
-  const double lnoise = learn_noise ? theta[o_noise] : 0.0;
+  const double lnoise = learn_noise ? theta[L.o_noise] : 0.0;
   // ---- per-point fields into the block's scratch ------------------------------------
   const double* xb = A.x + (size_t)b * A.n_max * D;
   const double* yb = A.y + (size_t)b * A.n_max;
   const double* fnb = A.fixed_noise ? A.fixed_noise + (size_t)b * A.n_max : nullptr;
   for (int i = tid; i < npad; i += NTHREADS) {
     const bool valid = i < n;
-#pragma unroll
-    for (int dd = 0; dd < D; ++dd) {
-      const double xc = valid ? (xb[(size_t)i * D + dd] - xb[dd]) : 0.0;
-      sc.fx[(size_t)dd * npad + i] = xc;
-      if (dd < DS) {
-#pragma unroll
-        for (int q = 0; q < QT; ++q) {
-          double sn = 0.0, cs = 1.0;
-          if (valid && q < Q) sincospi(2.0 * theta[1 + Q + q * DS + dd] * xc, &sn, &cs);
-          *reinterpret_cast<double2*>(sc.fcs + ((size_t)(dd * QT + q) * npad + i) * 2) =
-              make_double2(cs, sn);
-        }
-      }
-    }
+    point_fields<KIND, QT, D>(xb, i, valid, theta + L.o_mu, Q, sc.fx, sc.fcs, npad);
     sc.rhs[i] = valid ? (yb[i] - mean) : 0.0;
     sc.dn[i] = valid ? ((fnb ? fnb[i] : 0.0) + lnoise) : 0.0;
   }
@@ -1377,11 +1443,7 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
 
   // ================= phase P: Cholesky + forward solve, with the jitter ladder ========
   for (int attempt = 0; attempt <= 3; ++attempt) {
-    double jitter = 0.0;
-    if (attempt > 0) {
-      jitter = (A.flags & PGM_FLAG_JITTER_F32) ? 1e-6 : 1e-8;
-      for (int t = 1; t < attempt; ++t) jitter *= 10.0;
-    }
+    const double jitter = chol_jitter(attempt, A.flags);
     if (tid == 0) *s_fail = 0;
     iq_part = 0.0;
     ld_part = 0.0;
@@ -1544,11 +1606,7 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
     double v2[2] = {iq_part, ld_part};
     block_reduce<2>(v2, red, fin);
   }
-  const double inv_quad = fin[0];
-  const double logdet = 2.0 * fin[1];
-  const double mll = (info >= 0)
-                         ? -0.5 * (inv_quad + logdet + (double)n * 1.8378770664093454836) / n
-                         : nan("");
+  const double mll = (info >= 0) ? mll_value(fin[0], 2.0 * fin[1], n) : nan("");
   __syncthreads();
   PGM_PROF(6);
   if (tid == 0) *mll_out = mll;
@@ -1705,28 +1763,7 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
     __syncthreads();
     block_reduce<C::NV + 1>(v, red, fin);
   }
-  if (tid < P) {
-    const double half = 0.5 / (double)n;
-    double gv;
-    if (tid == 0) {
-      gv = fin[C::NV] / (double)n;
-    } else if (tid < 1 + Q) {
-      gv = half * fin[tid - 1];
-    } else if (tid < 1 + Q + Q * DS) {
-      const int t = tid - 1 - Q, q = t / DS, dd = t - q * DS;
-      gv = half * (-2.0 * M_PI * wq[q]) * fin[QT + q * DS + dd];
-    } else if (tid < o_noise) {
-      const int t = tid - 1 - Q - Q * DS, q = t / DS, dd = t - q * DS;
-      gv = half * (-4.0 * M_PI * M_PI * theta[tid] * wq[q]) * fin[QT + QT * DS + q * DS + dd];
-    } else if (tid < o_lam) {
-      gv = half * fin[C::NG];   // learned noise: tr W
-    } else {
-      // parameters behind the mixture: constant factors of lam_factor's derivative carriers
-      const int t = tid - o_lam;
-      gv = half * lam_grad_factor<KIND>(t, wq, lamq) * fin[QT + 2 * QT * DS + t];
-    }
-    grad_out[tid] = gv * jac[tid];
-  }
+  if (tid < P) grad_out[tid] = grad_slot<KIND, QT, D>(tid, n, L, fin, theta, wq, lamq) * jac[tid];
   __syncthreads();
   PGM_PROF(12);
   return info;
@@ -1760,7 +1797,7 @@ __global__ void __launch_bounds__(NTHREADS, (Cfg<KIND, QT, D>::F_BYTES <= 113 * 
     sm_mll_grad_kernel(EvalArgs A) {
   extern __shared__ __align__(16) double sm[];
   Scratch sc = make_scratch<KIND, QT, D>(A.ws + (size_t)blockIdx.x * A.ws_per_block, A.n_max);
-  const int P = param_count<KIND, QT, D>(A.Q, (A.flags & PGM_FLAG_LEARN_NOISE) != 0);
+  const int P = param_layout(KIND, D, A.Q, (A.flags & PGM_FLAG_LEARN_NOISE) != 0).P;
   PipeState ps;
   pipe_init_at<KIND, QT, D>(sm + Cfg<KIND, QT, D>::F_PAR, ps);
   // broadcast slot of the scheduler: in the spare words behind s_fail (static shared memory would
@@ -1814,33 +1851,14 @@ __global__ void __launch_bounds__(NTHREADS)
   tri_unrank(blockIdx.x, ti, tj);
   const int Q = A.Q;
   const bool learn_noise = (A.flags & PGM_FLAG_LEARN_NOISE) != 0;
-  const int P = param_count<KIND, QT, D>(Q, learn_noise);
-  const int o_noise = 1 + Q + 2 * Q * DS, o_lam = o_noise + (learn_noise ? 1 : 0);
+  const ParamLayout L = param_layout(KIND, D, Q, learn_noise);
+  const int P = L.P;
   const int n = A.n_valid ? A.n_valid[b] : A.n_max;
   if (ti * TS >= n) return;
-  if (tid < P) {
-    const double rv = A.raw[(size_t)b * P + tid];
-    const int kd = A.con_kind[tid];
-    const size_t bo = (A.flags & PGM_FLAG_BOUNDS_PER_LC) ? (size_t)b * P : 0;
-    const double lb = A.con_lb[bo + tid], ub = A.con_ub[bo + tid];
-    double th = rv;
-    if (kd == 1) th = softplus_d(rv) + lb;
-    else if (kd == 2) th = lb + (ub - lb) * sigmoid_d(rv);
-    else if (kd == 3) th = ub / (softplus_d(rv) + lb);
-    theta[tid] = th;
-  }
+  load_theta(A, b, P, A.raw + (size_t)b * P, theta, nullptr);
   load_exp_tab(tab);
   __syncthreads();
-  if (!C::STAT && tid < QT) wq[tid] = (tid < Q) ? theta[1 + tid] : 0.0;
-  if (!C::STAT && tid < QT * DS) {
-    const int q = tid / DS, dd = tid - q * DS;
-    const double sg = (q < Q) ? theta[1 + Q + Q * DS + q * DS + dd] : 0.0;
-    aq[q * DS + dd] = 2.0 * M_PI * M_PI * sg * sg;
-  }
-  if (tid == 32) {
-    if constexpr (C::STAT) stat_setup<KIND>(theta + o_lam, wq, aq, lamq);
-    else lam_setup<KIND>(theta + o_lam, lamq);
-  }
+  kernel_constants<KIND, QT, D>(theta, Q, L, wq, aq, lamq);
   // fields: item 0 of a point = its centred inputs, items 1.. = (cos, sin)(2 pi mu_qd x_d)
   const double* xb = A.x + (size_t)b * A.n_max * D;
   constexpr int ITEMS = 1 + DS * QT;
@@ -1857,13 +1875,13 @@ __global__ void __launch_bounds__(NTHREADS)
       const int f = item - 1, dd = f / QT, q = f - dd * QT;
       double sn = 0.0, cs = 1.0;
       if (valid && q < Q)
-        sincospi(2.0 * theta[1 + Q + q * DS + dd] * (xb[(size_t)gi * D + dd] - xb[dd]), &sn, &cs);
+        sincospi(2.0 * theta[L.o_mu + q * DS + dd] * (xb[(size_t)gi * D + dd] - xb[dd]), &sn, &cs);
       vec[D * TS + (f * TS + r) * 2] = cs;
       vec[D * TS + (f * TS + r) * 2 + 1] = sn;
     }
   }
   __syncthreads();
-  const double lnoise = learn_noise ? theta[o_noise] : 0.0;
+  const double lnoise = learn_noise ? theta[L.o_noise] : 0.0;
   const double* fnb = A.fixed_noise ? A.fixed_noise + (size_t)b * A.n_max : nullptr;
   double* Kb = Kout + (size_t)b * A.n_max * A.n_max;
   double wreg[QT], areg[QT * DS], lam[4];
@@ -1921,7 +1939,7 @@ __global__ void __launch_bounds__(NTHREADS, (Cfg<KIND, QT, D>::F_BYTES <= 113 * 
   extern __shared__ __align__(16) double sm[];
   const EvalArgs& A = F.e;
   Scratch sc = make_scratch<KIND, QT, D>(A.ws + (size_t)blockIdx.x * A.ws_per_block, A.n_max);
-  const int P = param_count<KIND, QT, D>(A.Q, (A.flags & PGM_FLAG_LEARN_NOISE) != 0);
+  const int P = param_layout(KIND, D, A.Q, (A.flags & PGM_FLAG_LEARN_NOISE) != 0).P;
   double* par = sm + C::F_PAR;
   double* s_raw = par + C::PAR_RAW;
   double* s_m = s_raw + C::PMAX;

@@ -123,12 +123,6 @@ __device__ __forceinline__ LcView lc_view(const LargeArgs& A, int b = -1) {
   v.st = make_batch_state(A.ws, A.n_max, A.B);
   return v;
 }
-__device__ __forceinline__ double lg_jitter(int attempt, int flags) {
-  if (attempt <= 0) return 0.0;
-  double j = (flags & PGM_FLAG_JITTER_F32) ? 1e-6 : 1e-8;
-  for (int t = 1; t < attempt; ++t) j *= 10.0;
-  return j;
-}
 
 __device__ __forceinline__ double* lg_tile(double* base, int i, int j) {
   return base + ((size_t)i * (i + 1) / 2 + j) * TT;
@@ -141,8 +135,6 @@ __device__ __forceinline__ double* lg_tile(double* base, int i, int j) {
 // ------------------------------------------------------------------------------------
 template <int KIND, int QT, int D>
 __global__ void __launch_bounds__(NTHREADS) lg_setup(LargeArgs A) {
-  using C = Cfg<KIND, QT, D>;
-  constexpr int DS = C::DS;
   __shared__ double theta[64], jac[64];
   const int tid = threadIdx.x;
   const LcView v = lc_view(A);
@@ -150,71 +142,29 @@ __global__ void __launch_bounds__(NTHREADS) lg_setup(LargeArgs A) {
   const LargeWs& w = v.w;
   const int Q = A.Q;
   const bool learn_noise = (A.flags & PGM_FLAG_LEARN_NOISE) != 0;
-  const int P = param_count<KIND, QT, D>(Q, learn_noise);
-  const int o_noise = 1 + Q + 2 * Q * DS, o_lam = o_noise + (learn_noise ? 1 : 0);
+  const ParamLayout L = param_layout(KIND, D, Q, learn_noise);
+  const int P = L.P;
   const int n = v.n, npad = v.npad;
   if (blockIdx.x * NTHREADS >= npad) return;
-  if (tid < P) {
-    const double rv = A.raw[(size_t)v.b * P + tid];
-    const int kd = A.con_kind[tid];
-    const size_t bo = (A.flags & PGM_FLAG_BOUNDS_PER_LC) ? (size_t)v.b * P : 0;
-    const double lb = A.con_lb[bo + tid], ub = A.con_ub[bo + tid];
-    double th = rv, jc = 1.0;
-    if (kd == 1) {
-      th = softplus_d(rv) + lb;
-      jc = sigmoid_d(rv);
-    } else if (kd == 2) {
-      const double s = sigmoid_d(rv);
-      th = lb + (ub - lb) * s;
-      jc = (ub - lb) * s * (1.0 - s);
-    } else if (kd == 3) {   // PGM_CON_RSOFTPLUS: ub / (softplus(raw) + lb)
-      const double v = softplus_d(rv) + lb;
-      th = ub / v;
-      jc = -ub * sigmoid_d(rv) / (v * v);
-    }
-    theta[tid] = th;
-    jac[tid] = jc;
-  }
+  load_theta(A, v.b, P, A.raw + (size_t)v.b * P, theta, jac);
   __syncthreads();
   if (blockIdx.x == 0) {
     if (tid < P) {
       w.par[LG_PAR_TH + tid] = theta[tid];
       w.par[LG_PAR_JC + tid] = jac[tid];
     }
-    if (!C::STAT && tid < QT) w.par[LG_PAR_WQ + tid] = (tid < Q) ? theta[1 + tid] : 0.0;
-    if (!C::STAT && tid < QT * DS) {
-      const int q = tid / DS, dd = tid - q * DS;
-      const double sg = (q < Q) ? theta[1 + Q + Q * DS + q * DS + dd] : 0.0;
-      w.par[LG_PAR_AQ + q * DS + dd] = 2.0 * M_PI * M_PI * sg * sg;
-    }
-    if (tid == 32) {
-      if constexpr (C::STAT)
-        stat_setup<KIND>(theta + o_lam, w.par + LG_PAR_WQ, w.par + LG_PAR_AQ, w.par + LG_PAR_LM);
-      else lam_setup<KIND>(theta + o_lam, w.par + LG_PAR_LM);
-    }
+    kernel_constants<KIND, QT, D>(theta, Q, L, w.par + LG_PAR_WQ, w.par + LG_PAR_AQ,
+                                  w.par + LG_PAR_LM);
   }
   const double mean = theta[0];
-  const double lnoise = learn_noise ? theta[o_noise] : 0.0;
+  const double lnoise = learn_noise ? theta[L.o_noise] : 0.0;
   const int i = blockIdx.x * NTHREADS + tid;
   if (i >= npad) return;
   const bool valid = i < n;
   const double* xb = A.x + (size_t)v.b * A.n_max * D;
   const double* yb = A.y + (size_t)v.b * A.n_max;
   const double* fnb = A.fixed_noise ? A.fixed_noise + (size_t)v.b * A.n_max : nullptr;
-#pragma unroll
-  for (int dd = 0; dd < D; ++dd) {
-    const double xc = valid ? (xb[(size_t)i * D + dd] - xb[dd]) : 0.0;
-    w.fx[(size_t)dd * npad + i] = xc;
-    if (dd < DS) {
-#pragma unroll
-      for (int q = 0; q < QT; ++q) {
-        double sn = 0.0, cs = 1.0;
-        if (valid && q < Q) sincospi(2.0 * theta[1 + Q + q * DS + dd] * xc, &sn, &cs);
-        *reinterpret_cast<double2*>(w.fcs + ((size_t)(dd * QT + q) * npad + i) * 2) =
-            make_double2(cs, sn);
-      }
-    }
-  }
+  point_fields<KIND, QT, D>(xb, i, valid, theta + L.o_mu, Q, w.fx, w.fcs, npad);
   w.rhs[i] = valid ? (yb[i] - mean) : 0.0;
   w.dn[i] = valid ? ((fnb ? fnb[i] : 0.0) + lnoise) : 0.0;
 }
@@ -347,7 +297,7 @@ __global__ void __launch_bounds__(NTHREADS, UpdSmem<KIND, QT, D>::MIN_BLOCKS)
   }
   if (i >= N || j >= N) return;
   if (v.st.fail[v.b]) return;
-  const double jitter = lg_jitter(v.st.attempt[v.b], A.flags);
+  const double jitter = chol_jitter(v.st.attempt[v.b], A.flags);
   double* stages = sm;
   double* Cst = stages + 2 * OPBUF;
   double* Ct = sm + L::CT_OFF;            // !build: the block's own C tile
@@ -631,7 +581,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
   int* flags = v.st.tflag + (size_t)v.b * large_ntri(A.n_max);
   auto flag_of = [&](int a, int b2) { return flags + ((size_t)a * (a + 1) / 2 + b2); };
   volatile int* failp = v.st.fail + v.b;
-  const double jitter = lg_jitter(v.st.attempt[v.b], A.flags);
+  const double jitter = chol_jitter(v.st.attempt[v.b], A.flags);
   double* stages = sm;
   double* S2 = stages;                  // diagonal job: X = L^-1 (the stages are idle then)
   double* Cst = stages + 2 * OPBUF;
@@ -1165,16 +1115,13 @@ __global__ void __launch_bounds__(NTHREADS, GradSmem<KIND, QT, D>::MIN_BLOCKS)
 template <int KIND, int QT, int D>
 __global__ void __launch_bounds__(NTHREADS) lg_finish(LargeArgs A, int want_grad) {
   using C = Cfg<KIND, QT, D>;
-  constexpr int DS = C::DS;
   __shared__ double red[8 * (C::NV + 4)], fin[C::NV + 4];
   const int tid = threadIdx.x;
   const LcView v = lc_view(A);
   const LargeWs& w = v.w;
   const int n = v.n, N = v.N;
-  const int Q = A.Q;
-  const bool learn_noise = (A.flags & PGM_FLAG_LEARN_NOISE) != 0;
-  const int P = param_count<KIND, QT, D>(Q, learn_noise);
-  const int o_noise = 1 + Q + 2 * Q * DS, o_lam = o_noise + (learn_noise ? 1 : 0);
+  const ParamLayout L = param_layout(KIND, D, A.Q, (A.flags & PGM_FLAG_LEARN_NOISE) != 0);
+  const int P = L.P;
   double* mll_out = A.mll + v.b;
   double* grad_out = A.grad ? A.grad + (size_t)v.b * P : nullptr;
   if (v.st.state[v.b] != LG_FACTORED) {
@@ -1190,8 +1137,8 @@ __global__ void __launch_bounds__(NTHREADS) lg_finish(LargeArgs A, int want_grad
     vv[C::NV + 2] += w.ldz[2 * jb + 1];
   }
   if (want_grad) {
-    // per-tile partials: 64x64 tiles (lg_grad) or 128x128 tiles (lg_grad_tc, PGM_FLAG_TF32X3 = 16)
-    const int NTg = (A.flags & 16) ? (N + 1) / 2 : N;
+    // per-tile partials: 64x64 tiles (lg_grad) or 128x128 tiles (lg_grad_tc, PGM_FLAG_TF32X3)
+    const int NTg = (A.flags & PGM_FLAG_TF32X3) ? (N + 1) / 2 : N;
     const int njobs = NTg * (NTg + 1) / 2;
     for (int t = tid; t < njobs; t += NTHREADS)
 #pragma unroll
@@ -1202,33 +1149,11 @@ __global__ void __launch_bounds__(NTHREADS) lg_finish(LargeArgs A, int want_grad
         A.alpha_out[(size_t)v.b * A.n_max + i2] = (i2 < n) ? w.alpha[i2] : 0.0;
   }
   block_reduce<C::NV + 3>(vv, red, fin);
-  if (tid == 0) {
-    const double logdet = 2.0 * fin[C::NV + 1], inv_quad = fin[C::NV + 2];
-    *mll_out = -0.5 * (inv_quad + logdet + (double)n * 1.8378770664093454836) / n;
-  }
+  if (tid == 0) *mll_out = mll_value(fin[C::NV + 2], 2.0 * fin[C::NV + 1], n);
   if (!want_grad || tid >= P) return;
-  const double* theta = w.par + LG_PAR_TH;
-  const double* wq = w.par + LG_PAR_WQ;
-  const double* lamq = w.par + LG_PAR_LM;
-  const double half = 0.5 / (double)n;
-  double gv;
-  if (tid == 0) {
-    gv = fin[C::NV] / (double)n;
-  } else if (tid < 1 + Q) {
-    gv = half * fin[tid - 1];
-  } else if (tid < 1 + Q + Q * DS) {
-    const int t = tid - 1 - Q, q = t / DS, dd = t - q * DS;
-    gv = half * (-2.0 * M_PI * wq[q]) * fin[QT + q * DS + dd];
-  } else if (tid < o_noise) {
-    const int t = tid - 1 - Q - Q * DS, q = t / DS, dd = t - q * DS;
-    gv = half * (-4.0 * M_PI * M_PI * theta[tid] * wq[q]) * fin[QT + QT * DS + q * DS + dd];
-  } else if (tid < o_lam) {
-    gv = half * fin[C::NG];
-  } else {
-    const int t = tid - o_lam;
-    gv = half * lam_grad_factor<KIND>(t, wq, lamq) * fin[QT + 2 * QT * DS + t];
-  }
-  grad_out[tid] = gv * w.par[LG_PAR_JC + tid];
+  grad_out[tid] = grad_slot<KIND, QT, D>(tid, n, L, fin, w.par + LG_PAR_TH, w.par + LG_PAR_WQ,
+                                         w.par + LG_PAR_LM) *
+                  w.par[LG_PAR_JC + tid];
 }
 
 // ------------------------------------------------------------------------------------
@@ -1312,7 +1237,9 @@ __global__ void __launch_bounds__(NTHREADS, (Cfg<KIND, QT, D>::SMEM_BYTES <= 113
 #pragma unroll
     for (int q = 0; q < 4; ++q) lam[q] = w.par[LG_PAR_LM + q];
     const double* theta = w.par + LG_PAR_TH;
-    // ---- test tile fields (centred on the light curve's first training input, as lg_setup)
+    // ---- test tile fields (centred on the light curve's first training input, as lg_setup).
+    // Written out rather than through point_fields / param_layout: with nvcc 12.9 either form
+    // raises the registers of lg_predict<1,1,2> from 104 to 107 and of <1,8,2> from 244 to 250.
     const double* xb = A.x + (size_t)b * A.n_max * D;
     const double* xs = PA.xstar + ((size_t)b * PA.m + (size_t)t * TS) * D;
     if (tid < TS) {

@@ -39,10 +39,6 @@
 
 namespace pgm {
 
-#define PGM_FLAG_TF32X3 16   // G phase on tcgen05 (3xTF32); set by pgm_sm_mll_grad_tf32x3_f32
-#define PGM_FLAG_TF32X3_CHOL 32   /* ... and the trailing updates of the panel-schedule Cholesky */
-#define PGM_FLAG_NOSYNC 64        /* staged engine: no host synchronisation (one-launch schedule only) */
-
 constexpr int TC_THREADS = 320;        // producer warp + MMA warp + 8 epilogue warps
 constexpr int TC_EPI_THREADS = 256;
 
@@ -471,7 +467,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
   const float* phi = tc_pack_base(A.ws, A.n_max, A.B, v.b);
   const float* plo = phi + (size_t)NTmax * KCH * tc::IMG_FLOATS;
   const int nchunks = 2 * (J1 - J0);
-  const double jitter = lg_jitter(v.st.attempt[v.b], A.flags);
+  const double jitter = chol_jitter(v.st.attempt[v.b], A.flags);
 
   const unsigned base = (smem_u32(smraw) + 1023u) & ~1023u;
   unsigned char* gen = smraw + (base - smem_u32(smraw));
