@@ -57,6 +57,29 @@ CASES = [
     ("stat_qp_plus_rbf_1d_n130", dict(dim=1, kind=23, B=2, n=130, Q=0, learn_noise=False)),  # 1DPeriodicStochastic
     ("stat_matern12_1d_n110_learn", dict(dim=1, kind=28, B=2, n=110, Q=0, learn_noise=True)),
     ("stat_matern25_1d_n140", dict(dim=1, kind=33, B=2, n=140, Q=0, learn_noise=False)),
+    # ARD 2-D with one mixture (QT = 1) and sum-of-products with two (QT = 2)
+    ("sm2d_prodsum_4x48_q1", dict(dim=2, kind=1, B=2, bands=4, per=48, Q=1, learn_noise=False)),
+    ("sm2d_sumprod_4x48_q1", dict(dim=2, kind=2, B=2, bands=4, per=48, Q=1, learn_noise=False)),
+    ("sm2d_sumprod_4x48_q2_learn", dict(dim=2, kind=2, B=2, bands=4, per=48, Q=2, learn_noise=True)),
+    # ARD 2-D with QT = 8: one block per SM, full shared-memory layout; ragged down to n = 1
+    ("sm2d_prodsum_3x64_q8", dict(dim=2, kind=1, B=2, bands=3, per=64, Q=8, learn_noise=False)),
+    ("sm2d_sumprod_3x64_q6_learn", dict(dim=2, kind=2, B=3, bands=3, per=64, Q=6, learn_noise=True,
+                                        n_valid=[192, 65, 1])),
+    # padded mixtures inside QT = 8 (Q = 5 is the flicker term packed behind num_mixtures = 4)
+    ("sm1d_n130_q5_learn", dict(dim=1, B=2, n=130, Q=5, learn_noise=True)),
+    ("sep_rbf_3x40_q6_learn", dict(dim=2, kind=3, B=2, bands=3, per=40, Q=6, learn_noise=True)),
+    ("sep_matern_4x48_q5", dict(dim=2, kind=4, B=2, bands=4, per=48, Q=5, learn_noise=False)),
+    ("sep_rq_3x50_q8_learn", dict(dim=2, kind=5, B=2, bands=3, per=50, Q=8, learn_noise=True)),
+    ("sep_rq_3x50_q7", dict(dim=2, kind=5, B=1, bands=3, per=50, Q=7, learn_noise=False)),
+    ("sep_const_3x50_q7", dict(dim=2, kind=6, B=2, bands=3, per=50, Q=7, learn_noise=False)),
+    # stationary time kernel x wavelength kernel: RBF x {RBF, Matern-1.5, Constant},
+    # Matern-1.5 x RQ, quasi-periodic x {Matern-1.5, RQ}
+    ("stat_rbf_rbf_3x40_learn", dict(dim=2, kind=9, B=2, bands=3, per=40, Q=0, learn_noise=True)),
+    ("stat_rbf_matern_4x32", dict(dim=2, kind=10, B=2, bands=4, per=32, Q=0, learn_noise=False)),
+    ("stat_rbf_const_3x48_learn", dict(dim=2, kind=12, B=2, bands=3, per=48, Q=0, learn_noise=True)),
+    ("stat_matern_rq_4x40", dict(dim=2, kind=16, B=2, bands=4, per=40, Q=0, learn_noise=False)),
+    ("stat_qp_matern_3x40_learn", dict(dim=2, kind=20, B=2, bands=3, per=40, Q=0, learn_noise=True)),
+    ("stat_qp_rq_4x32", dict(dim=2, kind=21, B=2, bands=4, per=32, Q=0, learn_noise=False)),
 ]
 
 

@@ -1,5 +1,7 @@
-"""Generate tests/golden_predict/*.npz: posterior predictions of the oracle (N1) for a few of the
-golden cases (``python -m oracle.make_golden_predict``).  TEST INFRASTRUCTURE."""
+"""Generate posterior predictions of the oracle (N1) for a few of the golden cases
+(``python -m oracle.make_golden_predict [name ...]``; names regenerate a subset, as for
+``oracle.make_golden``): name.npz in tests/golden_predict/ for the first six cases, in
+tests/golden/predict/ for the later ones.  TEST INFRASTRUCTURE."""
 from __future__ import annotations
 
 import os
@@ -11,16 +13,24 @@ from .sm_gp import ModelSpec, predict
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "..", "tests", "golden")
-OUT = os.path.join(HERE, "..", "tests", "golden_predict")
-CASES = ["sm1d_n100_q2_learn", "sm1d_n200_q4", "sm1d_ragged_q4", "sm2d_prodsum_4x48_q4",
-         "sep_rq_4x48_q4", "sep_const_3x40_q3_learn"]
+OUT = os.path.join(GOLD, "predict")
+OUT_FIRST = os.path.join(HERE, "..", "tests", "golden_predict")
+CASES_FIRST = ["sm1d_n100_q2_learn", "sm1d_n200_q4", "sm1d_ragged_q4", "sm2d_prodsum_4x48_q4",
+               "sep_rq_4x48_q4", "sep_const_3x40_q3_learn"]
+CASES = CASES_FIRST + ["sm2d_prodsum_3x64_q8", "sep_matern_4x48_q5", "sm1d_n130_q5_learn",
+                       "stat_qp_rq_4x32"]
 M = 150   # test points per light curve (not a multiple of 64: ragged last test tile)
 
 
 def main():
+    import sys
     torch.set_default_dtype(torch.float64)
     os.makedirs(OUT, exist_ok=True)
+    os.makedirs(OUT_FIRST, exist_ok=True)
+    only = sys.argv[1:]          # optional name prefixes: regenerate a subset
     for name in CASES:
+        if only and not any(name.startswith(o) for o in only):
+            continue
         g = np.load(os.path.join(GOLD, name + ".npz"))
         B, n, d = g["x"].shape
         spec = ModelSpec(d=int(g["d"]), Q=int(g["Q"]), kind=int(g["kind"]),
@@ -44,7 +54,8 @@ def main():
                                    torch.tensor(lb), torch.tensor(ub), spec, torch.tensor(xs[b]))
             assert int(info) == 0
             mean[b], var[b] = mu.numpy(), vv.numpy()
-        np.savez_compressed(os.path.join(OUT, name + ".npz"), xstar=xs, mean=mean, var=var)
+        out = OUT_FIRST if name in CASES_FIRST else OUT
+        np.savez_compressed(os.path.join(out, name + ".npz"), xstar=xs, mean=mean, var=var)
         print(name, mean[0, :3], var[0, :3])
 
 

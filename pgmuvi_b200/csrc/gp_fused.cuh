@@ -1070,8 +1070,13 @@ struct FitArgs {
   int32_t* n_iter;
 };
 
+// torch.nn.functional.softplus (beta 1, threshold 20), the transform of GPyTorch's Positive /
+// GreaterThan: x itself above the threshold, where its derivative is exactly 1
 __device__ __forceinline__ double softplus_d(double x) {
-  return x > 30.0 ? x : log1p(exp(x));
+  return x > 20.0 ? x : log1p(exp(x));
+}
+__device__ __forceinline__ double softplus_grad_d(double x) {
+  return x > 20.0 ? 1.0 : 1.0 / (1.0 + exp(-x));
 }
 __device__ __forceinline__ double sigmoid_d(double x) { return 1.0 / (1.0 + exp(-x)); }
 
@@ -1113,7 +1118,7 @@ __device__ __forceinline__ void constrain(int kd, double raw, double lb, double 
   double t = raw, j = 1.0;
   if (kd == PGM_CON_SOFTPLUS) {
     t = softplus_d(raw) + lb;
-    j = sigmoid_d(raw);
+    j = softplus_grad_d(raw);
   } else if (kd == PGM_CON_INTERVAL) {
     const double s = sigmoid_d(raw);
     t = lb + (ub - lb) * s;
@@ -1121,7 +1126,7 @@ __device__ __forceinline__ void constrain(int kd, double raw, double lb, double 
   } else if (kd == PGM_CON_RSOFTPLUS) {
     const double v = softplus_d(raw) + lb;
     t = ub / v;
-    j = -ub * sigmoid_d(raw) / (v * v);
+    j = -ub * softplus_grad_d(raw) / (v * v);
   }
   *th = t;
   if (jc) *jc = j;

@@ -203,18 +203,22 @@ def test_staged_engine_jitter_ladder_and_bitwise_agreement_with_fused(cuda_devic
 # ---------------------------------------------------------------------------------------
 # N1: posterior prediction (pgm_sm_predict_f64)
 # ---------------------------------------------------------------------------------------
-PRED_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden_predict")
-PRED_CASES = sorted(f[:-4] for f in os.listdir(PRED_DIR) if f.endswith(".npz"))
+HERE = os.path.dirname(os.path.abspath(__file__))
+PRED_FILES = {f[:-4]: os.path.join(dd, f)
+              for dd in (os.path.join(HERE, "golden_predict"), os.path.join(HERE, "golden", "predict"))
+              for f in os.listdir(dd) if f.endswith(".npz")}
+PRED_CASES = sorted(PRED_FILES)
 
 
 @pytest.mark.parametrize("name", PRED_CASES)
 def test_prediction_matches_oracle_goldens(name, cuda_device):
     """mean* and the exact latent variance at 150 test points per light curve against the
-    oracle's Cholesky-solve prediction (tests/golden_predict, oracle/make_golden_predict.py).
+    oracle's Cholesky-solve prediction (tests/golden_predict and tests/golden/predict,
+    oracle/make_golden_predict.py).
     Tolerance 1e-9 of the prior variance scale (var* is a difference of O(1) quantities)."""
     from pgmuvi_b200 import ops
     g = load_golden(name)
-    p = np.load(os.path.join(PRED_DIR, name + ".npz"))
+    p = np.load(PRED_FILES[name])
     dev = cuda_device
     mean, var, info = ops.sm_predict(
         _t(g["x"], dev), _t(g["y"], dev), _t(g["noise"], dev), _t(g["raw"], dev),

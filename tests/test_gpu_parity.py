@@ -63,7 +63,8 @@ def test_kernel_builder_matches_goldens(name, cuda_device):
 
 
 @pytest.mark.parametrize("name", ["sm1d_n100_q2_learn", "sm1d_n200_q4", "sm2d_prodsum_4x48_q4",
-                                  "sm1d_ragged_q4"])
+                                  "sm1d_ragged_q4", "sm2d_prodsum_3x64_q8",
+                                  "sm2d_sumprod_3x64_q6_learn"])
 def test_fused_fit_kernel_matches_oracle_adamw_steps(name, cuda_device):
     """pgm_sm_fit (whole loop on device) vs trainers.train restated in the oracle: loss
     before each step and raw parameters after each step (AdamW, lr 0.1, torch defaults)."""
@@ -249,7 +250,8 @@ F32_RTOL = 1e-4   # north star: MLL and gradients within 1e-4 relative in fp32
 
 
 @pytest.mark.parametrize("name", ["sm1d_n100_q2_learn", "sm1d_n512_q4", "sm1d_ragged_q4",
-                                  "sm2d_prodsum_4x48_q4", "sep_rq_4x48_q4"])
+                                  "sm2d_prodsum_4x48_q4", "sep_rq_4x48_q4", "sm2d_prodsum_3x64_q8",
+                                  "sm1d_n130_q5_learn"])
 def test_f32_entry_matches_f64_path_on_the_same_rounded_inputs(name, cuda_device):
     """pgm_sm_mll_grad_f32 = fp32 storage, fp64 arithmetic: on the fp32-rounded inputs it must
     equal the fp64 entry point rounded once to fp32, and stay within the fp32 bar of the
