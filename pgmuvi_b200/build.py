@@ -25,8 +25,6 @@ NVCC_FLAGS = [
     # -lineinfo); the driver inflates it when the module is loaded
     "-Xfatbin=-compress-all", "--compress-mode=size",
 ]
-if os.environ.get("PGM_DEBUG_HOOKS"):   # per-phase clock64 profile (PGM_DEBUG_PROF=1 at run time)
-    NVCC_FLAGS.append("-DPGM_DEBUG_HOOKS")
 # (KIND, QT, D) instantiations: 1-D SM, 2-D ARD product-of-sums, 2-D sum-of-products
 CONFIGS = [(k, q, d) for (k, d) in ((0, 1), (1, 2), (2, 2)) for q in (1, 2, 4, 8)]
 # separable SM(time) x {RBF, Matern-1.5, RQ, Constant}(wavelength): QT in {4, 8}

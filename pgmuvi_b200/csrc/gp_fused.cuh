@@ -160,29 +160,6 @@ __device__ __forceinline__ void load_exp_tab(double* tab) {
   if (threadIdx.x < EXP_TAB) tab[threadIdx.x] = c_exp2_tab[threadIdx.x];
 }
 
-#ifdef PGM_DEBUG_HOOKS
-// -DPGM_DEBUG_HOOKS: per-phase clock64 totals of thread 0 and decomposition switches
-// (PGM_DEBUG_MODE: 0x100 no operand loads, 0x200 no MMAs, 0x400 no exp/cos epilogue work,
-// 0x800 ignore potrf failures, 0x1000 skip the diagonal-block factorisation, 0x2000 no tile
-// bulk stores, 0x4000 no resident-tile products, 0x8000 no epilogue loops) -
-// timing experiments only, results are garbage
-__constant__ int c_dbg = 0;
-#define PGM_DBG(bit) (c_dbg & (bit))
-__constant__ long long* c_prof = nullptr;
-#define PGM_PROF_START() long long prof_t = clock64()
-#define PGM_PROF(slot)                                                       \
-  do {                                                                       \
-    if (c_prof && threadIdx.x == 0) {                                        \
-      const long long t_ = clock64();                                        \
-      c_prof[blockIdx.x * 16 + (slot)] += t_ - prof_t;                       \
-      prof_t = t_;                                                           \
-    }                                                                        \
-  } while (0)
-#else
-#define PGM_DBG(bit) 0
-#define PGM_PROF_START() do { } while (0)
-#define PGM_PROF(slot) do { } while (0)
-#endif
 __device__ __forceinline__ double exp_neg(double x, const double* __restrict__ tab) {
   // clamp x >= -700 on the integer pipe (sign-magnitude: larger high word = more negative)
   const unsigned hx = min((unsigned)__double2hiint(x), 0xC085E000u);
@@ -448,7 +425,6 @@ __device__ __forceinline__ int gemm_stream_r(double (&acc)[4][2][2], Ring& rg, i
     if (use > 0) mbar_wait(rg.empty + 8 * s, (use - 1) & 1);
     const unsigned bar = rg.full + 8 * s;
     const unsigned dst = smem_u32(rg.stages + s * 2 * OPBUF);
-    if (PGM_DBG(0x100)) { mbar_arrive(bar); return; }
     mbar_expect_tx(bar, 2 * CHUNK_BYTES);
     bulk_g2s(dst, ga, CHUNK_BYTES, bar);
     bulk_g2s(dst + CHUNK_BYTES, gb, CHUNK_BYTES, bar);
@@ -473,8 +449,7 @@ __device__ __forceinline__ int gemm_stream_r(double (&acc)[4][2][2], Ring& rg, i
     mbar_wait(rg.full + 8 * s, (q / NST) & 1);
     const double* sA = rg.stages + s * 2 * OPBUF;
     const double* sB = sA + OPBUF;
-    if (PGM_DBG(0x200)) {
-    } else if (MODE0 != M_FULL && c < 2)
+    if (MODE0 != M_FULL && c < 2)
       compute_chunk<MODE0, LOWER>(acc, sA, sB, c * (KC / 8), wm, wn, g, tq);
     else
       compute_chunk<M_FULL, LOWER>(acc, sA, sB, 0, wm, wn, g, tq);
@@ -504,7 +479,6 @@ __device__ __forceinline__ void ring_issue_first(const Ring& rg, const double* g
   const unsigned bar = rg.full + 8 * s;
   const unsigned dst = smem_u32(rg.stages + s * 2 * OPBUF);
   fence_proxy_async_smem();   // stage 0 was last written by cp.async (the per-point fields)
-  if (PGM_DBG(0x100)) { mbar_arrive(bar); return; }
   mbar_expect_tx(bar, 2 * CHUNK_BYTES);
   bulk_g2s(dst, ga, CHUNK_BYTES, bar);
   bulk_g2s(dst + CHUNK_BYTES, gb, CHUNK_BYTES, bar);
@@ -542,7 +516,7 @@ __device__ __forceinline__ void store_tile_bulk(const double (&acc)[4][2][2], do
   store_acc_tile(acc, stage, sign);
   fence_proxy_async_smem();
   __syncthreads();
-  if (threadIdx.x == 0 && !PGM_DBG(0x2000)) {
+  if (threadIdx.x == 0) {
     bulk_s2g(gtile, smem_u32(stage), 2 * OPBUF * sizeof(double));
     bulk_commit();
   }
@@ -1379,7 +1353,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   const unsigned rbar = bars + 8 * 10;
   constexpr bool LEAN = C::LEAN;
 
-  PGM_PROF_START();
   __syncthreads();
   // ---- constraints: raw -> theta, d theta / d raw  (A.2) -----------------------------
   load_theta(A, b, P, raw, theta, jac);
@@ -1428,7 +1401,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   for (int q = 0; q < QT * DS; ++q) areg[q] = aq[q];
 #pragma unroll
   for (int q = 0; q < 4; ++q) lam[q] = lamq[q];
-  PGM_PROF(0);
   double acc[4][2][2];
   double iq_part = 0.0;  // partial of z^T z
   double ld_part = 0.0;  // partial of sum log L_kk
@@ -1441,7 +1413,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
     store_acc_tile(acc, Cst, 1.0);
     __syncthreads();
     zero_acc(acc);
-    if (PGM_DBG(0x4000)) return;
     compute_chunk<M_B_LE, false>(acc, Cst, R, 0, wm, wn, g, tq);
     compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
   };
@@ -1477,7 +1448,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
           cp_async_wait<0>();
           __syncthreads();
         }
-        PGM_PROF(1);
         // epilogue: C = Ktilde_ij - acc (diagonal tiles: lower triangle only).  The
         // accumulators are parked in stage 1 (the image the next product reads as its A
         // operand) so that the registers go to the exp / cos chains: one rolled loop over the
@@ -1485,7 +1455,7 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
         // (padded points carry finite dummy fields); MMA tiles above the diagonal are skipped.
         store_acc_tile(acc, Cst, 1.0);
 #pragma unroll 1
-        for (int p8 = PGM_DBG(0x8000) ? 8 : 0; p8 < 8; ++p8) {
+        for (int p8 = 0; p8 < 8; ++p8) {
           const int mi = p8 >> 1, ni2 = p8 & 1;
           if (i == j && frag_mt(wm, mi) < frag_nt(wn, ni2)) continue;
           const int r = frag_row(wm, mi, g), c0 = frag_col(wn, ni2, tq, 0);
@@ -1496,8 +1466,7 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
 #pragma unroll
           for (int e = 0; e < 2; ++e) {
             const int gj = j * TS + c0 + e;
-            double kv = PGM_DBG(0x400) ? 1e-3
-                                       : k_entry<KIND, QT, D>(rowv, colv, r, c0 + e, wreg, areg, lam, tab);
+            double kv = k_entry<KIND, QT, D>(rowv, colv, r, c0 + e, wreg, areg, lam, tab);
             kv = (gi < n && gj <= gi) ? kv : 0.0;
             if (gi == gj) kv = (gi < n) ? (kv + sc.dn[gi] + jitter) : 1.0;
             out[e] = kv - (e ? cv.y : cv.x);
@@ -1509,12 +1478,10 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
             *cp = make_double2(out[0], out[1]);
           }
         }
-        PGM_PROF(2);
         if (i == j) {
           __syncthreads();
-          if (!PGM_DBG(0x1000)) potrf_inv_64(S, S2, dinv, s_fail);
-          PGM_PROF(3);
-          if (*s_fail && !PGM_DBG(0x800)) { failed = true; break; }
+          potrf_inv_64(S, S2, dinv, s_fail);
+          if (*s_fail) { failed = true; break; }
           // X_jj -> tile(j,j) and the resident R, X_jj^T -> tilesT[j]  (tile images with
           // explicit zeros in the other triangle); L_jj itself is not needed any more
           double* dt = tile(j, j);
@@ -1558,7 +1525,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
             }
           }
           __syncthreads();
-          PGM_PROF(4);
         } else {
           // L_ij = C * X_jj^T  straight from shared memory (C in stage 1, X_jj resident)
           __syncthreads();
@@ -1569,10 +1535,8 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
             pre = 1;
           }
           zero_acc(acc);
-          if (!PGM_DBG(0x4000)) {
-            compute_chunk<M_B_LE, false>(acc, Cst, R, 0, wm, wn, g, tq);
-            compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
-          }
+          compute_chunk<M_B_LE, false>(acc, Cst, R, 0, wm, wn, g, tq);
+          compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
           // partial products L_ij z_j for the forward solve of row i (deterministic order);
           // their global stores are issued after the tile has left, so that the proxy fence
           // of the bulk store (MEMBAR.ALL.CTA) has no global store of this thread to drain
@@ -1594,12 +1558,11 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
             for (int mi = 0; mi < 4; ++mi)
               sc.fpart[((size_t)tri(i, j) * 4 + wn) * TS + frag_row(wm, mi, g)] = pp[mi];
           }
-          PGM_PROF(5);
         }
       }
     }
     __syncthreads();
-    const int fl = PGM_DBG(0x800) ? 0 : *s_fail;
+    const int fl = *s_fail;
     if (!fl) { info = attempt; break; }
     if (fl & 2) { info = -1; break; }
     info = -2;
@@ -1613,7 +1576,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   }
   const double mll = (info >= 0) ? mll_value(fin[0], 2.0 * fin[1], n) : nan("");
   __syncthreads();
-  PGM_PROF(6);
   if (tid == 0) *mll_out = mll;
   if (!want_grad || info < 0) {
     if (want_grad && tid < P) grad_out[tid] = nan("");
@@ -1645,7 +1607,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
         auto nB = [&](int kk) { return tile(ni, nj + kk); };
         pre = gemm_stream<M_A_GE, false, 2>(acc, r2, i - j, tA, tB, pre, nnk, nA, nB, []() {});
         __syncthreads();
-        PGM_PROF(7);
         if (rwait) {
           mbar_wait(rbar, ps.rcnt & 1);
           ++ps.rcnt;
@@ -1672,7 +1633,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
           for (int mi = 0; mi < 4; ++mi)
             sc.apart[((size_t)tri(i, j) * 4 + wn) * TS + frag_row(wm, mi, g)] = pp[mi];
         }
-        PGM_PROF(8);
       }
     }
   }
@@ -1694,7 +1654,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
       __syncthreads();
     }
   }
-  PGM_PROF(9);
   // ================= phase G: K^-1 tiles -> gradient contraction =======================
   double ga[C::NG];
 #pragma unroll
@@ -1725,13 +1684,12 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
         if (i == j) pre = gemm_stream<M_A_GE, true, 2>(acc, r2, N - i, tA, tB, pre, nnk, nA, nB, pf);
         else pre = gemm_stream<M_A_GE, false, 2>(acc, r2, N - i, tA, tB, pre, nnk, nA, nB, pf);
         __syncthreads();
-        PGM_PROF(10);
         // K^-1 tile parked (R, free in this phase; LEAN: stage 1); rolled, branch-free contraction
         store_acc_tile(acc, parkg, 1.0);
         const double* al_r = rowg + C::NFB * TS;
         const double* al_c = colg + C::NFB * TS;
 #pragma unroll 1
-        for (int p8 = PGM_DBG(0x8000) ? 8 : 0; p8 < 8; ++p8) {
+        for (int p8 = 0; p8 < 8; ++p8) {
           const int mi = p8 >> 1, ni2 = p8 & 1;
           if (i == j && frag_mt(wm, mi) < frag_nt(wn, ni2)) continue;
           const int r = frag_row(wm, mi, g), c0 = frag_col(wn, ni2, tq, 0);
@@ -1744,11 +1702,9 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
             W = (gi < n && gj <= gi) ? W : 0.0;
             if (gi == gj) trW += W;
             const double wgt = (gi == gj) ? W : 2.0 * W;
-            if (!PGM_DBG(0x400))
-              k_grad_entry<KIND, QT, D>(rowg, colg, r, c0 + e, wreg, areg, lam, tab, wgt, ga);
+            k_grad_entry<KIND, QT, D>(rowg, colg, r, c0 + e, wreg, areg, lam, tab, wgt, ga);
           }
         }
-        PGM_PROF(11);
       }
     }
     ps.gq2 = r2.gq;
@@ -1770,7 +1726,6 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   }
   if (tid < P) grad_out[tid] = grad_slot<KIND, QT, D>(tid, n, L, fin, theta, wq, lamq) * jac[tid];
   __syncthreads();
-  PGM_PROF(12);
   return info;
 }
 

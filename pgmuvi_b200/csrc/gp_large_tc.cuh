@@ -92,23 +92,27 @@ static __global__ void __launch_bounds__(NTHREADS) lg_pack_tf32(LargeArgs A) {
 // ------------------------------------------------------------------------------------
 constexpr unsigned T_MASTER = 0, T_MLO = 128, T_PIECE = 256;
 
+// Pieces of 16 k, two per 32-k chunk (two truncating hi hi additions each): accuracy first.  32-k
+// pieces halve the drain work - C4's G phase 170 -> 112 ms - at 1.8x the error (DESIGN.md 4.2b).
+constexpr int TC_PPC = 2;              // pieces per 32-k chunk
+constexpr int TC_KPP = 4 / TC_PPC;     // 8-k MMA steps per piece
+constexpr int TC_FOLD = 4;             // pieces per register fold of tc_drain
+
 struct TcCtx {
   unsigned base;        // shared address of stage 0 (1024-byte aligned)
   unsigned bar_full, bar_empty, bar_pfull, bar_pempty, tslot;
   unsigned tmem;
-  int nst, ppc;         // pipeline stages, pieces per 32-k chunk (1 or 2)
 };
 
 // all threads; `bars` = shared address of 14 doubles.  Ends with a block barrier.
-__device__ __forceinline__ void tc_setup(TcCtx& cx, unsigned stage_base, unsigned bars, int nst,
-                                         int half_pieces) {
+template <int NST>
+__device__ __forceinline__ void tc_setup(TcCtx& cx, unsigned stage_base, unsigned bars) {
+  static_assert(NST >= 1 && NST <= 3, "the barrier region holds the full / empty pairs of 3 stages");
   cx.base = stage_base;
   cx.bar_full = bars; cx.bar_empty = bars + 24; cx.bar_pfull = bars + 48; cx.bar_pempty = bars + 64;
   cx.tslot = bars + 96;
-  cx.nst = nst;
-  cx.ppc = half_pieces ? 2 : 1;
   if (threadIdx.x == 0) {
-    for (int s = 0; s < nst; ++s) { mbar_init(cx.bar_full + 8 * s, 1); mbar_init(cx.bar_empty + 8 * s, 1); }
+    for (int s = 0; s < NST; ++s) { mbar_init(cx.bar_full + 8 * s, 1); mbar_init(cx.bar_empty + 8 * s, 1); }
     for (int s = 0; s < 2; ++s) { mbar_init(cx.bar_pfull + 8 * s, 1); mbar_init(cx.bar_pempty + 8 * s, 8); }
     asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
     fence_proxy_async();
@@ -125,10 +129,11 @@ __device__ __forceinline__ void tc_teardown(const TcCtx& cx) {
 }
 
 // warp 0, one lane: stream the four operand images of every chunk (hi / lo at ahi / alo + kc * IMG)
+template <int NST>
 __device__ __forceinline__ void tc_producer(const TcCtx& cx, const float* ahi, const float* alo,
                                             const float* bhi, const float* blo, int nchunks) {
   for (int c = 0; c < nchunks; ++c) {
-    const int s = c % cx.nst, use = c / cx.nst;
+    const int s = c % NST, use = c / NST;
     if (use > 0) mbar_wait(cx.bar_empty + 8 * s, (use - 1) & 1);
     const unsigned bar = cx.bar_full + 8 * s, dst = cx.base + (unsigned)s * 4 * tc::IMG_BYTES;
     const size_t o = (size_t)c * tc::IMG_FLOATS;
@@ -141,23 +146,23 @@ __device__ __forceinline__ void tc_producer(const TcCtx& cx, const float* ahi, c
 }
 
 // warp 1, one lane: per piece the cross terms (hi lo + lo hi) first, then hi hi
+template <int NST>
 __device__ __forceinline__ void tc_mma_issuer(const TcCtx& cx, int nchunks) {
   constexpr uint32_t idesc = tc::idesc_tf32(128, 128);
-  const int ppc = cx.ppc, kpp = 4 / ppc;
   for (int c = 0; c < nchunks; ++c) {
-    const int s = c % cx.nst, use = c / cx.nst;
+    const int s = c % NST, use = c / NST;
     mbar_wait(cx.bar_full + 8 * s, use & 1);
     tc::fence_after_sync();
     const unsigned st = cx.base + (unsigned)s * 4 * tc::IMG_BYTES;
-    for (int hp = 0; hp < ppc; ++hp) {
-      const int piece = c * ppc + hp, buf = piece & 1;
+    for (int hp = 0; hp < TC_PPC; ++hp) {
+      const int piece = c * TC_PPC + hp, buf = piece & 1;
       if (piece >= 2) {                  // the epilogue has drained this piece buffer
         mbar_wait(cx.bar_pempty + 8 * buf, ((piece >> 1) - 1) & 1);
         tc::fence_after_sync();
       }
       const unsigned tp = cx.tmem + T_PIECE + 128u * (unsigned)buf;
-      const int ks0 = hp * kpp;
-      for (int ks = ks0; ks < ks0 + kpp; ++ks) {
+      const int ks0 = hp * TC_KPP;
+      for (int ks = ks0; ks < ks0 + TC_KPP; ++ks) {
         const uint64_t ahi = tc::smem_desc_sw128(st + ks * 32);
         const uint64_t alo = tc::smem_desc_sw128(st + tc::IMG_BYTES + ks * 32);
         const uint64_t bhi = tc::smem_desc_sw128(st + 2 * tc::IMG_BYTES + ks * 32);
@@ -165,7 +170,7 @@ __device__ __forceinline__ void tc_mma_issuer(const TcCtx& cx, int nchunks) {
         tc::mma_tf32(tp, alo, bhi, idesc, ks > ks0 ? 1u : 0u);
         tc::mma_tf32(tp, ahi, blo, idesc, 1u);
       }
-      for (int ks = ks0; ks < ks0 + kpp; ++ks) {
+      for (int ks = ks0; ks < ks0 + TC_KPP; ++ks) {
         const uint64_t ahi = tc::smem_desc_sw128(st + ks * 32);
         const uint64_t bhi = tc::smem_desc_sw128(st + 2 * tc::IMG_BYTES + ks * 32);
         tc::mma_tf32(tp, ahi, bhi, idesc, 1u);
@@ -176,17 +181,17 @@ __device__ __forceinline__ void tc_mma_issuer(const TcCtx& cx, int nchunks) {
   }
 }
 
-// The 8 epilogue warps drain every piece: two levels.  Level 1: a running sum of `fold` consecutive
-// pieces in REGISTERS (64 floats per thread, plain round-to-nearest adds: `fold` = 4 keeps their error
-// at the level of one piece's own truncation) - 4 LDTM + 64 FADD per piece.  Level 2: every `fold`
+// The 8 epilogue warps drain every piece: two levels.  Level 1: a running sum of TC_FOLD consecutive
+// pieces in REGISTERS (64 floats per thread, plain round-to-nearest adds: a fold of 4 keeps their error
+// at the level of one piece's own truncation) - 4 LDTM + 64 FADD per piece.  Level 2: every TC_FOLD
 // pieces the running sum goes into the float-pair master accumulator in TMEM by Fast2Sum (|hi| >= |sum|
 // but for the first folds, where the missed rounding error is of no consequence).  Draining every piece
 // straight into the TMEM master (r02k: ~400 instructions per thread and piece, tensor pipe 18 % active)
 // made the drain, not the tensor pipe, the bound.  tlane = TMEM address of this thread's lane at its
 // first column.
-__device__ __forceinline__ void tc_drain(const TcCtx& cx, unsigned tlane, int nchunks, int fold) {
+__device__ __forceinline__ void tc_drain(const TcCtx& cx, unsigned tlane, int nchunks) {
   const int lane = threadIdx.x & 31;
-  const int npieces = nchunks * cx.ppc;
+  const int npieces = nchunks * TC_PPC;
   float m1[64];
   int in_fold = 0, nfold = 0;
   for (int piece = 0; piece < npieces; ++piece) {
@@ -219,7 +224,7 @@ __device__ __forceinline__ void tc_drain(const TcCtx& cx, unsigned tlane, int nc
         m1[48 + e] = first ? p3[e] : __fadd_rn(m1[48 + e], p3[e]);
       }
     }
-    if (++in_fold == fold || piece == npieces - 1) {
+    if (++in_fold == TC_FOLD || piece == npieces - 1) {
 #pragma unroll
       for (int c0 = 0; c0 < 64; c0 += 16) {
         float hi[16], lo[16];
@@ -302,13 +307,17 @@ struct TcGradSmem {
   static constexpr int PAR_RED = PAR_TAB + EXP_TAB;           // [8][NV] warp partials
   static constexpr int PAR_BAR = PAR_RED + 8 * C::NV;         // mbarriers (10) + TMEM slot
   static constexpr int PAR_END = PAR_BAR + 14;
-  static __host__ __device__ constexpr size_t bytes(int nst) {
-    return 1024 + (size_t)nst * 4 * tc::IMG_BYTES + (size_t)(2 * SIDE + PAR_END) * sizeof(double);
-  }
+  // 1024 bytes of alignment slack, NST pipeline stages of four operand images, the doubles above
+  static constexpr size_t STAGE = 4 * tc::IMG_BYTES;
+  static constexpr size_t FIXED = 1024 + (size_t)(2 * SIDE + PAR_END) * sizeof(double);
+  // pipeline stages: the most, up to 3, that fit in a block's 227 KB of shared memory
+  static constexpr int NST = FIXED + 3 * STAGE <= 227 * 1024 ? 3 : FIXED + 2 * STAGE <= 227 * 1024 ? 2 : 1;
+  static constexpr size_t BYTES = FIXED + NST * STAGE;
+  static_assert(BYTES <= 227 * 1024, "lg_grad_tc / lg_update_tc do not fit in shared memory");
 };
 
 template <int KIND, int QT, int D>
-__global__ void __launch_bounds__(TC_THREADS, 1) lg_grad_tc(LargeArgs A, int nst, int half_pieces, int fold) {
+__global__ void __launch_bounds__(TC_THREADS, 1) lg_grad_tc(LargeArgs A) {
   using C = Cfg<KIND, QT, D>;
   using SM = TcGradSmem<KIND, QT, D>;
   constexpr int DS = C::DS;
@@ -328,22 +337,22 @@ __global__ void __launch_bounds__(TC_THREADS, 1) lg_grad_tc(LargeArgs A, int nst
 
   const unsigned base = (smem_u32(smraw) + 1023u) & ~1023u;
   unsigned char* gen = smraw + (base - smem_u32(smraw));
-  double* sd = reinterpret_cast<double*>(gen + (size_t)nst * 4 * tc::IMG_BYTES);
+  double* sd = reinterpret_cast<double*>(gen + SM::NST * SM::STAGE);
   double* rowv = sd;
   double* colv = sd + SM::SIDE;
   double* par = sd + 2 * SM::SIDE;
   double* tab = par + SM::PAR_TAB;
   double* red = par + SM::PAR_RED;
   TcCtx cx;
-  tc_setup(cx, base, smem_u32(par + SM::PAR_BAR), nst, half_pieces);
+  tc_setup<SM::NST>(cx, base, smem_u32(par + SM::PAR_BAR));
 
   if (warp == 0) {
     if (lane == 0) {
       const size_t oa = ((size_t)I * KCH + kc0) * tc::IMG_FLOATS, ob = ((size_t)J * KCH + kc0) * tc::IMG_FLOATS;
-      tc_producer(cx, phi + oa, plo + oa, phi + ob, plo + ob, nchunks);
+      tc_producer<SM::NST>(cx, phi + oa, plo + oa, phi + ob, plo + ob, nchunks);
     }
   } else if (warp == 1) {
-    if (lane == 0) tc_mma_issuer(cx, nchunks);
+    if (lane == 0) tc_mma_issuer<SM::NST>(cx, nchunks);
   } else {
     // ---------------- epilogue warps: per-point fields while the products run ----------------
     const int et = tid - 64;                              // 0..255
@@ -370,7 +379,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) lg_grad_tc(LargeArgs A, int nst
     const int gi = I * 128 + r;
     const double al_i = rv[C::NFB * TS + rr];
     const unsigned tlane = cx.tmem + ((unsigned)(32 * q4) << 16) + (unsigned)(half * 64);
-    tc_drain(cx, tlane, nchunks, fold);
+    tc_drain(cx, tlane, nchunks);
     // tcgen05.ld is warp-collective: the chunk loop is uniform over the warp (rows 32 q4 .. + 31),
     // the lower-triangle / n masks act per entry
     const int gi_hi = I * 128 + 32 * q4 + 31;
@@ -449,7 +458,7 @@ static __global__ void __launch_bounds__(NTHREADS) lg_pack_panel_tf32(LargeArgs 
 // per 128x128 tile; build: C_ij = K~_ij - sum (first panel), exactly as lg_update mode 1
 template <int KIND, int QT, int D>
 __global__ void __launch_bounds__(TC_THREADS, 1)
-    lg_update_tc(LargeArgs A, int J0, int J1, int build, int nst, int half_pieces, int fold) {
+    lg_update_tc(LargeArgs A, int J0, int J1, int build) {
   using C = Cfg<KIND, QT, D>;
   using SM = TcGradSmem<KIND, QT, D>;
   constexpr int DS = C::DS;
@@ -471,21 +480,21 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
 
   const unsigned base = (smem_u32(smraw) + 1023u) & ~1023u;
   unsigned char* gen = smraw + (base - smem_u32(smraw));
-  double* sd = reinterpret_cast<double*>(gen + (size_t)nst * 4 * tc::IMG_BYTES);
+  double* sd = reinterpret_cast<double*>(gen + SM::NST * SM::STAGE);
   double* rowv = sd;
   double* colv = sd + SM::SIDE;
   double* par = sd + 2 * SM::SIDE;
   double* tab = par + SM::PAR_TAB;
   TcCtx cx;
-  tc_setup(cx, base, smem_u32(par + SM::PAR_BAR), nst, half_pieces);
+  tc_setup<SM::NST>(cx, base, smem_u32(par + SM::PAR_BAR));
 
   if (warp == 0) {
     if (lane == 0) {
       const size_t oa = (size_t)I * KCH * tc::IMG_FLOATS, ob = (size_t)J * KCH * tc::IMG_FLOATS;
-      tc_producer(cx, phi + oa, plo + oa, phi + ob, plo + ob, nchunks);
+      tc_producer<SM::NST>(cx, phi + oa, plo + oa, phi + ob, plo + ob, nchunks);
     }
   } else if (warp == 1) {
-    if (lane == 0) tc_mma_issuer(cx, nchunks);
+    if (lane == 0) tc_mma_issuer<SM::NST>(cx, nchunks);
   } else {
     const int et = tid - 64;
     const int q4 = warp & 3, half = (warp - 2) >> 2;
@@ -509,7 +518,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
     const int ti = 2 * I + (r >> 6), tj = 2 * J + half;       // the 64x64 tile of this thread's entries
     const int gi = I * 128 + r;
     const unsigned tlane = cx.tmem + ((unsigned)(32 * q4) << 16) + (unsigned)(half * 64);
-    tc_drain(cx, tlane, nchunks, fold);
+    tc_drain(cx, tlane, nchunks);
     // every lane of the warp shares ti, tj (32 rows of one 64-row sub-tile)
     if (ti < N && tj <= ti) {
       double* out = lg_tile(w.tilesL, ti, tj);

@@ -7,8 +7,6 @@
 #include <algorithm>
 #include <cstdlib>
 #include <string>
-#include <vector>
-#include <cstdio>
 
 namespace pgm {
 int fail(const std::string& m);
@@ -16,80 +14,43 @@ int cuda_fail(const char* what, cudaError_t e);
 int device_sms();
 inline int predict_blocks() { return 2 * device_sms(); }   // persistent blocks of lg_predict
 
-template <int KIND, int QT, int D>
-int launch_eval(const pgm::EvalArgs& A0, cudaStream_t st) {
-  using C = pgm::Cfg<KIND, QT, D>;
-  pgm::EvalArgs A = A0;
-  auto kern = pgm::sm_mll_grad_kernel<KIND, QT, D>;
-  size_t smem = C::F_BYTES;
-  if (const char* f = getenv("PGM_DEBUG_SMEM_KB")) smem = std::max(smem, (size_t)atoi(f) * 1024);
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)smem);
+// the per-light-curve arguments inside a fused kernel's argument block
+inline EvalArgs& eval_args(EvalArgs& A) { return A; }
+inline EvalArgs& eval_args(FitArgs& F) { return F.e; }
+
+// Persistent launch of a fused kernel: as many blocks as are resident at once, at most one per light
+// curve.  The ticket scheduler (sched) runs only on the full grid of two blocks per SM it is built
+// for; every other grid takes the light curves at a fixed stride.
+template <typename Args>
+int launch_persistent(void (*kern)(Args), Args args, size_t smem, const char* what, cudaStream_t st) {
+  EvalArgs& A = eval_args(args);
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute", e);
   int occ = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, pgm::NTHREADS, smem);
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NTHREADS, smem);
   if (e != cudaSuccess) return cuda_fail("occupancy", e);
   if (occ < 1) return fail("kernel does not fit on an SM");
-  int grid = device_sms() * occ;
-  if (grid > A.B) grid = A.B;
   A.sms = device_sms();
+  int grid = A.sms * occ;
+  if (grid > A.B) grid = A.B;
   if (A.sched && (occ != 2 || grid != 2 * A.sms || getenv("PGM_STATIC_STRIDE"))) A.sched = nullptr;
   if (A.sched) cudaMemsetAsync(A.sched, 0, PGM_SCHED_INTS * sizeof(int), st);
-#ifdef PGM_DEBUG_HOOKS
-  {
-    int dbg = 0;
-    if (const char* f = getenv("PGM_DEBUG_MODE")) dbg = (int)strtol(f, nullptr, 0);
-    cudaMemcpyToSymbolAsync(pgm::c_dbg, &dbg, sizeof(int), 0, cudaMemcpyHostToDevice, st);
-  }
-  long long* dprof = nullptr;
-  if (getenv("PGM_DEBUG_PROF")) {
-    cudaMalloc(&dprof, (size_t)grid * 16 * sizeof(long long));
-    cudaMemsetAsync(dprof, 0, (size_t)grid * 16 * sizeof(long long), st);
-  }
-  cudaMemcpyToSymbolAsync(pgm::c_prof, &dprof, sizeof(dprof), 0, cudaMemcpyHostToDevice, st);
-#endif
-  kern<<<grid, pgm::NTHREADS, smem, st>>>(A);
+  kern<<<grid, NTHREADS, smem, st>>>(args);
   e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail("sm_mll_grad_kernel launch", e);
-#ifdef PGM_DEBUG_HOOKS
-  if (dprof) {
-    cudaStreamSynchronize(st);
-    std::vector<long long> h((size_t)grid * 16);
-    cudaMemcpy(h.data(), dprof, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-    cudaFree(dprof);
-    static const char* nm[13] = {"setup", "P.gemm", "P.kepi", "P.potrf", "P.diagpost", "P.trsm", "mll",
-                                 "T.gemm1", "T.gemm2", "alpha", "G.gemm", "G.epi", "final"};
-    double tot = 0, v[13];
-    for (int s2 = 0; s2 < 13; ++s2) { v[s2] = 0; for (int b = 0; b < grid; ++b) v[s2] += (double)h[(size_t)b * 16 + s2]; v[s2] /= grid; tot += v[s2]; }
-    fprintf(stderr, "[pgm prof] per-CTA cycles (avg over %d CTAs), total %.0f:", grid, tot);
-    for (int s2 = 0; s2 < 13; ++s2) fprintf(stderr, " %s %.0f (%.1f%%)", nm[s2], v[s2], 100 * v[s2] / tot);
-    fprintf(stderr, "\n");
-  }
-#endif
+  if (e != cudaSuccess) return cuda_fail(what, e);
   return 0;
 }
 
 template <int KIND, int QT, int D>
-int launch_fit(const pgm::FitArgs& F, cudaStream_t st) {
-  using C = pgm::Cfg<KIND, QT, D>;
-  auto kern = pgm::sm_fit_kernel<KIND, QT, D>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)C::F_BYTES);
-  if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute", e);
-  int occ = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, pgm::NTHREADS, C::F_BYTES);
-  if (e != cudaSuccess) return cuda_fail("occupancy", e);
-  if (occ < 1) return fail("kernel does not fit on an SM");
-  int grid = device_sms() * occ;
-  if (grid > F.e.B) grid = F.e.B;
-  pgm::FitArgs F2 = F;
-  F2.e.sms = device_sms();
-  if (F2.e.sched && (occ != 2 || grid != 2 * F2.e.sms || getenv("PGM_STATIC_STRIDE"))) F2.e.sched = nullptr;
-  if (F2.e.sched) cudaMemsetAsync(F2.e.sched, 0, PGM_SCHED_INTS * sizeof(int), st);
-  kern<<<grid, pgm::NTHREADS, C::F_BYTES, st>>>(F2);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail("sm_fit_kernel launch", e);
-  return 0;
+int launch_eval(const EvalArgs& A, cudaStream_t st) {
+  return launch_persistent(sm_mll_grad_kernel<KIND, QT, D>, A, Cfg<KIND, QT, D>::F_BYTES,
+                           "sm_mll_grad_kernel launch", st);
+}
+
+template <int KIND, int QT, int D>
+int launch_fit(const FitArgs& F, cudaStream_t st) {
+  return launch_persistent(sm_fit_kernel<KIND, QT, D>, F, Cfg<KIND, QT, D>::F_BYTES,
+                           "sm_fit_kernel launch", st);
 }
 
 template <int KIND, int QT, int D>
@@ -112,13 +73,6 @@ int launch_dense(const pgm::EvalArgs& A, double* K, cudaStream_t st) {
 // dependency stage with B x (tiles of the stage) blocks; B = 1 is the single large GP.
 // Host-orchestrated on `st`; synchronises once per Cholesky pass to read how many light curves
 // must repeat it with more jitter (psd_safe_cholesky's ladder) - the call is blocking.
-// pieces per level-1 fold of the tcgen05 drain (gp_large_tc.cuh::tc_drain)
-inline int tc_fold() {
-  int f = 4;
-  if (const char* e = getenv("PGM_TC_FOLD")) f = std::max(1, atoi(e));
-  return f;
-}
-
 template <int KIND, int QT, int D>
 int launch_large(const pgm::LargeArgs& A, int want_grad, cudaStream_t st, int predict_only = 0) {
   using C = pgm::Cfg<KIND, QT, D>;
@@ -162,7 +116,7 @@ int launch_large(const pgm::LargeArgs& A, int want_grad, cudaStream_t st, int pr
     // ... and only while a dependency stage cannot fill the device by itself: big batches have
     // all the parallelism they need in one launch per stage (C5: 52.8 vs 62.9 ms)
     const bool few = (long long)B * N < 1024;
-    const bool one_launch = !getenv("PGM_STAGED_ROWWISE") && few && N <= all_n && ncb <= 2147483647LL;
+    const bool one_launch = few && N <= all_n && ncb <= 2147483647LL;
     if (one_launch) {   // dataflow Cholesky: the whole pass in one flag-ordered launch
       cudaMemsetAsync(bs.tflag, 0, (size_t)B * large_ntri(n) * sizeof(int), st);
       k_chol<<<dim3((unsigned)ncb), blk, CHOL_SMEM, st>>>(A);
@@ -178,18 +132,13 @@ int launch_large(const pgm::LargeArgs& A, int want_grad, cudaStream_t st, int pr
       }
       if (J1 < N && (A.flags & PGM_FLAG_TF32X3_CHOL) && !(J1 & 1)) {
         // trailing update on tcgen05 (3xTF32): pack the panel's L tiles, one CTA per 128x128 tile
-        using TS_ = TcGradSmem<KIND, QT, D>;
+        constexpr size_t TC_SMEM = TcGradSmem<KIND, QT, D>::BYTES;
         auto k_utc = lg_update_tc<KIND, QT, D>;
-        int nst = 3;
-        while (nst > 1 && TS_::bytes(nst) > 227 * 1024) --nst;
-        if (TS_::bytes(nst) > 227 * 1024) return fail("lg_update_tc does not fit in shared memory");
-        e = cudaFuncSetAttribute(k_utc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TS_::bytes(nst));
+        e = cudaFuncSetAttribute(k_utc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM);
         if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute(lg_update_tc)", e);
-        int halfp = 1;
-        if (const char* f = getenv("PGM_TC_HALF_PIECES")) halfp = atoi(f) ? 1 : 0;
         const int NT = (N + 1) / 2, Mt = NT - J1 / 2;
         lg_pack_panel_tf32<<<dim3(J1 - J0, 2 * NT - J1, B), blk, 0, st>>>(A, J0, J1);
-        k_utc<<<dim3(tc_grid(Mt), B), TC_THREADS, TS_::bytes(nst), st>>>(A, J0, J1, build, nst, halfp, tc_fold());
+        k_utc<<<dim3(tc_grid(Mt), B), TC_THREADS, TC_SMEM, st>>>(A, J0, J1, build);
       } else if (J1 < N) {
         const int M = N - J1;
         k_upd<<<dim3(M * (M + 1) / 2, B), blk, UPD_SMEM, st>>>(A, 1, J1, J0, J1, build);
@@ -209,7 +158,7 @@ int launch_large(const pgm::LargeArgs& A, int want_grad, cudaStream_t st, int pr
     if (!again) break;
   }
   if (want_grad || predict_only) {
-    if (getenv("PGM_STAGED_ROWWISE") || (long long)B * N >= 1024) {   // one launch per tile row
+    if ((long long)B * N >= 1024) {            // one launch per tile row
       for (int i = 1; i < N; ++i) lg_inv_row<<<dim3(i, B), blk, LG_INV_SMEM, st>>>(A, i);
     } else if (N > 1) {                        // whole T phase in one launch, flag-ordered
       cudaMemsetAsync(bs.tflag, 0, (size_t)B * large_ntri(n) * sizeof(int), st);
@@ -223,20 +172,12 @@ int launch_large(const pgm::LargeArgs& A, int want_grad, cudaStream_t st, int pr
       // G phase on tcgen05: X^T -> packed TF32 hi / lo operand images, then one CTA per 128x128
       // tile of K~^-1 (3xTF32 products in tensor memory, FP64 contraction epilogue)
       const int NT = (N + 1) / 2;
-      using TS_ = TcGradSmem<KIND, QT, D>;
+      constexpr size_t TC_SMEM = TcGradSmem<KIND, QT, D>::BYTES;
       auto k_tc = lg_grad_tc<KIND, QT, D>;
-      int nst = 3;
-      if (const char* f = getenv("PGM_TC_STAGES")) nst = std::min(3, std::max(1, atoi(f)));
-      while (nst > 1 && TS_::bytes(nst) > 227 * 1024) --nst;
-      if (TS_::bytes(nst) > 227 * 1024) return fail("lg_grad_tc does not fit in shared memory");
-      e = cudaFuncSetAttribute(k_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TS_::bytes(nst));
+      e = cudaFuncSetAttribute(k_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM);
       if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute(lg_grad_tc)", e);
       lg_pack_tf32<<<dim3(N, 2 * NT, B), blk, 0, st>>>(A);
-      // pieces of 16 k (two truncating hi hi additions each) by default: accuracy first.  32-k pieces
-      // (PGM_TC_HALF_PIECES=0) halve the drain work - C4's G phase 170 -> 112 ms - at 1.8x the error.
-      int halfp = 1;
-      if (const char* f = getenv("PGM_TC_HALF_PIECES")) halfp = atoi(f) ? 1 : 0;
-      k_tc<<<dim3(tc_grid(NT), B), TC_THREADS, TS_::bytes(nst), st>>>(A, nst, halfp, tc_fold());
+      k_tc<<<dim3(tc_grid(NT), B), TC_THREADS, TC_SMEM, st>>>(A);
     } else if (!predict_only) {
       k_grad<<<dim3(N * (N + 1) / 2, B), blk, GRAD_SMEM, st>>>(A);
     }
