@@ -189,6 +189,44 @@ __device__ __forceinline__ void lg_prefetch_side(double* vec, const LargeWs& w, 
   }
 }
 
+// kernel constants of the light curve (written by lg_setup) in registers, for k_entry / k_grad_entry
+template <int KIND, int QT, int D>
+struct LgConst {
+  double w[QT], a[QT * Cfg<KIND, QT, D>::DS], lam[4];
+  __device__ __forceinline__ void load(const double* par) {
+#pragma unroll
+    for (int q = 0; q < QT; ++q) w[q] = par[LG_PAR_WQ + q];
+#pragma unroll
+    for (int q = 0; q < QT * Cfg<KIND, QT, D>::DS; ++q) a[q] = par[LG_PAR_AQ + q];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) lam[q] = par[LG_PAR_LM + q];
+  }
+};
+
+// entry (gi, gj) of the lower triangle of K~ = K + noise + jitter: zero above the diagonal and
+// outside the n valid points, 1 on the diagonal of the padding (r, c: rows of rowv / colv)
+template <int KIND, int QT, int D>
+__device__ __forceinline__ double lg_k_masked(const double* rowv, const double* colv, int r, int c,
+                                              int gi, int gj, int n, const double* dn, double jitter,
+                                              const double (&w)[QT],
+                                              const double (&a)[QT * Cfg<KIND, QT, D>::DS],
+                                              const double (&lam)[4], const double* tab) {
+  double kv = k_entry<KIND, QT, D>(rowv, colv, r, c, w, a, lam, tab);
+  kv = (gi < n && gj <= gi) ? kv : 0.0;
+  if (gi == gj) kv = (gi < n) ? (kv + dn[gi] + jitter) : 1.0;
+  return kv;
+}
+
+// thread 0: mbarriers of gemm_stream's 2-stage Ring{bars, bars + 16} (full / empty) and, unless
+// `extra` is 0, one single-arrival barrier for a resident tile.  A block barrier must follow.
+__device__ __forceinline__ void lg_ring_init(unsigned bars, unsigned extra = 0) {
+  if (threadIdx.x != 0) return;
+  for (int s = 0; s < 2; ++s) { mbar_init(bars + 8 * s, 1); mbar_init(bars + 8 * (2 + s), NTHREADS / 32); }
+  if (extra) mbar_init(extra, 1);
+  asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+  fence_proxy_async();
+}
+
 // Job index of a block of a one-launch dataflow phase: a ticket taken when the block STARTS, so that
 // the job order is the order in which blocks actually begin to run.  Every job only waits for jobs of
 // lower index, and a block holding ticket t started after the blocks holding 0 .. t-1 did, so waiting
@@ -277,7 +315,6 @@ __global__ void __launch_bounds__(NTHREADS, UpdSmem<KIND, QT, D>::MIN_BLOCKS)
     lg_update(LargeArgs A, int mode, int jj, int k0, int k1, int build) {
   using C = Cfg<KIND, QT, D>;
   using L = UpdSmem<KIND, QT, D>;
-  constexpr int DS = C::DS;
   extern __shared__ __align__(16) double sm[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, tq = lane & 3, wm = warp >> 2, wn = warp & 3;
@@ -308,12 +345,7 @@ __global__ void __launch_bounds__(NTHREADS, UpdSmem<KIND, QT, D>::MIN_BLOCKS)
   const unsigned bars = smem_u32(par + C::PAR_BAR);
   const unsigned cbar = bars + 8 * 10;
   load_exp_tab(tab);
-  if (tid == 0) {   // mbarriers: 2-stage ring (full / empty) + the C-tile barrier
-    for (int s2 = 0; s2 < 2; ++s2) { mbar_init(bars + 8 * s2, 1); mbar_init(bars + 8 * (2 + s2), NTHREADS / 32); }
-    mbar_init(cbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    fence_proxy_async();
-  }
+  lg_ring_init(bars, cbar);
   __syncthreads();
   Ring r2{bars, bars + 16, stages, 0};
   double* out = lg_tile(w.tilesL, i, j);
@@ -359,13 +391,8 @@ __global__ void __launch_bounds__(NTHREADS, UpdSmem<KIND, QT, D>::MIN_BLOCKS)
     }
     return;
   }
-  double wreg[QT], areg[QT * DS], lam[4];
-#pragma unroll
-  for (int q = 0; q < QT; ++q) wreg[q] = w.par[LG_PAR_WQ + q];
-#pragma unroll
-  for (int q = 0; q < QT * DS; ++q) areg[q] = w.par[LG_PAR_AQ + q];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) lam[q] = w.par[LG_PAR_LM + q];
+  LgConst<KIND, QT, D> kc;
+  kc.load(w.par);
   store_acc_tile(acc, Cst, 1.0);
 #pragma unroll 1
   for (int p8 = 0; p8 < 8; ++p8) {
@@ -378,10 +405,8 @@ __global__ void __launch_bounds__(NTHREADS, UpdSmem<KIND, QT, D>::MIN_BLOCKS)
     double o2[2];
 #pragma unroll
     for (int e = 0; e < 2; ++e) {
-      const int gj = j * TS + c0 + e;
-      double kv = k_entry<KIND, QT, D>(rowv, colv, r, c0 + e, wreg, areg, lam, tab);
-      kv = (gi < n && gj <= gi) ? kv : 0.0;
-      if (gi == gj) kv = (gi < n) ? (kv + w.dn[gi] + jitter) : 1.0;
+      const double kv = lg_k_masked<KIND, QT, D>(rowv, colv, r, c0 + e, gi, j * TS + c0 + e, n, w.dn,
+                                                 jitter, kc.w, kc.a, kc.lam, tab);
       o2[e] = kv - (e ? cv.y : cv.x);
     }
     *cp = make_double2(o2[0], o2[1]);
@@ -399,6 +424,56 @@ __global__ void __launch_bounds__(NTHREADS, UpdSmem<KIND, QT, D>::MIN_BLOCKS)
 // diagonal block j: C_jj -> X_jj = L_jj^-1 (tilesL / tilesX diagonal slots), X_jj^T (tilesT),
 // z_j = X_jj rhs_j, log-det and z^T z partials
 // ------------------------------------------------------------------------------------
+// After potrf_inv_64 (S2 = X_jj, dinv = 1 / diag L_jj), in two steps.  (a) What the other tiles of
+// column j wait for: X_jj in the L array's diagonal slot and z_j = X_jj zi; red[r] = z_r^2 and
+// red[64 + r] = -log dinv[r] for step (b).
+__device__ __forceinline__ void lg_diag_solve(const LargeWs& w, int j, const double* S2,
+                                              const double* zi, const double* dinv, double* red) {
+  const int tid = threadIdx.x;
+  double* tl = lg_tile(w.tilesL, j, j);
+  for (int idx = tid; idx < TT / 2; idx += NTHREADS) {
+    const int r = idx >> 5, c2 = (idx & 31) * 2;
+    double2 vv;
+    vv.x = (c2 <= r) ? S2[r * LD_S + c2] : 0.0;
+    vv.y = (c2 + 1 <= r) ? S2[r * LD_S + c2 + 1] : 0.0;
+    *reinterpret_cast<double2*>(tl + img(r, c2)) = vv;
+  }
+  const int r = tid >> 2, l4 = tid & 3;
+  double zz = 0.0;
+  for (int c = l4; c <= r; c += 4) zz += S2[r * LD_S + c] * zi[c];
+  zz += shfl_xor_d(zz, 1);
+  zz += shfl_xor_d(zz, 2);
+  if (l4 == 0) {
+    w.z[j * TS + r] = zz;
+    red[r] = zz * zz;
+    red[TS + r] = -log(dinv[r]);
+  }
+}
+// (b) What later phases read: X_jj (tilesX) and X_jj^T (tilesT), and the log-det / quadratic-form
+// partials.  `red` of step (a) must be complete (a block barrier in between).
+__device__ __forceinline__ void lg_diag_images(const LargeWs& w, int j, const double* S2,
+                                               const double* red) {
+  const int tid = threadIdx.x;
+  double* tx = lg_tile(w.tilesX, j, j);
+  double* tt = w.tilesT + (size_t)j * TT;
+  for (int idx = tid; idx < TT / 2; idx += NTHREADS) {
+    const int r = idx >> 5, c2 = (idx & 31) * 2;
+    double2 vv, vt;
+    vv.x = (c2 <= r) ? S2[r * LD_S + c2] : 0.0;
+    vv.y = (c2 + 1 <= r) ? S2[r * LD_S + c2 + 1] : 0.0;
+    vt.x = (r <= c2) ? S2[c2 * LD_S + r] : 0.0;
+    vt.y = (r <= c2 + 1) ? S2[(c2 + 1) * LD_S + r] : 0.0;
+    const int o = img(r, c2);
+    *reinterpret_cast<double2*>(tx + o) = vv;
+    *reinterpret_cast<double2*>(tt + o) = vt;
+  }
+  if (tid < 2) {
+    double s = 0.0;
+    for (int r = 0; r < TS; ++r) s += red[tid * TS + r];
+    w.ldz[2 * j + (tid ? 0 : 1)] = s;   // ldz[2j] = sum log L_kk, ldz[2j+1] = z_j^T z_j
+  }
+}
+
 constexpr size_t LG_DIAG_SMEM = (size_t)(2 * S_ELEMS + 4 * TS + 8) * sizeof(double);
 static __global__ void __launch_bounds__(NTHREADS) lg_diag(LargeArgs A, int j) {
   extern __shared__ __align__(16) double sm[];
@@ -428,43 +503,44 @@ static __global__ void __launch_bounds__(NTHREADS) lg_diag(LargeArgs A, int j) {
     if (tid == 0) atomicOr(v.st.fail + v.b, *s_fail);
     return;
   }
-  double* tx = lg_tile(w.tilesX, j, j);
-  double* tt = w.tilesT + (size_t)j * TT;
-  for (int idx = tid; idx < TT / 2; idx += NTHREADS) {
-    const int r = idx >> 5, c2 = (idx & 31) * 2;
-    double2 vv, vt;
-    vv.x = (c2 <= r) ? S2[r * LD_S + c2] : 0.0;
-    vv.y = (c2 + 1 <= r) ? S2[r * LD_S + c2 + 1] : 0.0;
-    vt.x = (r <= c2) ? S2[c2 * LD_S + r] : 0.0;
-    vt.y = (r <= c2 + 1) ? S2[(c2 + 1) * LD_S + r] : 0.0;
-    const int o = img(r, c2);
-    *reinterpret_cast<double2*>(tl + o) = vv;
-    *reinterpret_cast<double2*>(tx + o) = vv;
-    *reinterpret_cast<double2*>(tt + o) = vt;
-  }
-  {
-    const int r = tid >> 2, l4 = tid & 3;
-    double zz = 0.0;
-    for (int c = l4; c <= r; c += 4) zz += S2[r * LD_S + c] * zi[c];
-    zz += shfl_xor_d(zz, 1);
-    zz += shfl_xor_d(zz, 2);
-    if (l4 == 0) {
-      w.z[j * TS + r] = zz;
-      red[r] = zz * zz;
-      red[TS + r] = -log(dinv[r]);
-    }
-  }
+  lg_diag_solve(w, j, S2, zi, dinv, red);
   __syncthreads();
-  if (tid < 2) {
-    double s = 0.0;
-    for (int r = 0; r < TS; ++r) s += red[tid * TS + r];
-    w.ldz[2 * j + (tid ? 0 : 1)] = s;   // ldz[2j] = sum log L_kk, ldz[2j+1] = z_j^T z_j
-  }
+  lg_diag_images(w, j, S2, red);
 }
 
 // ------------------------------------------------------------------------------------
 // L_ij = C_ij X_jj^T for i > j;  rhs_i -= L_ij z_j
 // ------------------------------------------------------------------------------------
+// row t (< 64) of a [4][64] set of per-warp-column partials, summed in a fixed order
+__device__ __forceinline__ double lg_sum4(const double* red, int t) {
+  return (red[t] + red[TS + t]) + (red[2 * TS + t] + red[3 * TS + t]);
+}
+
+// L_ij = C X_jj^T (images of C in Cst, of X_jj in R), the row partials of L_ij z_j over the four
+// warp columns into red[4][64], and the bulk store of L_ij to `dst`, left in flight.  The barriers of
+// the store also publish `red`.
+__device__ __forceinline__ void lg_offdiag_solve(double* Cst, const double* R, const double* zj,
+                                                 double* red, double* dst) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int g = lane >> 2, tq = lane & 3, wm = warp >> 2, wn = warp & 3;
+  double acc[4][2][2];
+  zero_acc(acc);
+  compute_chunk<M_B_LE, false>(acc, Cst, R, 0, wm, wn, g, tq);
+  compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
+#pragma unroll
+  for (int mi = 0; mi < 4; ++mi) {
+    double s = 0.0;
+#pragma unroll
+    for (int ni = 0; ni < 2; ++ni)
+#pragma unroll
+      for (int e = 0; e < 2; ++e) s += acc[mi][ni][e] * zj[frag_col(wn, ni, tq, e)];
+    s += shfl_xor_d(s, 1);
+    s += shfl_xor_d(s, 2);
+    if (tq == 0) red[wn * TS + frag_row(wm, mi, g)] = s;
+  }
+  store_tile_bulk(acc, Cst, dst, 1.0);
+}
+
 constexpr size_t LG_TRSM_SMEM = (size_t)(4 * OPBUF + 5 * TS + 8) * sizeof(double);
 static __global__ void __launch_bounds__(NTHREADS, 2) lg_trsm(LargeArgs A, int j) {
   extern __shared__ __align__(16) double sm[];
@@ -473,8 +549,7 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_trsm(LargeArgs A, int j
   double* zj = R + 2 * OPBUF;
   double* red = zj + TS;   // [4][64]
   const unsigned bar = smem_u32(red + 4 * TS);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int g = lane >> 2, tq = lane & 3, wm = warp >> 2, wn = warp & 3;
+  const int tid = threadIdx.x;
   const LcView v = lc_view(A);
   const int i = j + 1 + blockIdx.x;
   if (v.st.state[v.b] != LG_ACTIVE || i >= v.N) return;
@@ -494,24 +569,8 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_trsm(LargeArgs A, int j
     bulk_g2s(smem_u32(R), lg_tile(w.tilesL, j, j), 2 * CHUNK_BYTES, bar);
   }
   mbar_wait(bar, 0);
-  double acc[4][2][2];
-  zero_acc(acc);
-  compute_chunk<M_B_LE, false>(acc, Cst, R, 0, wm, wn, g, tq);
-  compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
-#pragma unroll
-  for (int mi = 0; mi < 4; ++mi) {
-    double s = 0.0;
-#pragma unroll
-    for (int ni = 0; ni < 2; ++ni)
-#pragma unroll
-      for (int e = 0; e < 2; ++e) s += acc[mi][ni][e] * zj[frag_col(wn, ni, tq, e)];
-    s += shfl_xor_d(s, 1);
-    s += shfl_xor_d(s, 2);
-    if (tq == 0) red[wn * TS + frag_row(wm, mi, g)] = s;
-  }
-  store_tile_bulk(acc, Cst, tij, 1.0);   // barriers inside also publish `red`
-  if (tid < TS)
-    w.rhs[i * TS + tid] -= (red[tid] + red[TS + tid]) + (red[2 * TS + tid] + red[3 * TS + tid]);
+  lg_offdiag_solve(Cst, R, zj, red, tij);
+  if (tid < TS) w.rhs[i * TS + tid] -= lg_sum4(red, tid);
   if (tid == 0) bulk_wait_all();
 }
 
@@ -565,7 +624,6 @@ template <int KIND, int QT, int D>
 __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
   using C = Cfg<KIND, QT, D>;
   using L = CholAllSmem<KIND, QT, D>;
-  constexpr int DS = C::DS;
   extern __shared__ __align__(16) double sm[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, tq = lane & 3, wm = warp >> 2, wn = warp & 3;
@@ -600,22 +658,12 @@ __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
   const unsigned bars = smem_u32(par + C::PAR_BAR);
   const unsigned rbar = bars + 8 * 10;
   load_exp_tab(tab);
-  if (tid == 0) {   // mbarriers: 2-stage ring (full / empty) + the resident-tile barrier
-    for (int s = 0; s < 2; ++s) { mbar_init(bars + 8 * s, 1); mbar_init(bars + 8 * (2 + s), NTHREADS / 32); }
-    mbar_init(rbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    fence_proxy_async();
-    *s_fail = 0;
-  }
+  lg_ring_init(bars, rbar);
+  if (tid == 0) *s_fail = 0;
   __syncthreads();
   Ring r2{bars, bars + 16, stages, 0};
-  double wreg[QT], areg[QT * DS], lam[4];
-#pragma unroll
-  for (int q = 0; q < QT; ++q) wreg[q] = w.par[LG_PAR_WQ + q];
-#pragma unroll
-  for (int q = 0; q < QT * DS; ++q) areg[q] = w.par[LG_PAR_AQ + q];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) lam[q] = w.par[LG_PAR_LM + q];
+  LgConst<KIND, QT, D> kc;
+  kc.load(w.par);
   if (i == j) {
     // Diagonal job = the critical path of the factorisation (column j + 1 cannot start before it):
     // K~_jj (+ noise, jitter) does not depend on the operands this block is about to wait for, so it
@@ -632,13 +680,9 @@ __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
       const int r = frag_row(wm, mi, g), c0 = frag_col(wn, ni2, tq, 0);
       const int gi = i * TS + r;
 #pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        const int gj = j * TS + c0 + e;
-        double kv = k_entry<KIND, QT, D>(rowv, rowv, r, c0 + e, wreg, areg, lam, tab);
-        kv = (gi < n && gj <= gi) ? kv : 0.0;
-        if (gi == gj) kv = (gi < n) ? (kv + w.dn[gi] + jitter) : 1.0;
-        S[r * LD_S + c0 + e] = kv;
-      }
+      for (int e = 0; e < 2; ++e)
+        S[r * LD_S + c0 + e] = lg_k_masked<KIND, QT, D>(rowv, rowv, r, c0 + e, gi, j * TS + c0 + e, n,
+                                                        w.dn, jitter, kc.w, kc.a, kc.lam, tab);
     }
     __syncthreads();      // everyone is done with the fields in stage 0
   }
@@ -684,7 +728,9 @@ __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
     cp_async_commit();
     cp_async_wait<0>();
     __syncthreads();
-    // epilogue: C = K~_ij - acc, image in stage 1
+    // epilogue: C = K~_ij - acc, image in stage 1.  The entry is masked here rather than by
+    // lg_k_masked (i > j: no diagonal entry): with nvcc 12.9 its dead diagonal branch raises
+    // lg_chol_all<1,4,2> and <4,8,2> from 126 to 128 registers.
     store_acc_tile(acc, Cst, 1.0);
 #pragma unroll 1
     for (int p8 = 0; p8 < 8; ++p8) {
@@ -697,7 +743,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
 #pragma unroll
       for (int e = 0; e < 2; ++e) {
         const int gj = j * TS + c0 + e;
-        double kv = k_entry<KIND, QT, D>(rowv, colv, r, c0 + e, wreg, areg, lam, tab);
+        double kv = k_entry<KIND, QT, D>(rowv, colv, r, c0 + e, kc.w, kc.a, kc.lam, tab);
         kv = (gi < n && gj <= gi) ? kv : 0.0;
         o2[e] = kv - (e ? cv.y : cv.x);
       }
@@ -719,50 +765,12 @@ __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
     // What column j's other blocks wait for goes out FIRST (X_jj in the L array's diagonal slot and
     // z_j), then the flag; the copies later phases read (X_jj / X_jj^T for the inverse and the
     // gradient, the log-det / quadratic-form partials) follow behind the flag (r02y).
-    double* tl = lg_tile(w.tilesL, j, j);
-    if (ok) {
-      for (int idx = tid; idx < TT / 2; idx += NTHREADS) {
-        const int r = idx >> 5, c2 = (idx & 31) * 2;
-        double2 vv;
-        vv.x = (c2 <= r) ? S2[r * LD_S + c2] : 0.0;
-        vv.y = (c2 + 1 <= r) ? S2[r * LD_S + c2 + 1] : 0.0;
-        *reinterpret_cast<double2*>(tl + img(r, c2)) = vv;
-      }
-      {
-        const int r = tid >> 2, l4 = tid & 3;
-        double zz = 0.0;
-        for (int c = l4; c <= r; c += 4) zz += S2[r * LD_S + c] * zi[c];
-        zz += shfl_xor_d(zz, 1);
-        zz += shfl_xor_d(zz, 2);
-        if (l4 == 0) {
-          w.z[j * TS + r] = zz;
-          red2[r] = zz * zz;
-          red2[TS + r] = -log(dinv[r]);
-        }
-      }
-    }
+    if (ok) lg_diag_solve(w, j, S2, zi, dinv, red2);
     fence_proxy_async();   // the tile written above is read by bulk copies of other blocks
     __syncthreads();
     if (tid == 0) lg_set_flag(flag_of(j, j));
     if (ok) {
-      double* tx = lg_tile(w.tilesX, j, j);
-      double* tt = w.tilesT + (size_t)j * TT;
-      for (int idx = tid; idx < TT / 2; idx += NTHREADS) {
-        const int r = idx >> 5, c2 = (idx & 31) * 2;
-        double2 vv, vt;
-        vv.x = (c2 <= r) ? S2[r * LD_S + c2] : 0.0;
-        vv.y = (c2 + 1 <= r) ? S2[r * LD_S + c2 + 1] : 0.0;
-        vt.x = (r <= c2) ? S2[c2 * LD_S + r] : 0.0;
-        vt.y = (r <= c2 + 1) ? S2[(c2 + 1) * LD_S + r] : 0.0;
-        const int o = img(r, c2);
-        *reinterpret_cast<double2*>(tx + o) = vv;
-        *reinterpret_cast<double2*>(tt + o) = vt;
-      }
-      if (tid < 2) {
-        double s2 = 0.0;
-        for (int r = 0; r < TS; ++r) s2 += red2[tid * TS + r];
-        w.ldz[2 * j + (tid ? 0 : 1)] = s2;   // ldz[2j] = sum log L_kk, ldz[2j+1] = z_j^T z_j
-      }
+      lg_diag_images(w, j, S2, red2);
       fence_proxy_async();   // tilesX / tilesT are read by bulk copies of the following kernels
     }
     return;
@@ -779,24 +787,8 @@ __global__ void __launch_bounds__(NTHREADS, 2) lg_chol_all(LargeArgs A) {
   const bool failed = (*failp != 0);
   mbar_wait(rbar, 0);
   __syncthreads();
-  zero_acc(acc);
-  compute_chunk<M_B_LE, false>(acc, Cst, R, 0, wm, wn, g, tq);
-  compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
-#pragma unroll
-  for (int mi = 0; mi < 4; ++mi) {
-    double s = 0.0;
-#pragma unroll
-    for (int ni = 0; ni < 2; ++ni)
-#pragma unroll
-      for (int e = 0; e < 2; ++e) s += acc[mi][ni][e] * zj[frag_col(wn, ni, tq, e)];
-    s += shfl_xor_d(s, 1);
-    s += shfl_xor_d(s, 2);
-    if (tq == 0) red[wn * TS + frag_row(wm, mi, g)] = s;
-  }
-  store_tile_bulk(acc, Cst, lg_tile(w.tilesL, i, j), 1.0);   // its barriers also publish `red`
-  if (tid < TS && !failed)
-    w.fpart[((size_t)i * (i + 1) / 2 + j) * TS + tid] =
-        (red[tid] + red[TS + tid]) + (red[2 * TS + tid] + red[3 * TS + tid]);
+  lg_offdiag_solve(Cst, R, zj, red, lg_tile(w.tilesL, i, j));
+  if (tid < TS && !failed) w.fpart[((size_t)i * (i + 1) / 2 + j) * TS + tid] = lg_sum4(red, tid);
   __syncthreads();
   if (tid == 0) {
     bulk_wait_all();
@@ -855,14 +847,14 @@ __device__ __forceinline__ void lg_inv_partial(const double (&acc)[4][2][2], con
     if (tq == 0) red[wn * TS + frag_row(wm, mi, g)] = s;
   }
 }
-__device__ __forceinline__ void lg_inv_partial_store(double* __restrict__ dst, const double* red) {
-  const int tid = threadIdx.x;
-  if (tid < TS) dst[tid] = (red[tid] + red[TS + tid]) + (red[2 * TS + tid] + red[3 * TS + tid]);
-}
-
+// Tile (i, j), i > j, of X = L^-1 and its alpha partial.  `ready(kk)`: producer-thread hook run
+// before the operands of k-tile kk are loaded; `flags` (or null): the light curve's per-tile flags,
+// the tile's own is raised once the tile is stored.  The alpha partial is stored behind the flag (no
+// block of the launch reads it).
 constexpr size_t LG_INV_SMEM = (size_t)(6 * OPBUF + 16) * sizeof(double);
-static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_row(LargeArgs A, int i) {
-  extern __shared__ __align__(16) double sm[];
+template <typename FR>
+__device__ __forceinline__ void lg_inv_tile(double* sm, const LargeWs& w, int i, int j, FR ready,
+                                            int* flags) {
   double* stages = sm;
   double* Cst = stages + 2 * OPBUF;
   double* R = sm + 4 * OPBUF;
@@ -870,16 +862,7 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_row(LargeArgs A, in
   const unsigned rbar = bars + 8 * 4;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, tq = lane & 3, wm = warp >> 2, wn = warp & 3;
-  const LcView v = lc_view(A);
-  if (v.st.state[v.b] != LG_FACTORED || i >= v.N) return;
-  const LargeWs& w = v.w;
-  const int j = blockIdx.x;
-  if (tid == 0) {
-    for (int s = 0; s < 2; ++s) { mbar_init(bars + 8 * s, 1); mbar_init(bars + 8 * (2 + s), NTHREADS / 32); }
-    mbar_init(rbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    fence_proxy_async();
-  }
+  lg_ring_init(bars, rbar);
   __syncthreads();
   if (tid == 0) {
     mbar_expect_tx(rbar, 2 * CHUNK_BYTES);
@@ -891,7 +874,7 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_row(LargeArgs A, in
   auto tA = [&](int kk) { return kk == 0 ? w.tilesT + (size_t)j * TT : lg_tile(w.tilesX, j + kk, j); };
   auto tB = [&](int kk) { return lg_tile(w.tilesL, i, j + kk); };
   auto none = [&](int) { return (double*)nullptr; };
-  gemm_stream<M_A_GE, false, 2>(acc, r2, i - j, tA, tB, 0, 0, none, none, []() {});
+  gemm_stream_r<M_A_GE, false, 2>(acc, r2, i - j, tA, tB, 0, 0, none, none, []() {}, ready);
   __syncthreads();
   store_acc_tile(acc, Cst, 1.0);
   __syncthreads();
@@ -901,8 +884,18 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_row(LargeArgs A, in
   compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
   lg_inv_partial(acc, w.z + i * TS, stages, wm, wn, g, tq);
   store_tile_bulk(acc, Cst, lg_tile(w.tilesX, i, j), -1.0);   // its barriers also publish the partials
-  if (tid == 0) bulk_wait_all();
-  lg_inv_partial_store(w.fpart + ((size_t)i * (i + 1) / 2 + j) * TS, stages);
+  if (tid == 0) {
+    bulk_wait_all();
+    if (flags) lg_set_flag(flags + ((size_t)i * (i + 1) / 2 + j));
+  }
+  if (tid < TS) w.fpart[((size_t)i * (i + 1) / 2 + j) * TS + tid] = lg_sum4(stages, tid);
+}
+
+static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_row(LargeArgs A, int i) {
+  extern __shared__ __align__(16) double sm[];
+  const LcView v = lc_view(A);
+  if (v.st.state[v.b] != LG_FACTORED || i >= v.N) return;
+  lg_inv_tile(sm, v.w, i, (int)blockIdx.x, [](int) {}, nullptr);
 }
 
 // ------------------------------------------------------------------------------------
@@ -916,13 +909,6 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_row(LargeArgs A, in
 // ------------------------------------------------------------------------------------
 static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_all(LargeArgs A) {
   extern __shared__ __align__(16) double sm[];
-  double* stages = sm;
-  double* Cst = stages + 2 * OPBUF;
-  double* R = sm + 4 * OPBUF;
-  const unsigned bars = smem_u32(sm + 6 * OPBUF);
-  const unsigned rbar = bars + 8 * 4;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int g = lane >> 2, tq = lane & 3, wm = warp >> 2, wn = warp & 3;
   // tile-major block order (all light curves' tile t before any tile t + 1): in a batch the
   // blocks adjacent in dispatch order are independent, a single GP gets plain row-major order
   const unsigned job = lg_ticket(make_batch_state(A.ws, A.n_max, A.B).count + 2, sm);
@@ -932,25 +918,7 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_all(LargeArgs A) {
   tri_unrank((int)tix, i, j);   // (a, b), a >= b  ->  tile (a + 1, b)
   i += 1;
   if (v.st.state[v.b] != LG_FACTORED || i >= v.N) return;
-  const LargeWs& w = v.w;
   int* flags = v.st.tflag + (size_t)v.b * large_ntri(A.n_max);
-  if (tid == 0) {
-    for (int s = 0; s < 2; ++s) { mbar_init(bars + 8 * s, 1); mbar_init(bars + 8 * (2 + s), NTHREADS / 32); }
-    mbar_init(rbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    fence_proxy_async();
-  }
-  __syncthreads();
-  if (tid == 0) {
-    mbar_expect_tx(rbar, 2 * CHUNK_BYTES);
-    bulk_g2s(smem_u32(R), lg_tile(w.tilesX, i, i), 2 * CHUNK_BYTES, rbar);
-  }
-  Ring r2{bars, bars + 16, stages, 0};
-  double acc[4][2][2];
-  zero_acc(acc);
-  auto tA = [&](int kk) { return kk == 0 ? w.tilesT + (size_t)j * TT : lg_tile(w.tilesX, j + kk, j); };
-  auto tB = [&](int kk) { return lg_tile(w.tilesL, i, j + kk); };
-  auto none = [&](int) { return (double*)nullptr; };
   // producer thread only: X_{j+kk, j} must be final; the flag of k-tile kk + 1 is peeked one tile ahead
   int pk_k = -1, pk_v = 0;
   auto xflag = [&](int kk) { return flags + ((size_t)(j + kk) * (j + kk + 1) / 2 + j); };
@@ -964,21 +932,7 @@ static __global__ void __launch_bounds__(NTHREADS, 2) lg_inv_all(LargeArgs A) {
       pk_k = kk + 1;
     }
   };
-  gemm_stream_r<M_A_GE, false, 2>(acc, r2, i - j, tA, tB, 0, 0, none, none, []() {}, ready);
-  __syncthreads();
-  store_acc_tile(acc, Cst, 1.0);
-  __syncthreads();
-  mbar_wait(rbar, 0);
-  zero_acc(acc);
-  compute_chunk<M_B_LE, false>(acc, Cst, R, 0, wm, wn, g, tq);
-  compute_chunk<M_B_LE, false>(acc, Cst + OPBUF, R + OPBUF, KC / 8, wm, wn, g, tq);
-  lg_inv_partial(acc, w.z + i * TS, stages, wm, wn, g, tq);
-  store_tile_bulk(acc, Cst, lg_tile(w.tilesX, i, j), -1.0);   // its barriers also publish the partials
-  if (tid == 0) {
-    bulk_wait_all();
-    lg_set_flag(flags + ((size_t)i * (i + 1) / 2 + j));
-  }
-  lg_inv_partial_store(w.fpart + ((size_t)i * (i + 1) / 2 + j) * TS, stages);   // behind the flag
+  lg_inv_tile(sm, v.w, i, j, ready, flags);
 }
 
 // alpha_j = X_jj^T z_j + sum_{i>j} X_ij^T z_i   (tilesX holds X_jj and the X_ij^T tiles)
@@ -1026,7 +980,6 @@ __global__ void __launch_bounds__(NTHREADS, GradSmem<KIND, QT, D>::MIN_BLOCKS)
     lg_grad(LargeArgs A) {
   using C = Cfg<KIND, QT, D>;
   using L = GradSmem<KIND, QT, D>;
-  constexpr int DS = C::DS;
   static_assert(C::NV <= LG_GP, "gradient partial slot too small");
   extern __shared__ __align__(16) double sm[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1048,11 +1001,7 @@ __global__ void __launch_bounds__(NTHREADS, GradSmem<KIND, QT, D>::MIN_BLOCKS)
   double* tab = par + C::PAR_TAB;
   const unsigned bars = smem_u32(par + C::PAR_BAR);
   load_exp_tab(tab);
-  if (tid == 0) {   // mbarriers of the 2-stage ring (full / empty)
-    for (int s2 = 0; s2 < 2; ++s2) { mbar_init(bars + 8 * s2, 1); mbar_init(bars + 8 * (2 + s2), NTHREADS / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    fence_proxy_async();
-  }
+  lg_ring_init(bars);
   __syncthreads();
   Ring r2{bars, bars + 16, stages, 0};
   double acc[4][2][2];
@@ -1069,13 +1018,8 @@ __global__ void __launch_bounds__(NTHREADS, GradSmem<KIND, QT, D>::MIN_BLOCKS)
   if (i == j) gemm_stream<M_A_GE, true, 2>(acc, r2, N - i, tA, tB, 0, 0, none, none, pf);
   else gemm_stream<M_A_GE, false, 2>(acc, r2, N - i, tA, tB, 0, 0, none, none, pf);
   __syncthreads();
-  double wreg[QT], areg[QT * DS], lam[4];
-#pragma unroll
-  for (int q = 0; q < QT; ++q) wreg[q] = w.par[LG_PAR_WQ + q];
-#pragma unroll
-  for (int q = 0; q < QT * DS; ++q) areg[q] = w.par[LG_PAR_AQ + q];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) lam[q] = w.par[LG_PAR_LM + q];
+  LgConst<KIND, QT, D> kc;
+  kc.load(w.par);
   store_acc_tile(acc, R, 1.0);
   double ga[C::NG];
 #pragma unroll
@@ -1097,7 +1041,7 @@ __global__ void __launch_bounds__(NTHREADS, GradSmem<KIND, QT, D>::MIN_BLOCKS)
       W = (gi < n && gj <= gi) ? W : 0.0;
       if (gi == gj) trW += W;
       const double wgt = (gi == gj) ? W : 2.0 * W;
-      k_grad_entry<KIND, QT, D>(rowv, colv, r, c0 + e, wreg, areg, lam, tab, wgt, ga);
+      k_grad_entry<KIND, QT, D>(rowv, colv, r, c0 + e, kc.w, kc.a, kc.lam, tab, wgt, ga);
     }
   }
   double vv[C::NV];
@@ -1229,13 +1173,8 @@ __global__ void __launch_bounds__(NTHREADS, (Cfg<KIND, QT, D>::SMEM_BYTES <= 113
     const int n = A.n_valid ? A.n_valid[b] : A.n_max;
     const int N = (n + TS - 1) / TS, npad = N * TS;
     const LargeWs w = make_large_ws(A.ws + large_ws_elems(A.n_max) * (size_t)b, A.n_max);
-    double wreg[QT], areg[QT * DS], lam[4];
-#pragma unroll
-    for (int q = 0; q < QT; ++q) wreg[q] = w.par[LG_PAR_WQ + q];
-#pragma unroll
-    for (int q = 0; q < QT * DS; ++q) areg[q] = w.par[LG_PAR_AQ + q];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) lam[q] = w.par[LG_PAR_LM + q];
+    LgConst<KIND, QT, D> kc;
+    kc.load(w.par);
     const double* theta = w.par + LG_PAR_TH;
     // ---- test tile fields (centred on the light curve's first training input, as lg_setup).
     // Written out rather than through point_fields / param_layout: with nvcc 12.9 either form
@@ -1277,7 +1216,7 @@ __global__ void __launch_bounds__(NTHREADS, (Cfg<KIND, QT, D>::SMEM_BYTES <= 113
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
           const int gc = j * TS + c0 + e;
-          double k1 = k_entry<KIND, QT, D>(rowv, colv, r, c0 + e, wreg, areg, lam, tab);
+          double k1 = k_entry<KIND, QT, D>(rowv, colv, r, c0 + e, kc.w, kc.a, kc.lam, tab);
           k1 = (gc < n && t * TS + r < PA.m) ? k1 : 0.0;
           kv[e] = k1;
           mu[mi] += k1 * al_c[c0 + e];
@@ -1316,7 +1255,7 @@ __global__ void __launch_bounds__(NTHREADS, (Cfg<KIND, QT, D>::SMEM_BYTES <= 113
     if (tid < TS && t * TS + tid < PA.m) {
       const double m1 = (scr[tid] + scr[TS + tid]) + (scr[2 * TS + tid] + scr[3 * TS + tid]);
       const double v1 = (scr[4 * TS + tid] + scr[5 * TS + tid]) + (scr[6 * TS + tid] + scr[7 * TS + tid]);
-      const double kss = k_entry<KIND, QT, D>(rowv, rowv, tid, tid, wreg, areg, lam, tab);
+      const double kss = k_entry<KIND, QT, D>(rowv, rowv, tid, tid, kc.w, kc.a, kc.lam, tab);
       mean_out[t * TS + tid] = theta[0] + m1;
       var_out[t * TS + tid] = kss - v1;
     }

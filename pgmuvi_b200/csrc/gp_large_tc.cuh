@@ -361,6 +361,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) lg_grad_tc(LargeArgs A) {
     if (et < EXP_TAB) tab[et] = c_exp2_tab[et];
     tc_load_side<KIND, QT, D>(rowv, w, npad, N, I, et, true);
     tc_load_side<KIND, QT, D>(colv, w, npad, N, J, et, true);
+    // Not LgConst: with nvcc 12.9 it raises <0,8,1> / <2,4,2> from 176 to 200 B of stack and their
+    // spill stores / loads from 180 / 232 to 216 / 272 and 204 / 260 B.
     double wreg[QT], areg[QT * DS], lam[4];
 #pragma unroll
     for (int q = 0; q < QT; ++q) wreg[q] = w.par[LG_PAR_WQ + q];
@@ -499,6 +501,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
     const int et = tid - 64;
     const int q4 = warp & 3, half = (warp - 2) >> 2;
     const int r = 32 * q4 + lane;
+    // Not LgConst: with nvcc 12.9 it adds 12 to 16 B of spill loads to <0,4,1>, <1,4,2>, <2,4,2>.
     double wreg[QT], areg[QT * DS], lam[4];
     if (build) {
       if (et < EXP_TAB) tab[et] = c_exp2_tab[et];
@@ -535,13 +538,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
           if (build) {
             double k2[2];
 #pragma unroll
-            for (int u = 0; u < 2; ++u) {
-              const int gj = tj * TS + c0 + e + u;
-              double kk2 = k_entry<KIND, QT, D>(rv, cv, rr, c0 + e + u, wreg, areg, lam, tab);
-              kk2 = (gi < n && gj <= gi) ? kk2 : 0.0;
-              if (gi == gj) kk2 = (gi < n) ? (kk2 + w.dn[gi] + jitter) : 1.0;
-              k2[u] = kk2;
-            }
+            for (int u = 0; u < 2; ++u)
+              k2[u] = lg_k_masked<KIND, QT, D>(rv, cv, rr, c0 + e + u, gi, tj * TS + c0 + e + u, n, w.dn,
+                                               jitter, wreg, areg, lam, tab);
             o2 = make_double2(k2[0] - s0, k2[1] - s1);
           } else {
             o2 = *p;
