@@ -68,6 +68,49 @@ def power_slow(t, y, dy, freq, fit_mean=True, center_data=True):
     return out
 
 
+def power_exact(t, y, dy, freq, fit_mean=True, center_data=True, chunk=256):
+    """``power_slow`` restated in extended precision (``np.longdouble``, 64-bit mantissa on x86)
+    on ``t - t[0]``, vectorised over chunks of ``chunk`` frequencies.  The periodogram does not
+    depend on the time origin; shifting it in extended precision keeps the phases 2 pi f t exact
+    to ~1e-19 relative even for Julian dates (t ~ 2.45e6 d), where the fp64 ``power_slow`` loses
+    ~1e-10 in the power.  ``freq`` may itself be a longdouble array (e.g. ``f0 + k * df`` formed
+    without rounding to fp64).  About 0.7 us per (frequency, point) on one x86 core: sample the
+    grid rather than evaluating all of it for long light curves."""
+    L = np.longdouble
+    t = np.asarray(t, np.float64)
+    t = t.astype(L) - L(t[0])
+    y = np.asarray(y, np.float64).astype(L)
+    w = np.ones_like(y) if dy is None else np.asarray(dy, np.float64).astype(L) ** -2
+    w = w / w.sum()
+    if fit_mean or center_data:
+        y = y - np.dot(w, y)
+    wy, Y, YY = w * y, np.dot(w, y), np.dot(w, y * y)
+    two_pi = 2 * L("3.14159265358979323846264338327950288")
+    freq = np.asarray(freq).astype(L)
+    out = np.empty(freq.size, np.float64)
+    for s in range(0, freq.size, chunk):
+        ph = two_pi * freq[s:s + chunk, None] * t[None, :]
+        sn, cs = np.sin(ph), np.cos(ph)
+        S2 = 2 * ((sn * cs) @ w)
+        C2 = (cs * cs - sn * sn) @ w
+        if fit_mean:
+            S, C = sn @ w, cs @ w
+            S2 -= 2 * S * C
+            C2 -= C * C - S * S
+        arg = ph - 0.5 * np.arctan2(S2, C2)[:, None]
+        st, ct = np.sin(arg), np.cos(arg)
+        YC, YS = ct @ wy, st @ wy
+        CC, SS = (ct * ct) @ w, (st * st) @ w
+        if fit_mean:
+            Ct, St = ct @ w, st @ w
+            YC -= Y * Ct
+            YS -= Y * St
+            CC -= Ct * Ct
+            SS -= St * St
+        out[s:s + chunk] = ((YC * YC / CC + YS * YS / SS) / YY).astype(np.float64)
+    return out
+
+
 def top_peaks(power, distance, num_peaks):
     """find_peaks(power, distance=distance), sorted by height, first num_peaks
     (lightcurve.py:4531-4532, 4555)."""
@@ -106,19 +149,21 @@ def fdr_bh(fap_values, alpha=0.05):
     return res
 
 
-def multiband_power(t, y, bands, dy, freq):
+def multiband_power(t, y, bands, dy, freq, exact=False):
     """astropy ``LombScargleMultiband(t, y, bands, dy).power(freq, method='fast')`` restated
     (astropy/timeseries/periodograms/lombscargle_multiband/implementations/mbfast_impl.py, the
     ``ls_method`` default of pgmuvi/multiband_ls_significance.py:136): a floating-mean single-band
     periodogram per band, combined with the bands' reference chi-squares chi2_0b = sum w (y - ybar_w)^2
-    as weights.  astropy is absent from the image: parity with it is unpinned."""
+    as weights.  astropy is absent from the image: parity with it is unpinned.  ``exact``: each
+    band's power from ``power_exact`` (extended precision) instead of ``power_slow``."""
+    band_power = power_exact if exact else power_slow
     t, y, bands = (np.asarray(a) for a in (t, y, bands))
     dy = np.ones_like(t, dtype=np.float64) if dy is None else np.asarray(dy, np.float64)
     ub = np.unique(bands)
     powers, chi2 = [], []
     for b in ub:
         m = bands == b
-        powers.append(power_slow(t[m], y[m], dy[m], freq))
+        powers.append(band_power(t[m], y[m], dy[m], freq))
         w = dy[m] ** -2.0
         ybar = np.dot(w, y[m]) / w.sum()
         chi2.append(np.dot(w, (y[m] - ybar) ** 2))
