@@ -16,8 +16,11 @@
  *        0      Cholesky succeeded without jitter
  *        1..3   succeeded after adding jitter 1e-8*10^(k-1) (f64) / 1e-6*10^(k-1) (f32)
  *               to the diagonal (GPyTorch psd_safe_cholesky ladder, SURVEY.md A.5)
- *        -1     NaN encountered (GPyTorch NanError)
+ *        -1     NaN in K~ (GPyTorch NanError): a NaN in x, in the fixed noise or in a raw
+ *               parameter other than the mean, also when an earlier pivot is not positive
  *        -2     not positive definite after 3 jitter tries (GPyTorch NotPSDError)
+ *    A light curve with info < 0 has NaN mll and grad_raw, and alpha_out (where an entry point
+ *    has one) is NaN over [0, n_valid) and 0 beyond.
  *
  * Packed raw-parameter layout, P = 1 + Q + 2*Q*ds (+1 if PGM_FLAG_LEARN_NOISE) + NL:
  *     [ mean | w[0..Q) | mu[q*ds+k] | sigma[q*ds+k] | (learned noise) | lam[0..NL) ]

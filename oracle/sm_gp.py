@@ -269,8 +269,20 @@ def noise_diag(n, fixed_noise, learned_noise, dtype):
 # ---------------------------------------------------------------------------------------
 # Cholesky with GPyTorch's jitter ladder (A.5: linear_operator psd_safe_cholesky)
 # ---------------------------------------------------------------------------------------
-def psd_safe_cholesky(A, max_tries=3):
-    """Try plain; on failure add jitter*10^i (1e-6 fp32 / 1e-8 fp64) to failed members only.
+def default_jitter(dtype):
+    """First rung of the ladder: GPyTorch's cholesky_jitter, 1e-6 for float32 and 1e-8 for float64."""
+    return 1e-6 if dtype == torch.float32 else 1e-8
+
+
+def jitter_rung(info, jitter):
+    """Diagonal jitter that rung `info` (1..3) adds: jitter * 10^(info - 1)."""
+    return jitter * 10 ** (int(info) - 1)
+
+
+def psd_safe_cholesky(A, max_tries=3, jitter=None):
+    """Try plain; on failure add jitter*10^i to failed members only.  `jitter` is the first rung,
+    None: default_jitter(A.dtype).  jitter=1e-6 on float64 input gives the float32 ladder
+    (PGM_FLAG_JITTER_F32) in float64 arithmetic.
 
     Returns (L, info) with info[b] = 0 ok without jitter, k>0 = succeeded at jitter try k,
     -1 = NaN input (NanError), -2 = not PD after max_tries (NotPSDError).
@@ -282,7 +294,8 @@ def psd_safe_cholesky(A, max_tries=3):
     info_out[nan] = -1
     L, info = torch.linalg.cholesky_ex(Af)
     bad = (info > 0) & ~nan
-    jitter = 1e-6 if A.dtype == torch.float32 else 1e-8
+    if jitter is None:
+        jitter = default_jitter(A.dtype)
     prev = 0.0
     for i in range(max_tries):
         if not bad.any():
@@ -305,16 +318,17 @@ def psd_safe_cholesky(A, max_tries=3):
 # ---------------------------------------------------------------------------------------
 # exact MLL (A.5: ExactMarginalLogLikelihood.forward -> MVN.log_prob, per datum)
 # ---------------------------------------------------------------------------------------
-def _mll_from_theta(x, y, fixed_noise, theta, spec: ModelSpec):
+def _mll_from_theta(x, y, fixed_noise, theta, spec: ModelSpec, jitter=None):
     """Per-datum MLL from constrained theta.  x [n,d], y [n], theta [P]."""
     n = y.shape[-1]
+    if jitter is None:
+        jitter = default_jitter(y.dtype)
     mean, w, mu, sigma, noise = unpack_params(theta, spec)
     K = kernel_dense(x, x, theta, spec)
     Kt = K + torch.diag_embed(noise_diag(n, fixed_noise, noise, y.dtype))
-    L, info = psd_safe_cholesky(Kt.detach())
+    L, info = psd_safe_cholesky(Kt.detach(), jitter=jitter)
     if int(info) > 0:  # re-apply the jitter that made it succeed, keeping the graph
-        jitter = (1e-6 if y.dtype == torch.float32 else 1e-8) * 10 ** (int(info) - 1)
-        Kt = Kt + jitter * torch.eye(n, dtype=y.dtype)
+        Kt = Kt + jitter_rung(info, jitter) * torch.eye(n, dtype=y.dtype)
     if int(info) < 0:
         return torch.full((), float("nan"), dtype=y.dtype), info
     L = torch.linalg.cholesky(Kt)
@@ -326,12 +340,12 @@ def _mll_from_theta(x, y, fixed_noise, theta, spec: ModelSpec):
     return mll, info
 
 
-def mll_and_grad_autograd(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec):
+def mll_and_grad_autograd(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec, jitter=None):
     """One light curve through GPyTorch's op sequence with torch autograd
     (trainers.py:179-181).  Returns (mll, dmll/draw [P], info)."""
     raw = raw.detach().clone().requires_grad_(True)
     theta = constrain(raw, kinds, lb, ub)
-    mll, info = _mll_from_theta(x, y, fixed_noise, theta, spec)
+    mll, info = _mll_from_theta(x, y, fixed_noise, theta, spec, jitter)
     if int(info) < 0:
         return mll.detach(), torch.full_like(raw, float("nan")).detach(), info
     (g,) = torch.autograd.grad(mll, raw)
@@ -350,24 +364,25 @@ def constraint_jacobian(raw, kinds, lb, ub):
     return j
 
 
-def mll_and_grad_analytic(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec):
+def mll_and_grad_analytic(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec, jitter=None):
     """Same quantity via the closed form of A.5 (what the CUDA gradient kernel computes):
 
         W = alpha alpha^T - Kt^-1,  dMLL/dtheta = (1/2n) sum_ij W_ij dK_ij/dtheta,
         dMLL/dnoise = (1/2n) tr W,  dMLL/dc = (1/n) sum_i alpha_i,   then x Jacobian.
-    """
+
+    `jitter`: first rung of the Cholesky's jitter ladder (psd_safe_cholesky)."""
     dt = y.dtype
     n = y.shape[-1]
     Q, d = spec.Q, spec.ds
     if spec.kind >= KIND_STAT_BASE:
         # stationary kinds: the closed form is d K / d theta by autograd of the dense kernel,
         # contracted with W (the Cholesky part is still the explicit one below)
-        return _mll_and_grad_stat(x, y, fixed_noise, raw, kinds, lb, ub, spec)
+        return _mll_and_grad_stat(x, y, fixed_noise, raw, kinds, lb, ub, spec, jitter)
     theta = constrain(raw, kinds, lb, ub)
     mean, w, mu, sigma, noise = unpack_params(theta, spec)
     K = kernel_dense(x, x, theta, spec)
     Kt = K + torch.diag_embed(noise_diag(n, fixed_noise, noise, dt))
-    L, info = psd_safe_cholesky(Kt)
+    L, info = psd_safe_cholesky(Kt, jitter=jitter)
     if int(info) < 0:
         nanv = torch.full((), float("nan"), dtype=dt)
         return nanv, torch.full_like(raw, float("nan")), info
@@ -452,7 +467,7 @@ def mll_and_grad_analytic(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec
     return mll, g, info
 
 
-def _mll_and_grad_stat(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec):
+def _mll_and_grad_stat(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec, jitter=None):
     """mll_and_grad_analytic for the stationary kinds: W from the explicit Cholesky, then
     g_theta = (1/2n) sum_ij W_ij dK_ij/dtheta with dK/dtheta from autograd of kernel_dense."""
     dt = y.dtype
@@ -462,12 +477,14 @@ def _mll_and_grad_stat(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec):
     mean, w, mu, sigma, noise = unpack_params(theta, spec)
     K = kernel_dense(x, x, theta, spec)
     Kt = K + torch.diag_embed(noise_diag(n, fixed_noise, noise, dt))
-    L, info = psd_safe_cholesky(Kt.detach())
+    if jitter is None:
+        jitter = default_jitter(dt)
+    L, info = psd_safe_cholesky(Kt.detach(), jitter=jitter)
     if int(info) < 0:
         nanv = torch.full((), float("nan"), dtype=dt)
         return nanv, torch.full_like(raw, float("nan")), info
     if int(info) > 0:
-        Kt = Kt + 1e-8 * 10 ** (int(info) - 1) * torch.eye(n, dtype=dt)
+        Kt = Kt + jitter_rung(info, jitter) * torch.eye(n, dtype=dt)
     r = (y - mean.detach()).unsqueeze(-1)
     alpha = torch.cholesky_solve(r, L)
     Kinv = torch.cholesky_inverse(L)
@@ -482,7 +499,7 @@ def _mll_and_grad_stat(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec):
 # ---------------------------------------------------------------------------------------
 # N1: posterior prediction (GPyTorch ExactGP eval mode: ExactPredictionStrategy, exact form)
 # ---------------------------------------------------------------------------------------
-def predict(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec, xstar):
+def predict(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec, xstar, jitter=None):
     """Posterior mean and LATENT variance at xstar [m, d] (what ``model(x*)`` returns in eval
     mode, pgmuvi/lightcurve.py:9862; the likelihood then adds its homoskedastic noise):
         mean* = c + K*^T Kt^-1 (y - c),   var* = k** - K*^T Kt^-1 K*      (Cholesky solves).
@@ -492,7 +509,7 @@ def predict(x, y, fixed_noise, raw, kinds, lb, ub, spec: ModelSpec, xstar):
     theta = constrain(raw, kinds, lb, ub)
     mean, w, mu, sigma, noise = unpack_params(theta, spec)
     Kt = kernel_dense(x, x, theta, spec) + torch.diag_embed(noise_diag(n, fixed_noise, noise, y.dtype))
-    L, info = psd_safe_cholesky(Kt)
+    L, info = psd_safe_cholesky(Kt, jitter=jitter)
     Ks = kernel_dense(x, xstar, theta, spec)                    # [n, m]
     alpha = torch.cholesky_solve((y - mean).unsqueeze(-1), L)
     v = torch.linalg.solve_triangular(L, Ks, upper=False)
@@ -550,13 +567,21 @@ def adam_step(p, g, m, v, step, lr, b1=0.9, b2=0.999, eps=1e-8, weight_decay=0.0
 
 def train_loop(x, y, fixed_noise, raw0, kinds, lb, ub, spec: ModelSpec, maxiter=100,
                miniter=10, stop=None, lr=1e-4, optim="SGD", eps=1e-8, stopavg=9,
-               use_torch_optim=True):
+               use_torch_optim=True, jitter=None, on_failure="raise"):
     """trainers.py:167-209 restated for one light curve on packed raw parameters.
 
     Returns dict(loss=[...], delta_loss=[...], raw=[P-vectors, initial first]).  The loss
     recorded at iteration i is evaluated BEFORE that iteration's step (trainers.py:179-188);
     parameters are recorded AFTER it (trainers.py:190-192).
+
+    `jitter`: first rung of the Cholesky's jitter ladder (psd_safe_cholesky).
+    on_failure="raise" raises when an evaluation's Cholesky fails, as the reference does;
+    on_failure="stop" ends the loop there instead, the rule of the engine's fit kernel: the failed
+    evaluation's loss (NaN) is recorded and no step is taken.  The result then also has
+    info=[per-iteration Cholesky info].
     """
+    if on_failure not in ("raise", "stop"):
+        raise ValueError("on_failure must be 'raise' or 'stop'")
     raw = raw0.detach().clone().requires_grad_(True)
     if optim == "SGD":
         opt = torch.optim.SGD([raw], lr=lr)
@@ -567,11 +592,18 @@ def train_loop(x, y, fixed_noise, raw0, kinds, lb, ub, spec: ModelSpec, maxiter=
     else:
         raise ValueError("optim must be 'SGD', 'Adam' or 'AdamW'")
     res = {"loss": [], "delta_loss": [], "raw": [raw.detach().clone().numpy()]}
+    if on_failure == "stop":
+        res["info"] = []
     for i in range(maxiter):
         opt.zero_grad()
         theta = constrain(raw, kinds, lb, ub)
-        mll, info = _mll_from_theta(x, y, fixed_noise, theta, spec)
+        mll, info = _mll_from_theta(x, y, fixed_noise, theta, spec, jitter)
+        if on_failure == "stop":
+            res["info"].append(int(info))
         if int(info) < 0:
+            if on_failure == "stop":
+                res["loss"].append(np.array(float("nan")))
+                break
             raise RuntimeError(f"Cholesky failed (info={int(info)}) at iteration {i}")
         loss = -mll
         loss.backward()

@@ -1238,6 +1238,17 @@ __device__ __forceinline__ void point_fields(const double* x, int i, bool valid,
   }
 }
 
+// NaN among the D inputs of point i: K~ then has a NaN in row and column i.  The Cholesky only meets
+// it at a pivot, possibly after an earlier pivot has already failed; GPyTorch reports any NaN in K~
+// as a NaN failure (info -1) before it tries the ladder, so both engines record it up front.
+template <int D>
+__device__ __forceinline__ bool point_has_nan(const double* x, int i) {
+  bool r = false;
+#pragma unroll
+  for (int dd = 0; dd < D; ++dd) r |= isnan(x[(size_t)i * D + dd]);
+  return r;
+}
+
 // per-datum exact marginal log-likelihood -(y^T K~^-1 y + log |K~| + n log 2 pi) / (2 n)
 __device__ __forceinline__ double mll_value(double inv_quad, double logdet, int n) {
   return -0.5 * (inv_quad + logdet + (double)n * 1.8378770664093454836) / n;
@@ -1349,6 +1360,7 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   double* dinv = par + C::PAR_DINV;
   double* tab = par + C::PAR_TAB;
   int* s_fail = reinterpret_cast<int*>(sm + C::F_PAR + C::PAR_END);
+  int* s_nan = s_fail + 1;     // a NaN among the inputs of K~ (point_has_nan)
   const unsigned bars = smem_u32(par + C::PAR_BAR);
   const unsigned rbar = bars + 8 * 10;
   constexpr bool LEAN = C::LEAN;
@@ -1357,7 +1369,9 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   // ---- constraints: raw -> theta, d theta / d raw  (A.2) -----------------------------
   load_theta(A, b, P, raw, theta, jac);
   load_exp_tab(tab);
+  if (tid == 0) *s_nan = 0;
   __syncthreads();
+  if (tid >= 1 && tid < P && isnan(theta[tid])) *s_nan = 1;   // every slot but the mean is in K~
   kernel_constants<KIND, QT, D>(theta, Q, L, wq, aq, lamq);
   const double mean = theta[0];
   const double lnoise = learn_noise ? theta[L.o_noise] : 0.0;
@@ -1369,7 +1383,9 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
     const bool valid = i < n;
     point_fields<KIND, QT, D>(xb, i, valid, theta + L.o_mu, Q, sc.fx, sc.fcs, npad);
     sc.rhs[i] = valid ? (yb[i] - mean) : 0.0;
-    sc.dn[i] = valid ? ((fnb ? fnb[i] : 0.0) + lnoise) : 0.0;
+    const double dn = valid ? ((fnb ? fnb[i] : 0.0) + lnoise) : 0.0;
+    sc.dn[i] = dn;
+    if (valid && (isnan(dn) || point_has_nan<D>(xb, i))) *s_nan = 1;
   }
   __syncthreads();
 
@@ -1564,7 +1580,7 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
     __syncthreads();
     const int fl = *s_fail;
     if (!fl) { info = attempt; break; }
-    if (fl & 2) { info = -1; break; }
+    if ((fl & 2) || *s_nan) { info = -1; break; }
     info = -2;
     __syncthreads();
   }
@@ -1579,6 +1595,9 @@ __device__ int eval_lightcurve(const EvalArgs& A, int b, const double* raw, doub
   if (tid == 0) *mll_out = mll;
   if (!want_grad || info < 0) {
     if (want_grad && tid < P) grad_out[tid] = nan("");
+    if (A.alpha_out)   // info < 0 (alpha_out needs PGM_FLAG_GRAD): NaN like mll and grad
+      for (int i2 = tid; i2 < A.n_max; i2 += NTHREADS)
+        A.alpha_out[(size_t)b * A.n_max + i2] = (i2 < n) ? nan("") : 0.0;
     ps.gq2 = r2.gq;
     return info;
   }

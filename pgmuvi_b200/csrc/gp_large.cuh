@@ -44,6 +44,7 @@ struct BatchState {
   int *state;     // 0 = needs the P phase, 1 = factored, 2 = failed
   int *attempt;   // jitter rung 0..3
   int *fail;      // potrf failure bits of the current pass
+  int *nan_in;    // 1: a NaN among the inputs of K~ (lg_setup), so a failure is reported as -1
   int *count;     // light curves that must repeat the P phase
   int *tflag;     // [B, ntri(n_max)] "X tile is final" flags of the one-launch T phase
 };
@@ -60,14 +61,15 @@ __host__ __device__ inline size_t large_ntri(int n_max) {
 }
 __host__ __device__ inline size_t large_ws_bytes(int n_max, int B) {
   return large_ws_elems(n_max) * sizeof(double) * (size_t)B +
-         ((size_t)(3 * B + 4) + (size_t)B * large_ntri(n_max)) * sizeof(int);
+         ((size_t)(4 * B + 4) + (size_t)B * large_ntri(n_max)) * sizeof(int);
 }
 __host__ __device__ inline BatchState make_batch_state(double* base, int n_max, int B) {
   BatchState st;
   st.state = reinterpret_cast<int*>(base + large_ws_elems(n_max) * (size_t)B);
   st.attempt = st.state + B;
   st.fail = st.attempt + B;
-  st.count = st.fail + B;
+  st.nan_in = st.fail + B;
+  st.count = st.nan_in + B;
   st.tflag = st.count + 4;
   return st;
 }
@@ -153,6 +155,7 @@ __global__ void __launch_bounds__(NTHREADS) lg_setup(LargeArgs A) {
       w.par[LG_PAR_TH + tid] = theta[tid];
       w.par[LG_PAR_JC + tid] = jac[tid];
     }
+    if (tid >= 1 && tid < P && isnan(theta[tid])) v.st.nan_in[v.b] = 1;   // every slot but the mean
     kernel_constants<KIND, QT, D>(theta, Q, L, w.par + LG_PAR_WQ, w.par + LG_PAR_AQ,
                                   w.par + LG_PAR_LM);
   }
@@ -166,7 +169,9 @@ __global__ void __launch_bounds__(NTHREADS) lg_setup(LargeArgs A) {
   const double* fnb = A.fixed_noise ? A.fixed_noise + (size_t)v.b * A.n_max : nullptr;
   point_fields<KIND, QT, D>(xb, i, valid, theta + L.o_mu, Q, w.fx, w.fcs, npad);
   w.rhs[i] = valid ? (yb[i] - mean) : 0.0;
-  w.dn[i] = valid ? ((fnb ? fnb[i] : 0.0) + lnoise) : 0.0;
+  const double dn = valid ? ((fnb ? fnb[i] : 0.0) + lnoise) : 0.0;
+  w.dn[i] = dn;
+  if (valid && (isnan(dn) || point_has_nan<D>(xb, i))) v.st.nan_in[v.b] = 1;
 }
 
 // per-point data of tile row / col I -> rowv / colv (cp.async, as in the fused kernel)
@@ -806,7 +811,7 @@ static __global__ void lg_ladder(LargeArgs A) {
   if (!fl) {
     st.state[b] = LG_FACTORED;
     A.info[b] = st.attempt[b];
-  } else if (fl & 2) {
+  } else if ((fl & 2) || st.nan_in[b]) {   // a NaN in K~, possibly behind an earlier failed pivot
     st.state[b] = LG_FAILED;
     A.info[b] = -1;
   } else if (st.attempt[b] < 3) {
@@ -1071,6 +1076,9 @@ __global__ void __launch_bounds__(NTHREADS) lg_finish(LargeArgs A, int want_grad
   if (v.st.state[v.b] != LG_FACTORED) {
     if (tid == 0) *mll_out = nan("");
     if (want_grad && tid < P) grad_out[tid] = nan("");
+    if (want_grad && A.alpha_out)
+      for (int i2 = tid; i2 < A.n_max; i2 += NTHREADS)
+        A.alpha_out[(size_t)v.b * A.n_max + i2] = (i2 < n) ? nan("") : 0.0;
     return;
   }
   double vv[C::NV + 3];

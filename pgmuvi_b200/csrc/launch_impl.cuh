@@ -101,7 +101,7 @@ int launch_large(const pgm::LargeArgs& A, int want_grad, cudaStream_t st, int pr
   cudaFuncSetAttribute(lg_inv_row, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_INV_SMEM);
   cudaFuncSetAttribute(lg_inv_all, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_INV_SMEM);
   BatchState bs = make_batch_state(A.ws, n, B);
-  cudaMemsetAsync(bs.state, 0, (size_t)(3 * B + 4) * sizeof(int), st);
+  cudaMemsetAsync(bs.state, 0, (size_t)(4 * B + 4) * sizeof(int), st);
   const dim3 blk(NTHREADS);
   for (int pass = 0; pass <= 3; ++pass) {
     cudaMemsetAsync(bs.count, 0, 4 * sizeof(int), st);   // [0] repeat count, [1] / [2] job tickets

@@ -104,6 +104,60 @@ def test_jitter_ladder():
     assert psd_safe_cholesky(A)[1].tolist()[0] == -1
 
 
+def test_jitter_base_parameter():
+    """jitter=None keeps the ladder by dtype (1e-8 float64, 1e-6 float32); jitter=1e-6 on float64
+    input is the float32 ladder in float64 arithmetic: a member rescued at rung 3 of the float64
+    ladder (t = 3e-7) is rescued at rung 1 there, factored as A + 1e-6 I."""
+    A = torch.eye(4).repeat(4, 1, 1)
+    A[1, 3, 3] = -3e-9
+    A[2, 3, 3] = -3e-8
+    A[3, 3, 3] = -3e-7
+    L, info = psd_safe_cholesky(A)
+    L8, info8 = psd_safe_cholesky(A, jitter=1e-8)
+    assert info.tolist() == info8.tolist() == [0, 1, 2, 3] and torch.equal(L, L8)
+    L6, info6 = psd_safe_cholesky(A, jitter=1e-6)
+    assert info6.tolist() == [0, 1, 1, 1]
+    assert torch.equal(L6[3], torch.linalg.cholesky(A[3] + 1e-6 * torch.eye(4)))
+    assert psd_safe_cholesky(A.float())[1].tolist() == [0, 1, 1, 1]
+    assert psd_safe_cholesky(A, jitter=1e-6)[1].tolist() == psd_safe_cholesky(A.float())[1].tolist()
+
+
+@pytest.mark.parametrize("name", ["sm1d_n40_q4", "stat_matern_rbf_4x48"])
+def test_jitter_base_through_mll_and_predict(name):
+    """A light curve shifted to lambda_min(K~) = -3e-7: the default call is the float64 ladder's rung
+    3 and equals jitter=1e-8; with jitter=1e-6 it is rung 1, and the closed form (the stationary
+    kinds' _mll_and_grad_stat included), autograd, predict and train_loop all add 1e-6."""
+    from oracle import predict
+    from oracle.sm_gp import kernel_dense
+    x, y, nz, raw, kinds, lb, ub, spec = _case(load_golden(name), 0)
+    th = constrain(raw, kinds, lb, ub)
+    Kt = kernel_dense(x, x, th, spec) + torch.diag_embed(
+        noise_diag(len(y), nz, unpack_params(th, spec)[4], y.dtype))
+    nz = nz - float(torch.linalg.eigvalsh(Kt)[0]) - 3e-7
+    a = (x, y, nz, raw, kinds, lb, ub, spec)
+    m0, g0, i0 = mll_and_grad_analytic(*a)
+    m8, g8, i8 = mll_and_grad_analytic(*a, jitter=1e-8)
+    assert int(i0) == int(i8) == 3 and float(m0) == float(m8) and torch.equal(g0, g8)
+    m6, g6, i6 = mll_and_grad_analytic(*a, jitter=1e-6)
+    ma, ga, ia = mll_and_grad_autograd(*a, jitter=1e-6)
+    mj, gj, ij = mll_and_grad_analytic(x, y, nz + 1e-6, raw, kinds, lb, ub, spec)
+    assert int(i6) == int(ia) == 1 and int(ij) == 0
+    for m, gr in ((ma, ga), (mj, gj)):
+        assert abs(float(m6) - float(m)) <= 1e-10 * abs(float(m))
+        assert float((g6 - gr).abs().max()) <= 1e-8 * float(gr.abs().max())
+    xs = x[:5] + 0.01
+    p6 = predict(*a, xs, jitter=1e-6)
+    pj = predict(x, y, nz + 1e-6, raw, kinds, lb, ub, spec, xs)
+    assert int(p6[2]) == 1 and torch.allclose(p6[0], pj[0], rtol=1e-10)
+    r6 = train_loop(*a, maxiter=1, lr=1e-3, jitter=1e-6, on_failure="stop")
+    assert r6["info"] == [1] and len(r6["raw"]) == 2
+    with pytest.raises(RuntimeError, match="info=-2"):
+        train_loop(x, y, nz - 1.0, raw, kinds, lb, ub, spec, maxiter=2, jitter=1e-6)
+    r = train_loop(x, y, nz - 1.0, raw, kinds, lb, ub, spec, maxiter=3, jitter=1e-6,
+                   on_failure="stop")
+    assert r["info"] == [-2] and np.isnan(r["loss"][0]) and len(r["raw"]) == 1
+
+
 @pytest.mark.parametrize("decoupled,wd", [(False, 0.0), (True, 0.01)])
 def test_adam_step_matches_torch(decoupled, wd):
     p0 = torch.randn(7, generator=torch.Generator().manual_seed(1))
