@@ -347,6 +347,26 @@ int pgm_sm_psd_peak_f64(const double* freq, const double* fscale, const double* 
                         double* grid, double* psd, int32_t* dom_idx, double* dom_freq,
                         double* dom_height, int32_t* n_peaks, void* stream);
 
+/*
+ * Expected (Fisher) information of the exact Gaussian log-likelihood l = n * mll in the
+ * CONSTRAINED parameters theta (the standard errors of a fit): fisher [B, P, P] with
+ *   I_pq = 1/2 tr(K~^-1 dK~/dtheta_p K~^-1 dK~/dtheta_q)   (covariance slots p, q >= 1)
+ *   I_00 = 1^T K~^-1 1   (constant mean),   I_0p = 0.
+ * K~ includes the noise and the jitter rung its Cholesky needed (info, as the _staged entries:
+ * 0..3 the rung, -1 NaN, -2 not positive definite); rows of a light curve with info < 0 are NaN.
+ * Runs the P and T phases of the staged engine, then B_s = X dK_s X^T (X = L^-1) per used slot on
+ * the FP64 tile engine and the Gram matrix <B_p, B_q> in a fixed order (deterministic); about
+ * (P - 1) n^3 flops per light curve.  Same arguments as pgm_sm_mll_grad_staged_f64 (flags:
+ * PGM_FLAG_LEARN_NOISE / PGM_FLAG_BOUNDS_PER_LC / PGM_FLAG_JITTER_F32; B <= 65535); workspace =
+ * pgm_fisher_workspace_bytes(...) (0 for invalid arguments).  Blocking.
+ */
+size_t pgm_fisher_workspace_bytes(int n_max, int B, int d, int Q, int kernel_kind, int flags);
+int pgm_sm_fisher_f64(const double* x, const int32_t* n_valid, const double* y,
+                      const double* fixed_noise, const double* raw, const int32_t* con_kind,
+                      const double* con_lb, const double* con_ub, int B, int n_max, int d, int Q,
+                      int kernel_kind, int flags, double* fisher, int32_t* info, void* workspace,
+                      size_t workspace_bytes, void* stream);
+
 /* Device yardsticks used by bench.py for the self-measured FP64 roofline: runs `iters`
  * dependent-free FP64 DMMA (kind 0), FP64 DFMA (kind 1), FP32 FFMA (kind 2) or interleaved
  * DMMA+DFMA (kind 3, equal flops each) instructions per thread on every SM and returns the

@@ -51,6 +51,7 @@ EXPORTS = (
     "pgm_sm_psd_peak_f64",
     "pgm_staged_tf32x3_workspace_bytes", "pgm_sm_mll_grad_staged_tf32x3_f64",
     "pgm_sm_mll_grad_tf32x3_f32", "pgm_fused_grid",
+    "pgm_fisher_workspace_bytes", "pgm_sm_fisher_f64",
 )
 
 _lib = None
@@ -128,6 +129,11 @@ def load():
     lib.pgm_sm_psd_peak_f64.restype = c_int
     lib.pgm_sm_psd_peak_f64.argtypes = [dp, dp, dp, dp, dp, c_int, c_int, c_int, dp, dp, ip, dp, dp,
                                         ip, vp]
+    lib.pgm_fisher_workspace_bytes.restype = c_size_t
+    lib.pgm_fisher_workspace_bytes.argtypes = [c_int] * 6
+    lib.pgm_sm_fisher_f64.restype = c_int
+    lib.pgm_sm_fisher_f64.argtypes = [dp, ip, dp, dp, dp, ip, dp, dp, c_int, c_int, c_int, c_int,
+                                      c_int, c_int, dp, ip, vp, c_size_t, vp]
     lib.pgm_peak_probe.restype = c_int
     lib.pgm_peak_probe.argtypes = [c_int, c_int, POINTER(c_double), vp]
     _lib = lib

@@ -212,6 +212,40 @@ def gather_results(local: torch.Tensor, counts=None):
     return torch.cat([o[:c] for o, c in zip(out, counts)], 0)
 
 
+def _pack_batch(lcs, packs, who):
+    """Pad and pack set-up light curves of one model family into host float64 buffers
+    ``(x [B, n_max, d], y [B, n_max], noise [B, n_max] or None, raw, lb, ub [B, P], n_valid [B])``
+    (padding beyond ``n_valid``: zeros, unit noise)."""
+    pk0 = packs[0]
+    for pk in packs[1:]:
+        if (pk.kind, pk.Q, pk.d, pk.learn_noise, pk.P) != (pk0.kind, pk0.Q, pk0.d, pk0.learn_noise,
+                                                        pk0.P) or not torch.equal(pk.kinds,
+                                                                                  pk0.kinds):
+            raise ValueError(f"{who}: all light curves must share one model family, number "
+                             "of mixtures and likelihood type")
+    B = len(lcs)
+    n_each = [int(lc._ydata_transformed.shape[0]) for lc in lcs]
+    n_max = max(n_each)
+    d, P = pk0.d, pk0.P
+    x = torch.zeros(B, n_max, d, dtype=torch.float64)
+    y = torch.zeros(B, n_max, dtype=torch.float64)
+    has_fixed = pk0.fixed_noise is not None
+    noise = torch.ones(B, n_max, dtype=torch.float64) if has_fixed else None
+    raw = torch.zeros(B, P, dtype=torch.float64)
+    lb = torch.zeros(B, P, dtype=torch.float64)
+    ub = torch.zeros(B, P, dtype=torch.float64)
+    for b, (lc, pk) in enumerate(zip(lcs, packs)):
+        n = n_each[b]
+        xt = lc._xdata_transformed.detach().to(torch.float64)
+        x[b, :n] = xt if xt.dim() > 1 else xt.unsqueeze(-1)
+        y[b, :n] = lc._ydata_transformed.detach().to(torch.float64)
+        if has_fixed:
+            noise[b, :n] = pk.fixed_noise.detach().to(torch.float64)
+        raw[b] = pk.raw().detach().to(torch.float64)
+        lb[b], ub[b] = pk.lb, pk.ub
+    return x, y, noise, raw, lb, ub, torch.tensor(n_each, dtype=torch.int32)
+
+
 def fit_batch(lightcurves, model="1D", likelihood=None, num_mixtures=None, periods=None,
               use_mls_init=False, constraint_set=None, training_iter=300, optim="AdamW",
               miniter=None, stop=1e-5, lr=0.1, stopavg=30, variance=False, keep_history=True,
@@ -295,36 +329,12 @@ def fit_batch(lightcurves, model="1D", likelihood=None, num_mixtures=None, perio
         raise UnsupportedModelError(
             f"fit_batch: model {model!r} has a non-constant mean function, whose parameters are "
             "optimised on the host; fit these light curves one by one with Lightcurve.fit")
-    for pk in packs[1:]:
-        if (pk.kind, pk.Q, pk.d, pk.learn_noise, pk.P) != (pk0.kind, pk0.Q, pk0.d, pk0.learn_noise,
-                                                        pk0.P) or not torch.equal(pk.kinds,
-                                                                                  pk0.kinds):
-            raise ValueError("fit_batch: all light curves must share one model family, number "
-                             "of mixtures and likelihood type")
     # ---- pack the (ragged) batch ----------------------------------------------------------
-    n_each = [int(lc._ydata_transformed.shape[0]) for lc in lcs]
-    n_max = max(n_each)
-    if n_max > 2048:
+    x, y, noise, raw, lb, ub, n_valid = _pack_batch(lcs, packs, "fit_batch")
+    if x.shape[1] > 2048:
         raise ValueError("fit_batch: light curves longer than 2048 points go through "
                          "Lightcurve.fit (staged whole-device engine)")
-    d, P = pk0.d, pk0.P
-    x = torch.zeros(B, n_max, d, dtype=torch.float64)
-    y = torch.zeros(B, n_max, dtype=torch.float64)
-    has_fixed = pk0.fixed_noise is not None
-    noise = torch.ones(B, n_max, dtype=torch.float64) if has_fixed else None
-    raw = torch.zeros(B, P, dtype=torch.float64)
-    lb = torch.zeros(B, P, dtype=torch.float64)
-    ub = torch.zeros(B, P, dtype=torch.float64)
-    for b, (lc, pk) in enumerate(zip(lcs, packs)):
-        n = n_each[b]
-        xt = lc._xdata_transformed.detach().to(torch.float64)
-        x[b, :n] = xt if xt.dim() > 1 else xt.unsqueeze(-1)
-        y[b, :n] = lc._ydata_transformed.detach().to(torch.float64)
-        if has_fixed:
-            noise[b, :n] = pk.fixed_noise.detach().to(torch.float64)
-        raw[b] = pk.raw().detach().to(torch.float64)
-        lb[b], ub[b] = pk.lb, pk.ub
-    n_valid = torch.tensor(n_each, dtype=torch.int32)
+    P = pk0.P
     # ---- shard, fit, gather ----------------------------------------------------------------
     distributed = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
     world = dist.get_world_size() if distributed else 1
@@ -385,3 +395,97 @@ def fit_batch(lightcurves, model="1D", likelihood=None, num_mixtures=None, perio
         if summ is not None:
             out["dominant_period"] = summ["dominant_period"]
     return out
+
+
+def uncertainties_batch(lightcurves, device=None, budget_bytes=None):
+    """:meth:`Lightcurve.parameter_uncertainties` for many set-up (usually fitted) light curves of
+    one model family: the ragged batch is packed as ``fit_batch`` packs it and the Fisher matrices
+    come from ``pgm_sm_fisher_f64`` in chunks whose workspace (``pgm_fisher_workspace_bytes``)
+    stays within ``budget_bytes`` (default: 80 % of the free device memory).  Returns one dict per
+    light curve, in order."""
+    from . import mll
+    from .mll import UnsupportedModelError, pack_model
+
+    lcs = list(lightcurves)
+    if not lcs:
+        raise ValueError("uncertainties_batch needs at least one light curve")
+    packs = [pack_model(lc.model, lc.likelihood) for lc in lcs]
+    if any(pk.external_mean for pk in packs):
+        raise UnsupportedModelError("parameter uncertainties: models with a non-constant mean "
+                                    "function are not supported")
+    x, y, noise, raw, lb, ub, n_valid = _pack_batch(lcs, packs, "uncertainties_batch")
+    pk0 = packs[0]
+    B, n_max = y.shape
+    dev = torch.device(device) if device is not None else mll.engine_device(pk0.params[0])
+    if budget_bytes is None:
+        budget_bytes = int(0.8 * torch.cuda.mem_get_info(dev)[0]) if dev.type == "cuda" else 1 << 62
+    per_lc = ops.fisher_workspace_bytes(n_max, 2, pk0.d, pk0.Q, pk0.kind, pk0.learn_noise) - \
+        ops.fisher_workspace_bytes(n_max, 1, pk0.d, pk0.Q, pk0.kind, pk0.learn_noise)
+    chunk = int(max(1, min(65535, budget_bytes // max(per_lc, 1))))
+    fisher = torch.empty(B, pk0.P, pk0.P, dtype=torch.float64)
+    info = torch.empty(B, dtype=torch.int32)
+    to = lambda t, a, z: None if t is None else t[a:z].contiguous().to(dev)
+    for a in range(0, B, chunk):
+        z = min(B, a + chunk)
+        f, i = ops.sm_fisher(to(x, a, z), to(y, a, z), to(noise, a, z), to(raw, a, z),
+                             pk0.kinds.to(dev), to(lb, a, z), to(ub, a, z), to(n_valid, a, z),
+                             pk0.kind, pk0.Q, pk0.learn_noise)
+        fisher[a:z], info[a:z] = f.cpu(), i.cpu()
+    return [_uncertainties(lc, pk, fisher[b], int(info[b])) for b, (lc, pk) in
+            enumerate(zip(lcs, packs))]
+
+
+def _uncertainties(lc, pk, fisher, info):
+    """Host assembly of one light curve: free-slot inverse of the Fisher matrix, then the delta
+    method through ``Lightcurve._report`` (autograd) for every ``get_parameters`` entry."""
+    from ._lib import CON_INTERVAL
+    P = pk.P
+    names, owner = [], []
+    for i, (p, nm) in enumerate(zip(pk.params, pk.names)):
+        k = p.numel()
+        names += [nm if k == 1 else f"{nm}[{j}]" for j in range(k)]
+        owner += [i] * k
+    frozen = torch.tensor([pk.names[owner[s]] == "?" or (int(pk.kinds[s]) == CON_INTERVAL and
+                                                         float(pk.lb[s]) == float(pk.ub[s]))
+                           for s in range(P)])
+    free = ~frozen
+    Ff = fisher[free][:, free]
+    dg = Ff.diagonal()
+    ok = bool(torch.isfinite(Ff).all()) and bool((dg > 0).all())
+    cov = torch.zeros(P, P, dtype=torch.float64)
+    if ok:
+        sc = dg.rsqrt()
+        L, inf = torch.linalg.cholesky_ex(Ff * sc[:, None] * sc[None, :])
+        ok = int(inf) == 0
+        if ok:
+            cf = torch.cholesky_inverse(L) * sc[:, None] * sc[None, :]
+    idx = torch.nonzero(free).flatten()
+    cov[idx[:, None], idx[None, :]] = cf if ok else float("nan")
+    stderr, o = {}, {}
+    pos = 0
+    for i, p in enumerate(pk.params):
+        o[id(p)] = (pos, p.numel())
+        pos += p.numel()
+    for name, param in lc.model.named_parameters():
+        key = ".".join(c.lstrip("raw_") for c in name.split(".")) if "raw" in name else name
+        ent = lc._model_pars.get(key)
+        con = ent["module"]._modules.get(ent["raw_name"] + "_constraint") if ent else None
+        theta = (con.transform(param) if con is not None else param).detach().to(torch.float64)
+        shape = lc._report(key, theta).shape       # get_parameters' shape (transforms broadcast)
+        if id(param) not in o:
+            stderr[key] = torch.zeros(shape, dtype=torch.float64)
+            continue
+        a, k = o[id(param)]
+        J = torch.autograd.functional.jacobian(
+            lambda th: lc._report(key, th.reshape(param.shape)).reshape(-1).to(torch.float64),
+            theta.reshape(-1))
+        var = torch.einsum("ij,jk,ik->i", J, cov[a:a + k, a:a + k], J)
+        stderr[key] = var.clamp_min(0).sqrt().reshape(shape) if ok else \
+            torch.full(shape, float("nan"), dtype=torch.float64)
+    period_stderr = None
+    mk = next((k for k in stderr if k.endswith("mixture_means")), None)
+    if mk is not None:
+        mu = lc.get_parameters()[mk].detach().to(torch.float64)
+        period_stderr = (stderr[mk][:, 0, 0] / mu[:, 0, 0] ** 2).numpy()
+    return {"names": names, "covariance": cov, "stderr": stderr, "period_stderr": period_stderr,
+            "fisher_ok": ok, "fisher": fisher, "info": info}

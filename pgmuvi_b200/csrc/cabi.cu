@@ -3,6 +3,7 @@
 #include "gp_fused.cuh"
 #include "gp_large.cuh"
 #include "gp_large_tc.cuh"
+#include "gp_fisher.cuh"
 #include "lombscargle.cuh"
 #include "../../include/pgmuvi_b200.h"
 
@@ -20,6 +21,8 @@ template <int KIND, int QT, int D> int launch_dense(const EvalArgs& A, double* K
 template <int KIND, int QT, int D>
 int launch_large(const LargeArgs& A, int want_grad, cudaStream_t st, int predict_only);
 template <int KIND, int QT, int D> int launch_predict(const PredictArgs& PA, cudaStream_t st);
+template <int KIND, int QT, int D>
+int launch_fisher(const LargeArgs& A, const FisherArgs& F, cudaStream_t st);
 
 thread_local std::string g_err;
 int fail(const std::string& m) {
@@ -76,6 +79,7 @@ using pgm::launch_eval;
 using pgm::launch_fit;
 using pgm::launch_large;
 using pgm::launch_predict;
+using pgm::launch_fisher;
 
 int pad_q(int Q) { return Q <= 1 ? 1 : Q <= 2 ? 2 : Q <= 4 ? 4 : 8; }
 
@@ -410,6 +414,43 @@ int pgm_sm_predict_f64(const double* x, const int32_t* n_valid, const double* y,
   PA.kscratch = reinterpret_cast<double*>(static_cast<char*>(workspace) + staged);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   PGM_DISPATCH(launch_predict, PA, st);
+  return 0;
+}
+
+size_t pgm_fisher_workspace_bytes(int n_max, int B, int d, int Q, int kernel_kind, int flags) {
+  if (n_max < 1 || B < 1 || check_common(B, n_max, d, Q, kernel_kind)) return 0;
+  return pgm::fisher_ws_bytes(n_max, B, host_param_count(d, Q, kernel_kind, flags) - 1);
+}
+
+int pgm_sm_fisher_f64(const double* x, const int32_t* n_valid, const double* y,
+                      const double* fixed_noise, const double* raw, const int32_t* con_kind,
+                      const double* con_lb, const double* con_ub, int B, int n_max, int d, int Q,
+                      int kernel_kind, int flags, double* fisher, int32_t* info, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  if (B == 0) return 0;
+  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !fisher || !info || !workspace)
+    return fail("null pointer argument");
+  if (B > 65535) return fail("pgm_sm_fisher_f64: B > 65535 (split the batch)");
+  const int nc = host_param_count(d, Q, kernel_kind, flags) - 1;
+  if (nc < 1 || nc > pgm::FS_NC_MAX) return fail("pgm_sm_fisher_f64: unsupported parameter count");
+  const long long N = (n_max + pgm::TS - 1) / pgm::TS, ntri = N * (N + 1) / 2;
+  if (ntri * nc > 2147483647LL) return fail("pgm_sm_fisher_f64: n_max too large (tiles x carriers)");
+  if (workspace_bytes < pgm_fisher_workspace_bytes(n_max, B, d, Q, kernel_kind, flags))
+    return fail("workspace too small (see pgm_fisher_workspace_bytes)");
+  pgm::LargeArgs A;
+  A.x = x; A.n_valid = n_valid; A.y = y; A.fixed_noise = fixed_noise; A.raw = raw;
+  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
+  A.B = B; A.n_max = n_max; A.Q = Q;
+  A.flags = flags & (PGM_FLAG_LEARN_NOISE | PGM_FLAG_BOUNDS_PER_LC | PGM_FLAG_JITTER_F32);
+  A.mll = nullptr; A.grad = nullptr; A.info = info;
+  A.ws = static_cast<double*>(workspace);
+  A.alpha_out = nullptr;
+  pgm::FisherArgs F;
+  F.nc = nc;
+  F.fisher = fisher;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  PGM_DISPATCH(launch_fisher, A, F, st);
   return 0;
 }
 

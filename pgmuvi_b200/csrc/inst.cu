@@ -7,4 +7,6 @@ template int launch_fit<PGM_INST_KIND, PGM_INST_QT, PGM_INST_D>(const FitArgs&, 
 template int launch_dense<PGM_INST_KIND, PGM_INST_QT, PGM_INST_D>(const EvalArgs&, double*, cudaStream_t);
 template int launch_large<PGM_INST_KIND, PGM_INST_QT, PGM_INST_D>(const LargeArgs&, int, cudaStream_t, int);
 template int launch_predict<PGM_INST_KIND, PGM_INST_QT, PGM_INST_D>(const PredictArgs&, cudaStream_t);
+template int launch_fisher<PGM_INST_KIND, PGM_INST_QT, PGM_INST_D>(const LargeArgs&, const FisherArgs&,
+                                                                  cudaStream_t);
 }  // namespace pgm

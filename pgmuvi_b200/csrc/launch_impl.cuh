@@ -4,6 +4,7 @@
 #include "gp_fused.cuh"
 #include "gp_large.cuh"
 #include "gp_large_tc.cuh"
+#include "gp_fisher.cuh"
 #include <algorithm>
 #include <cstdlib>
 #include <string>
@@ -212,6 +213,37 @@ int launch_predict(const pgm::PredictArgs& PA0, cudaStream_t st) {
   kern<<<grid, NTHREADS, C::SMEM_BYTES, st>>>(PA);
   e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail("lg_predict launch", e);
+  return 0;
+}
+
+// Fisher information = P + T phases of the staged engine (X = L^-1, row-major in tilesL), then one
+// launch per stage of gp_fisher.cuh.  The caller has checked the grid sizes (pgm_sm_fisher_f64).
+template <int KIND, int QT, int D>
+int launch_fisher(const pgm::LargeArgs& A, const pgm::FisherArgs& F, cudaStream_t st) {
+  using namespace pgm;
+  if (int r = launch_large<KIND, QT, D>(A, 0, st, 1)) return r;
+  const int N = (A.n_max + TS - 1) / TS, ntri = N * (N + 1) / 2, B = A.B;
+  auto k_car = fs_carriers<KIND, QT, D>;
+  constexpr size_t CAR_SMEM = FsCarrierSmem<KIND, QT, D>::BYTES;
+  cudaError_t e = cudaFuncSetAttribute(k_car, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAR_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(fs_xc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_PROD_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(fs_xcx, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_PROD_SMEM);
+  if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute(fisher kernels)", e);
+  const dim3 blk(NTHREADS);
+  k_car<<<dim3(ntri, B), blk, CAR_SMEM, st>>>(A, F);
+  if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail("fs_carriers launch", e);
+  fs_xc<<<dim3((unsigned)(ntri * F.nc), B), blk, FS_PROD_SMEM, st>>>(A, F);
+  if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail("fs_xc launch", e);
+  fs_xcx<<<dim3((unsigned)(ntri * F.nc), B), blk, FS_PROD_SMEM, st>>>(A, F);
+  if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail("fs_xcx launch", e);
+  fs_gram<<<dim3(ntri, B), blk, 0, st>>>(A, F);
+  if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail("fs_gram launch", e);
+  fs_ones<<<dim3(N, B), blk, 0, st>>>(A, F);
+  if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail("fs_ones launch", e);
+  fs_finish<KIND, QT, D><<<dim3(1, B), blk, 0, st>>>(A, F);
+  if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail("fs_finish launch", e);
   return 0;
 }
 

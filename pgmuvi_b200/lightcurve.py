@@ -327,14 +327,32 @@ class Lightcurve(torch.nn.Module):
                 val = (con.transform(param) if con is not None else param).data
             else:
                 key, val = name, param.data
-            if transform and self.xtransform is not None and any(
-                    p in key for p in ("mixture_means", "mixture_scales")):
-                val = 1 / self.xtransform.inverse(1 / val, shift=False)
-            elif transform and self.ytransform is not None and any(
-                    p in key for p in ("noise", "mean_module")):
-                val = self.ytransform.inverse(val)
-            pars[key] = val
+            pars[key] = self._report(key, val) if transform else val
         return pars
+
+    def _report(self, key, val):
+        """The x / y transforms ``get_parameters`` applies to the constrained value of ``key``."""
+        if self.xtransform is not None and any(p in key for p in ("mixture_means", "mixture_scales")):
+            return 1 / self.xtransform.inverse(1 / val, shift=False)
+        if self.ytransform is not None and any(p in key for p in ("noise", "mean_module")):
+            return self.ytransform.inverse(val)
+        return val
+
+    def parameter_uncertainties(self, device=None):
+        """Standard errors of the fitted hyper-parameters from the exact Fisher information of the
+        Gaussian log-likelihood (``pgm_sm_fisher_f64``, evaluated at the current parameters).
+
+        Returns ``{"names", "covariance", "stderr", "period_stderr", "fisher_ok", "fisher",
+        "info"}``: ``names`` / ``covariance`` / ``fisher`` per packed slot (constrained values, the
+        inverse Fisher matrix over the free slots, 0 for frozen ones); ``stderr`` keyed and shaped
+        like ``get_parameters()`` and in its units (delta method through the same transforms);
+        ``period_stderr = stderr(mu) / mu^2`` per spectral-mixture component (time dimension, raw
+        units) or None.  Frozen slots (an ``Interval(lb, lb)``, values that are not Parameters)
+        get 0.  If the Fisher matrix of the free slots is not positive definite, ``stderr`` is
+        NaN and ``fisher_ok`` False.  Models with a non-constant mean raise
+        ``UnsupportedModelError``."""
+        from .batch import uncertainties_batch
+        return uncertainties_batch([self], device=device)[0]
 
     def get_periods(self):
         """Periods ``1/mu`` (time dimension), mixture weights and scales ``1/(2 pi sigma)`` in the

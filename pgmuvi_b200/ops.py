@@ -377,6 +377,46 @@ def sm_mll_grad_large(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: 
     return mll[0], grad[0], (info[0] if nosync else int(info.item()))
 
 
+@torch.library.custom_op("pgmuvi_b200::sm_fisher", mutates_args=(), device_types="cuda")
+def sm_fisher(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor, con_kind: Tensor,
+              con_lb: Tensor, con_ub: Tensor, n_valid: Optional[Tensor], kind: int, Q: int,
+              learn_noise: bool) -> Tuple[Tensor, Tensor]:
+    """Expected (Fisher) information of the exact log-likelihood ``n * mll`` in the constrained
+    parameters, ``fisher [B, P, P]``, and the Cholesky ``info [B]`` (``pgm_sm_fisher_f64``: the
+    staged engine's P and T phases, then the Fisher kernels).  Rows of a light curve with
+    ``info < 0`` are NaN.  float64 only; blocking."""
+    (x, y, fixed_noise, raw, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
+        x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    if x.dtype != torch.float64:
+        raise RuntimeError("sm_fisher takes float64 tensors")
+    fisher = torch.empty(B, P, P, dtype=x.dtype, device=x.device)
+    info = torch.zeros(B, dtype=torch.int32, device=x.device)
+    if n_valid is not None:
+        n_valid = n_valid.to(torch.int32).contiguous()
+    lib = _lib.load()
+    # not cached between calls: a batch's workspace can take most of the device memory
+    ws = torch.empty(lib.pgm_fisher_workspace_bytes(n, B, d, Q, kind, flags), dtype=torch.uint8,
+                     device=x.device)
+    with torch.cuda.device(x.device):
+        check(lib.pgm_sm_fisher_f64(
+            ptr(x), ptr(n_valid), ptr(y), ptr(fixed_noise), ptr(raw), ptr(con_kind), ptr(con_lb),
+            ptr(con_ub), B, n, d, Q, kind, flags, ptr(fisher), ptr(info), ptr(ws), ws.numel(),
+            _stream()))
+    return fisher, info
+
+
+@sm_fisher.register_fake
+def _(x, y, fixed_noise, raw, con_kind, con_lb, con_ub, n_valid, kind, Q, learn_noise):
+    B, P = raw.shape
+    return y.new_empty(B, P, P), y.new_empty(B, dtype=torch.int32)
+
+
+def fisher_workspace_bytes(n_max: int, B: int, d: int, Q: int, kind: int, learn_noise: bool) -> int:
+    """Device bytes one :func:`sm_fisher` call of B light curves of up to n_max points needs."""
+    return int(_lib.load().pgm_fisher_workspace_bytes(n_max, B, d, Q, kind,
+                                                      FLAG_LEARN_NOISE if learn_noise else 0))
+
+
 def peak_probe(kind: int, iters: int = 4096) -> float:
     """Self-measured FP64 DMMA (0) / DFMA (1) / FP32 FFMA (2) throughput in TFLOP/s."""
     import ctypes
@@ -385,6 +425,6 @@ def peak_probe(kind: int, iters: int = 4096) -> float:
     return out.value
 
 
-__all__ = ["sm_mll_grad", "sm_mll_grad_alpha", "sm_mll_grad_large", "sm_mll_grad_staged", "sm_predict", "sm_kernel_dense", "optim_step", "sm_fit",
+__all__ = ["sm_mll_grad", "sm_fisher", "sm_mll_grad_alpha", "sm_mll_grad_large", "sm_mll_grad_staged", "sm_predict", "sm_kernel_dense", "optim_step", "sm_fit",
            "peak_probe", "param_count",
            "KIND_SM1D", "KIND_SM_ARD_PRODSUM", "KIND_SM_ARD_SUMPROD"]
