@@ -35,24 +35,66 @@ def stat_num_lam(kind):
     return (2, 2, 4, 6, 2, 2)[tk] + (0, 2, 2, 3, 1)[wk]
 
 
+def param_count(Q: int, d: int, learn_noise: bool, kind: int = -1) -> int:
+    """P of the packed layout ``[mean | w | mu | sigma | (noise) | lam]`` (pgmuvi_b200.h)."""
+    if is_stat(kind):            # stationary time kernels: no mixtures (Q = 0)
+        return 1 + (1 if learn_noise else 0) + stat_num_lam(kind)
+    if kind in SEP_KINDS:
+        return 1 + 3 * Q + (1 if learn_noise else 0) + NUM_LAM[kind]
+    return 1 + Q + 2 * Q * d + (1 if learn_noise else 0)
+
+
 CON_NONE, CON_SOFTPLUS, CON_INTERVAL, CON_RSOFTPLUS = 0, 1, 2, 3
 FLAG_GRAD, FLAG_LEARN_NOISE, FLAG_BOUNDS_PER_LC, FLAG_JITTER_F32, FLAG_TF32X3, FLAG_TF32X3_CHOL, FLAG_NOSYNC = (
     1, 2, 4, 8, 16, 32, 64)
 OPT_SGD, OPT_ADAM, OPT_ADAMW = 0, 1, 2
 
-EXPORTS = (
-    "pgm_version", "pgm_last_error", "pgm_workspace_bytes", "pgm_sm_mll_grad_f64",
-    "pgm_sm_kernel_dense_f64", "pgm_optim_step_f64", "pgm_sm_fit_f64", "pgm_peak_probe",
-    "pgm_staged_workspace_bytes", "pgm_sm_mll_grad_staged_f64",
-    "pgm_predict_workspace_bytes", "pgm_sm_predict_f64",
-    "pgm_f32_staging_bytes", "pgm_sm_mll_grad_f32", "pgm_sm_fit_f32",
-    "pgm_lombscargle_f64", "pgm_ls_peaks_f64",
-    "pgm_sm_mll_grad_alpha_f64", "pgm_sm_mll_grad_staged_alpha_f64",
-    "pgm_sm_psd_peak_f64",
-    "pgm_staged_tf32x3_workspace_bytes", "pgm_sm_mll_grad_staged_tf32x3_f64",
-    "pgm_sm_mll_grad_tf32x3_f32", "pgm_fused_grid",
-    "pgm_fisher_workspace_bytes", "pgm_sm_fisher_f64",
-)
+# every exported symbol: name -> (restype, argtypes); device pointers travel as integers
+_dp = _ip = _vp = c_void_p
+_MLL_GRAD = [_dp, _ip, _dp, _dp, _dp, _ip, _dp, _dp, c_int, c_int, c_int, c_int, c_int, c_int,
+             _dp, _dp, _ip, _vp, c_size_t, _vp]
+_MLL_GRAD_ALPHA = [_dp, _ip, _dp, _dp, _dp, _ip, _dp, _dp, c_int, c_int, c_int, c_int, c_int,
+                   c_int, _dp, _dp, _dp, _ip, _vp, c_size_t, _vp]
+_FIT = [_dp, _ip, _dp, _dp, _dp, _ip, _dp, _dp, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+        c_double, c_double, c_double, c_double, c_double, c_int, c_int, c_double, c_int, _dp, _dp,
+        _ip, _ip]
+PROTOTYPES = {
+    "pgm_version": (c_int, []),
+    "pgm_last_error": (c_char_p, []),
+    "pgm_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
+    "pgm_sm_mll_grad_f64": (c_int, _MLL_GRAD),
+    "pgm_sm_kernel_dense_f64": (c_int, [_dp, _ip, _dp, _dp, _ip, _dp, _dp, c_int, c_int, c_int,
+                                        c_int, c_int, c_int, _dp, _vp]),
+    "pgm_optim_step_f64": (c_int, [_dp, _dp, _dp, _dp, _ip, c_int, c_int, c_int, c_double,
+                                   c_double, c_double, c_double, c_double, c_int, _vp]),
+    "pgm_sm_fit_f64": (c_int, _FIT + [_dp, _vp, c_size_t, _vp]),
+    "pgm_peak_probe": (c_int, [c_int, c_int, POINTER(c_double), _vp]),
+    "pgm_staged_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "pgm_sm_mll_grad_staged_f64": (c_int, _MLL_GRAD),
+    "pgm_predict_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "pgm_sm_predict_f64": (c_int, [_dp, _ip, _dp, _dp, _dp, _ip, _dp, _dp, c_int, c_int, c_int,
+                                   c_int, c_int, c_int, _dp, c_int, _dp, _dp, _ip, _vp, c_size_t,
+                                   _vp]),
+    "pgm_f32_staging_bytes": (c_size_t, [c_int] * 8),
+    "pgm_sm_mll_grad_f32": (c_int, _MLL_GRAD),
+    "pgm_sm_fit_f32": (c_int, _FIT + [_vp, c_size_t, _vp]),
+    "pgm_lombscargle_f64": (c_int, [_dp, _ip, _dp, _dp, c_int, c_int, _dp, _dp, _ip, c_int, c_int,
+                                    _dp, _vp]),
+    "pgm_ls_peaks_f64": (c_int, [_dp, _ip, c_int, c_int, c_int, c_int, _ip, _dp, _vp, c_size_t,
+                                 _vp]),
+    "pgm_sm_mll_grad_alpha_f64": (c_int, _MLL_GRAD_ALPHA),
+    "pgm_sm_mll_grad_staged_alpha_f64": (c_int, _MLL_GRAD_ALPHA),
+    "pgm_sm_psd_peak_f64": (c_int, [_dp, _dp, _dp, _dp, _dp, c_int, c_int, c_int, _dp, _dp, _ip,
+                                    _dp, _dp, _ip, _vp]),
+    "pgm_staged_tf32x3_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "pgm_sm_mll_grad_staged_tf32x3_f64": (c_int, _MLL_GRAD),
+    "pgm_sm_mll_grad_tf32x3_f32": (c_int, _MLL_GRAD),
+    "pgm_fused_grid": (c_int, [c_int, c_int, c_int]),
+    "pgm_fisher_workspace_bytes": (c_size_t, [c_int] * 6),
+    "pgm_sm_fisher_f64": (c_int, [_dp, _ip, _dp, _dp, _dp, _ip, _dp, _dp, c_int, c_int, c_int,
+                                  c_int, c_int, c_int, _dp, _ip, _vp, c_size_t, _vp]),
+}
+EXPORTS = tuple(PROTOTYPES)
 
 _lib = None
 
@@ -71,71 +113,10 @@ def load():
             f"{LIB_PATH} not found: build it with `python -m pgmuvi_b200.build` "
             "(pgmuvi_b200 has no CPU fallback)")
     lib = ctypes.CDLL(LIB_PATH)
-    dp, ip, vp = c_void_p, c_void_p, c_void_p  # device pointers travel as integers
-    lib.pgm_version.restype = c_int
-    lib.pgm_last_error.restype = c_char_p
-    lib.pgm_workspace_bytes.restype = c_size_t
-    lib.pgm_workspace_bytes.argtypes = [c_int, c_int, c_int, c_int, c_int]
-    lib.pgm_sm_mll_grad_f64.restype = c_int
-    lib.pgm_sm_mll_grad_f64.argtypes = [dp, ip, dp, dp, dp, ip, dp, dp, c_int, c_int, c_int,
-                                        c_int, c_int, c_int, dp, dp, ip, vp, c_size_t, vp]
-    lib.pgm_sm_kernel_dense_f64.restype = c_int
-    lib.pgm_sm_kernel_dense_f64.argtypes = [dp, ip, dp, dp, ip, dp, dp, c_int, c_int, c_int,
-                                            c_int, c_int, c_int, dp, vp]
-    lib.pgm_optim_step_f64.restype = c_int
-    lib.pgm_optim_step_f64.argtypes = [dp, dp, dp, dp, ip, c_int, c_int, c_int, c_double,
-                                       c_double, c_double, c_double, c_double, c_int, vp]
-    lib.pgm_sm_fit_f64.restype = c_int
-    lib.pgm_sm_fit_f64.argtypes = [dp, ip, dp, dp, dp, ip, dp, dp, c_int, c_int, c_int, c_int,
-                                   c_int, c_int, c_int, c_double, c_double, c_double, c_double,
-                                   c_double, c_int, c_int, c_double, c_int, dp, dp, ip, ip, dp,
-                                   vp, c_size_t, vp]
-    lib.pgm_staged_workspace_bytes.restype = c_size_t
-    lib.pgm_staged_workspace_bytes.argtypes = [c_int, c_int]
-    lib.pgm_sm_mll_grad_staged_f64.restype = c_int
-    lib.pgm_sm_mll_grad_staged_f64.argtypes = lib.pgm_sm_mll_grad_f64.argtypes
-    lib.pgm_fused_grid.restype = c_int
-    lib.pgm_fused_grid.argtypes = [c_int, c_int, c_int]
-    lib.pgm_staged_tf32x3_workspace_bytes.restype = c_size_t
-    lib.pgm_staged_tf32x3_workspace_bytes.argtypes = [c_int, c_int]
-    lib.pgm_sm_mll_grad_staged_tf32x3_f64.restype = c_int
-    lib.pgm_sm_mll_grad_staged_tf32x3_f64.argtypes = lib.pgm_sm_mll_grad_f64.argtypes
-    lib.pgm_sm_mll_grad_tf32x3_f32.restype = c_int
-    lib.pgm_sm_mll_grad_tf32x3_f32.argtypes = lib.pgm_sm_mll_grad_f64.argtypes
-    lib.pgm_predict_workspace_bytes.restype = c_size_t
-    lib.pgm_predict_workspace_bytes.argtypes = [c_int, c_int, c_int]
-    lib.pgm_sm_predict_f64.restype = c_int
-    lib.pgm_sm_predict_f64.argtypes = [dp, ip, dp, dp, dp, ip, dp, dp, c_int, c_int, c_int, c_int,
-                                       c_int, c_int, dp, c_int, dp, dp, ip, vp, c_size_t, vp]
-    lib.pgm_f32_staging_bytes.restype = c_size_t
-    lib.pgm_f32_staging_bytes.argtypes = [c_int] * 8
-    lib.pgm_sm_mll_grad_f32.restype = c_int
-    lib.pgm_sm_mll_grad_f32.argtypes = lib.pgm_sm_mll_grad_f64.argtypes
-    lib.pgm_sm_fit_f32.restype = c_int
-    lib.pgm_sm_fit_f32.argtypes = [dp, ip, dp, dp, dp, ip, dp, dp, c_int, c_int, c_int, c_int,
-                                   c_int, c_int, c_int, c_double, c_double, c_double, c_double,
-                                   c_double, c_int, c_int, c_double, c_int, dp, dp, ip, ip,
-                                   vp, c_size_t, vp]
-    lib.pgm_lombscargle_f64.restype = c_int
-    lib.pgm_lombscargle_f64.argtypes = [dp, ip, dp, dp, c_int, c_int, dp, dp, ip, c_int, c_int,
-                                        dp, vp]
-    lib.pgm_ls_peaks_f64.restype = c_int
-    lib.pgm_ls_peaks_f64.argtypes = [dp, ip, c_int, c_int, c_int, c_int, ip, dp, vp, c_size_t, vp]
-    lib.pgm_sm_mll_grad_alpha_f64.restype = c_int
-    lib.pgm_sm_mll_grad_alpha_f64.argtypes = [dp, ip, dp, dp, dp, ip, dp, dp, c_int, c_int, c_int,
-                                              c_int, c_int, c_int, dp, dp, dp, ip, vp, c_size_t, vp]
-    lib.pgm_sm_mll_grad_staged_alpha_f64.restype = c_int
-    lib.pgm_sm_mll_grad_staged_alpha_f64.argtypes = lib.pgm_sm_mll_grad_alpha_f64.argtypes
-    lib.pgm_sm_psd_peak_f64.restype = c_int
-    lib.pgm_sm_psd_peak_f64.argtypes = [dp, dp, dp, dp, dp, c_int, c_int, c_int, dp, dp, ip, dp, dp,
-                                        ip, vp]
-    lib.pgm_fisher_workspace_bytes.restype = c_size_t
-    lib.pgm_fisher_workspace_bytes.argtypes = [c_int] * 6
-    lib.pgm_sm_fisher_f64.restype = c_int
-    lib.pgm_sm_fisher_f64.argtypes = [dp, ip, dp, dp, dp, ip, dp, dp, c_int, c_int, c_int, c_int,
-                                      c_int, c_int, dp, ip, vp, c_size_t, vp]
-    lib.pgm_peak_probe.restype = c_int
-    lib.pgm_peak_probe.argtypes = [c_int, c_int, POINTER(c_double), vp]
+    for name, (restype, argtypes) in PROTOTYPES.items():
+        fn = getattr(lib, name)
+        fn.restype = restype
+        fn.argtypes = argtypes
     _lib = lib
     return lib
 

@@ -9,6 +9,7 @@ from __future__ import annotations
 
 import hashlib
 import os
+import re
 import subprocess
 import sys
 from concurrent.futures import ThreadPoolExecutor
@@ -25,14 +26,10 @@ NVCC_FLAGS = [
     # -lineinfo); the driver inflates it when the module is loaded
     "-Xfatbin=-compress-all", "--compress-mode=size",
 ]
-# (KIND, QT, D) instantiations: 1-D SM, 2-D ARD product-of-sums, 2-D sum-of-products
-CONFIGS = [(k, q, d) for (k, d) in ((0, 1), (1, 2), (2, 2)) for q in (1, 2, 4, 8)]
-# separable SM(time) x {RBF, Matern-1.5, RQ, Constant}(wavelength): QT in {4, 8}
-CONFIGS += [(k, q, 2) for k in (3, 4, 5, 6) for q in (4, 8)]
-# stationary time kernels (N3): kind = 8 + 5 * TK + WK, TK in {RBF, Matern-1.5, quasi-periodic}, WK = 0 -> 1-D
-CONFIGS += [(8 + 5 * tk + wk, 4, 1 if wk == 0 else 2) for tk in (0, 1, 2) for wk in range(5)]
-CONFIGS += [(23, 4, 1)]   # quasi-periodic + RBF (PeriodicPlusStochasticGPModel), 1-D only
-CONFIGS += [(28, 4, 1), (33, 4, 1)]   # Matern-0.5 / Matern-2.5 (MaternGPModel nu), 1-D only
+# (KIND, QT, D) instantiations, listed once in csrc/configs.h
+with open(os.path.join(CSRC, "configs.h")) as _f:
+    CONFIGS = [tuple(map(int, c))
+               for c in re.findall(r"^PGM_CONFIG\((\d+), (\d+), (\d+)\)", _f.read(), re.M)]
 
 
 def _nvcc():

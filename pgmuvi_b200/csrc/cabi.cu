@@ -10,7 +10,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cmath>
-#include <cstring>
+#include <initializer_list>
 #include <string>
 
 namespace pgm {
@@ -81,84 +81,77 @@ using pgm::launch_large;
 using pgm::launch_predict;
 using pgm::launch_fisher;
 
-int pad_q(int Q) { return Q <= 1 ? 1 : Q <= 2 ? 2 : Q <= 4 ? 4 : 8; }
-
 // NF of the instantiated config serving (d, Q): sizes the workspace (upper bound over kinds)
-int nf_for(int d, int Q) { return d + 2 * d * pad_q(Q <= 4 ? 4 : Q) + 1; }  // Q = 0 -> QT = 4
+int nf_for(int d, int Q) { return d + 2 * d * (Q <= 4 ? 4 : 8) + 1; }  // Q = 0 -> QT = 4
 
-#define PGM_DISPATCH_Q(KIND, D, FN, ...)                     \
-  switch (pad_q(Q)) {                                        \
-    case 1: return FN<KIND, 1, D>(__VA_ARGS__);              \
-    case 2: return FN<KIND, 2, D>(__VA_ARGS__);              \
-    case 4: return FN<KIND, 4, D>(__VA_ARGS__);              \
-    default: return FN<KIND, 8, D>(__VA_ARGS__);             \
-  }
+// one row per compiled instantiation (configs.h): its launchers and the resident fused blocks per SM
+struct Config {
+  int kind, qt, d;
+  int (*eval)(const pgm::EvalArgs&, cudaStream_t);
+  int (*fit)(const pgm::FitArgs&, cudaStream_t);
+  int (*dense)(const pgm::EvalArgs&, double*, cudaStream_t);
+  int (*large)(const pgm::LargeArgs&, int, cudaStream_t, int);
+  int (*predict)(const pgm::PredictArgs&, cudaStream_t);
+  int (*fisher)(const pgm::LargeArgs&, const pgm::FisherArgs&, cudaStream_t);
+  int fused_blocks_per_sm;
+};
+#define PGM_CONFIG(KIND, QT, D)                                                              \
+  {KIND, QT, D, launch_eval<KIND, QT, D>, launch_fit<KIND, QT, D>, launch_dense<KIND, QT, D>, \
+   launch_large<KIND, QT, D>, launch_predict<KIND, QT, D>, launch_fisher<KIND, QT, D>,       \
+   pgm::Cfg<KIND, QT, D>::F_BYTES <= 113 * 1024 ? 2 : 1},
+const Config kConfigs[] = {
+#include "configs.h"
+};
+#undef PGM_CONFIG
 
-#define PGM_DISPATCH_Q48(KIND, D, FN, ...)                   \
-  if (Q <= 4) return FN<KIND, 4, D>(__VA_ARGS__);            \
-  return FN<KIND, 8, D>(__VA_ARGS__);
+const Config* reject(const char* why) {
+  fail(why);
+  return nullptr;
+}
 
-#define PGM_DISPATCH(FN, ...)                                                        \
-  do {                                                                               \
-    if (kernel_kind == PGM_KIND_SM1D) {                                              \
-      PGM_DISPATCH_Q(PGM_KIND_SM1D, 1, FN, __VA_ARGS__)                              \
-    } else if (kernel_kind == PGM_KIND_SM_ARD_PRODSUM) {                             \
-      PGM_DISPATCH_Q(PGM_KIND_SM_ARD_PRODSUM, 2, FN, __VA_ARGS__)                    \
-    } else if (kernel_kind == PGM_KIND_SM_ARD_SUMPROD) {                             \
-      PGM_DISPATCH_Q(PGM_KIND_SM_ARD_SUMPROD, 2, FN, __VA_ARGS__)                    \
-    } else if (kernel_kind == PGM_KIND_SEP_RBF) {                                    \
-      PGM_DISPATCH_Q48(PGM_KIND_SEP_RBF, 2, FN, __VA_ARGS__)                         \
-    } else if (kernel_kind == PGM_KIND_SEP_MATERN15) {                               \
-      PGM_DISPATCH_Q48(PGM_KIND_SEP_MATERN15, 2, FN, __VA_ARGS__)                    \
-    } else if (kernel_kind == PGM_KIND_SEP_RQ) {                                     \
-      PGM_DISPATCH_Q48(PGM_KIND_SEP_RQ, 2, FN, __VA_ARGS__)                          \
-    } else if (kernel_kind == PGM_KIND_SEP_CONST) {                                  \
-      PGM_DISPATCH_Q48(PGM_KIND_SEP_CONST, 2, FN, __VA_ARGS__)                       \
-    } else {                                                                         \
-      switch (kernel_kind) {                                                         \
-        case PGM_KIND_STAT(0, 0): return FN<PGM_KIND_STAT(0, 0), 4, 1>(__VA_ARGS__); \
-        case PGM_KIND_STAT(0, 1): return FN<PGM_KIND_STAT(0, 1), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(0, 2): return FN<PGM_KIND_STAT(0, 2), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(0, 3): return FN<PGM_KIND_STAT(0, 3), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(0, 4): return FN<PGM_KIND_STAT(0, 4), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(1, 0): return FN<PGM_KIND_STAT(1, 0), 4, 1>(__VA_ARGS__); \
-        case PGM_KIND_STAT(1, 1): return FN<PGM_KIND_STAT(1, 1), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(1, 2): return FN<PGM_KIND_STAT(1, 2), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(1, 3): return FN<PGM_KIND_STAT(1, 3), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(1, 4): return FN<PGM_KIND_STAT(1, 4), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(2, 0): return FN<PGM_KIND_STAT(2, 0), 4, 1>(__VA_ARGS__); \
-        case PGM_KIND_STAT(2, 1): return FN<PGM_KIND_STAT(2, 1), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(2, 2): return FN<PGM_KIND_STAT(2, 2), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(2, 3): return FN<PGM_KIND_STAT(2, 3), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(2, 4): return FN<PGM_KIND_STAT(2, 4), 4, 2>(__VA_ARGS__); \
-        case PGM_KIND_STAT(3, 0): return FN<PGM_KIND_STAT(3, 0), 4, 1>(__VA_ARGS__); \
-        case PGM_KIND_STAT(4, 0): return FN<PGM_KIND_STAT(4, 0), 4, 1>(__VA_ARGS__); \
-        default: return FN<PGM_KIND_STAT(5, 0), 4, 1>(__VA_ARGS__);                  \
-      }                                                                              \
-    }                                                                                \
-  } while (0)
-
-int check_common(int B, int n_max, int d, int Q, int kernel_kind) {
-  if (B < 0 || n_max < 1) return fail("B must be >= 0 and n_max >= 1");
+// Validates a model and returns the compiled instantiation that serves it: the row of its kind with
+// the smallest QT >= max(Q, 1).  Null (and pgm_last_error set) if the model is rejected.
+const Config* check_common(int B, int n_max, int d, int Q, int kernel_kind) {
+  if (B < 0 || n_max < 1) return reject("B must be >= 0 and n_max >= 1");
   if (kernel_kind >= PGM_KIND_STAT_BASE && kernel_kind <= PGM_KIND_STAT(5, 0)) {
-    if (Q != 0) return fail("stationary kinds have no mixtures: pass Q == 0");
+    if (Q != 0) return reject("stationary kinds have no mixtures: pass Q == 0");
     const int wk = (kernel_kind - PGM_KIND_STAT_BASE) % 5;
     if ((kernel_kind - PGM_KIND_STAT_BASE) / 5 >= 3 && wk != 0)
-      return fail("time kernels 3..5 exist for 1-D models only (wk = 0)");
-    if (d != (wk == 0 ? 1 : 2)) return fail("stationary kind / d mismatch (d = 1 without, 2 with a wavelength kernel)");
-    return 0;
-  }
-  if (Q < 1 || Q > 8) return fail("Q (num_mixtures) must be in 1..8");
-  if (kernel_kind == PGM_KIND_SM1D) {
-    if (d != 1) return fail("PGM_KIND_SM1D needs d == 1");
-  } else if (kernel_kind == PGM_KIND_SM_ARD_PRODSUM || kernel_kind == PGM_KIND_SM_ARD_SUMPROD) {
-    if (d != 2) return fail("ARD spectral-mixture kinds need d == 2");
-  } else if (kernel_kind >= PGM_KIND_SEP_RBF && kernel_kind <= PGM_KIND_SEP_CONST) {
-    if (d != 2) return fail("separable kinds need d == 2 (time, wavelength)");
+      return reject("time kernels 3..5 exist for 1-D models only (wk = 0)");
+    if (d != (wk == 0 ? 1 : 2))
+      return reject("stationary kind / d mismatch (d = 1 without, 2 with a wavelength kernel)");
   } else {
-    return fail("unknown kernel_kind");
+    if (Q < 1 || Q > 8) return reject("Q (num_mixtures) must be in 1..8");
+    if (kernel_kind == PGM_KIND_SM1D && d != 1) return reject("PGM_KIND_SM1D needs d == 1");
+    if ((kernel_kind == PGM_KIND_SM_ARD_PRODSUM || kernel_kind == PGM_KIND_SM_ARD_SUMPROD) && d != 2)
+      return reject("ARD spectral-mixture kinds need d == 2");
+    if (kernel_kind >= PGM_KIND_SEP_RBF && kernel_kind <= PGM_KIND_SEP_CONST && d != 2)
+      return reject("separable kinds need d == 2 (time, wavelength)");
   }
+  const Config* best = nullptr;
+  for (const Config& c : kConfigs)
+    if (c.kind == kernel_kind && c.qt >= std::max(Q, 1) && (!best || c.qt < best->qt)) best = &c;
+  return best ? best : reject("unknown kernel_kind");
+}
+
+int check_ptrs(std::initializer_list<const void*> ptrs) {
+  for (const void* p : ptrs)
+    if (!p) return fail("null pointer argument");
   return 0;
+}
+
+// the members EvalArgs and LargeArgs share: the model's inputs, its info output and the workspace
+template <typename Args>
+Args model_args(const double* x, const int32_t* n_valid, const double* y,
+                const double* fixed_noise, const double* raw, const int32_t* con_kind,
+                const double* con_lb, const double* con_ub, int B, int n_max, int Q, int flags,
+                int32_t* info, void* workspace) {
+  Args A{};
+  A.x = x; A.n_valid = n_valid; A.y = y; A.fixed_noise = fixed_noise; A.raw = raw;
+  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
+  A.B = B; A.n_max = n_max; A.Q = Q; A.flags = flags;
+  A.info = info; A.ws = static_cast<double*>(workspace);
+  return A;
 }
 
 
@@ -168,6 +161,17 @@ int host_param_count(int d, int Q, int kernel_kind, int flags) {
 }
 
 size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// the fused kernels' workspace (pgm_workspace_bytes): per-block scratch, then the light-curve
+// ticket counters at its tail
+int fused_ws(pgm::EvalArgs& A, int d, size_t workspace_bytes) {
+  const size_t need = pgm_workspace_bytes(8, A.n_max, d, A.Q, -1);
+  if (workspace_bytes < need) return fail("workspace too small (see pgm_workspace_bytes)");
+  A.ws_per_block = pgm::scratch_elems(A.n_max, nf_for(d, A.Q));
+  A.sched = reinterpret_cast<int*>(reinterpret_cast<char*>(A.ws) + need -
+                                   pgm::PGM_SCHED_INTS * sizeof(int));
+  return 0;
+}
 
 // fp64 staging area of the _f32 entry points, carved from the tail of the workspace
 struct Stage32 {
@@ -192,24 +196,55 @@ Stage32 carve32(char* base, int B, int n_max, int d, int P, bool bounds_per_lc, 
   s.bytes = off;
   return s;
 }
-int widen(const float* src, double* dst, size_t n, cudaStream_t st) {
-  if (!n) return 0;
+void widen(const float* src, double* dst, size_t n, cudaStream_t st) {
+  if (!n || !src) return;
   const int blocks = (int)std::min<size_t>((n + 255) / 256, 148 * 8);
   pgm::widen_kernel<<<blocks, 256, 0, st>>>(src, dst, n);
-  return 0;
 }
-int narrow(const double* src, float* dst, size_t n, cudaStream_t st) {
-  if (!n) return 0;
+void narrow(const double* src, float* dst, size_t n, cudaStream_t st) {
+  if (!n || !dst) return;
   const int blocks = (int)std::min<size_t>((n + 255) / 256, 148 * 8);
   pgm::narrow_kernel<<<blocks, 256, 0, st>>>(src, dst, n);
-  return 0;
 }
 
-template <int KIND, int QT, int D>
-int fused_blocks_per_sm() { return pgm::Cfg<KIND, QT, D>::F_BYTES <= 113 * 1024 ? 2 : 1; }
-int fused_occ_dispatch(int d, int Q, int kernel_kind) {
-  PGM_DISPATCH(fused_blocks_per_sm);
-  return 1;
+// the arrays of an _f32 entry point: inputs, and the outputs it returns (null: none)
+struct Io32 {
+  const float *x, *y, *fixed_noise, *raw, *con_lb, *con_ub;
+  float *mll, *grad, *raw_out, *loss, *hist;
+};
+
+// An _f32 entry point on an fp64 one (fp32 storage, fp64 arithmetic), for a call its caller has
+// validated up to the workspace size.  The fp64 entry's workspace (f64_bytes, rounded up to 256)
+// comes first, the staging area (pgm_f32_staging_bytes) behind it.  The inputs are widened into
+// the staging area, f64(staged, rounded f64_bytes) runs the fp64 entry on them, and the outputs
+// are narrowed back.
+template <typename F64>
+int stage_f32(const Io32& io, int B, int n_max, int d, int Q, int kernel_kind, int flags,
+              int maxiter, size_t f64_bytes, const char* f64_ws, void* workspace,
+              size_t workspace_bytes, void* stream, F64 f64) {
+  const size_t base = align256(f64_bytes);
+  if (workspace_bytes < base + pgm_f32_staging_bytes(B, n_max, d, Q, kernel_kind, flags, maxiter,
+                                                     io.hist != nullptr))
+    return fail(std::string("workspace too small (") + f64_ws +
+                " rounded up to 256 + pgm_f32_staging_bytes)");
+  const int P = host_param_count(d, Q, kernel_kind, flags);
+  const bool per_lc = (flags & PGM_FLAG_BOUNDS_PER_LC) != 0;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  Stage32 s = carve32(static_cast<char*>(workspace) + base, B, n_max, d, P, per_lc, maxiter,
+                      io.hist != nullptr);
+  const size_t Bn = (size_t)B * n_max, BP = (size_t)B * P, nb = per_lc ? BP : (size_t)P;
+  widen(io.x, s.x, Bn * d, st); widen(io.y, s.y, Bn, st); widen(io.fixed_noise, s.fn, Bn, st);
+  widen(io.raw, s.raw, BP, st); widen(io.con_lb, s.lb, nb, st); widen(io.con_ub, s.ub, nb, st);
+  if (!io.fixed_noise) s.fn = nullptr;
+  if (!io.grad) s.grad = nullptr;
+  if (!io.hist) s.hist = nullptr;
+  if (int r = f64(s, base)) return r;
+  narrow(s.mll, io.mll, (size_t)B, st); narrow(s.grad, io.grad, BP, st);
+  narrow(s.raw, io.raw_out, BP, st); narrow(s.loss, io.loss, (size_t)maxiter * B, st);
+  narrow(s.hist, io.hist, (size_t)(maxiter + 1) * BP, st);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail("f32 staging", e);
+  return 0;
 }
 
 }  // namespace
@@ -246,33 +281,22 @@ int pgm_sm_mll_grad_alpha_f64(const double* x, const int32_t* n_valid, const dou
                               int B, int n_max, int d, int Q, int kernel_kind, int flags,
                               double* mll, double* grad_raw, double* alpha_out, int32_t* info,
                               void* workspace, size_t workspace_bytes, void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  const Config* cfg = check_common(B, n_max, d, Q, kernel_kind);
+  if (!cfg) return -1;
   if (alpha_out && !(flags & PGM_FLAG_GRAD)) return fail("alpha_out needs PGM_FLAG_GRAD");
   if (B == 0) return 0;
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !mll || !info || !workspace)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, mll, info, workspace})) return r;
   if ((flags & PGM_FLAG_GRAD) && !grad_raw) return fail("PGM_FLAG_GRAD needs grad_raw");
-  const size_t per_block = pgm::scratch_elems(n_max, nf_for(d, Q));
-  if (workspace_bytes < pgm_workspace_bytes(8, n_max, d, Q, -1))
-    return fail("workspace too small (see pgm_workspace_bytes)");
-  pgm::EvalArgs A;
-  A.x = x; A.n_valid = n_valid; A.y = y; A.fixed_noise = fixed_noise; A.raw = raw;
-  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
-  A.B = B; A.n_max = n_max; A.Q = Q; A.flags = flags;
-  A.mll = mll; A.grad = grad_raw; A.info = info;
-  A.ws = static_cast<double*>(workspace); A.ws_per_block = per_block;
-  A.alpha_out = alpha_out;
-  A.sched = reinterpret_cast<int*>(static_cast<char*>(workspace) + pgm_workspace_bytes(8, n_max, d, Q, -1)
-                                   - pgm::PGM_SCHED_INTS * sizeof(int));
-  A.sms = 0;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PGM_DISPATCH(launch_eval, A, st);
-  return 0;
+  auto A = model_args<pgm::EvalArgs>(x, n_valid, y, fixed_noise, raw, con_kind, con_lb, con_ub,
+                                     B, n_max, Q, flags, info, workspace);
+  A.mll = mll; A.grad = grad_raw; A.alpha_out = alpha_out;
+  if (int r = fused_ws(A, d, workspace_bytes)) return r;
+  return cfg->eval(A, static_cast<cudaStream_t>(stream));
 }
 
 int pgm_fused_grid(int d, int Q, int kernel_kind) {
-  if (check_common(1, 64, d, Q, kernel_kind)) return -1;
-  return pgm::device_sms() * fused_occ_dispatch(d, Q, kernel_kind);
+  const Config* cfg = check_common(1, 64, d, Q, kernel_kind);
+  return cfg ? pgm::device_sms() * cfg->fused_blocks_per_sm : -1;
 }
 
 size_t pgm_staged_workspace_bytes(int n_max, int B) {
@@ -299,26 +323,19 @@ int pgm_sm_mll_grad_staged_alpha_f64(const double* x, const int32_t* n_valid, co
                                      int kernel_kind, int flags, double* mll, double* grad_raw,
                                      double* alpha_out, int32_t* info, void* workspace,
                                      size_t workspace_bytes, void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  const Config* cfg = check_common(B, n_max, d, Q, kernel_kind);
+  if (!cfg) return -1;
   if (alpha_out && !(flags & PGM_FLAG_GRAD)) return fail("alpha_out needs PGM_FLAG_GRAD");
   if (B == 0) return 0;
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !mll || !info || !workspace)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, mll, info, workspace})) return r;
   if ((flags & PGM_FLAG_GRAD) && !grad_raw) return fail("PGM_FLAG_GRAD needs grad_raw");
   if (workspace_bytes < ((flags & PGM_FLAG_TF32X3) ? pgm_staged_tf32x3_workspace_bytes(n_max, B)
                                                    : pgm_staged_workspace_bytes(n_max, B)))
     return fail("workspace too small (see pgm_staged_workspace_bytes / pgm_staged_tf32x3_workspace_bytes)");
-  pgm::LargeArgs A;
-  A.x = x; A.n_valid = n_valid; A.y = y; A.fixed_noise = fixed_noise; A.raw = raw;
-  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
-  A.B = B; A.n_max = n_max; A.Q = Q; A.flags = flags;
-  A.mll = mll; A.grad = grad_raw; A.info = info;
-  A.ws = static_cast<double*>(workspace);
-  A.alpha_out = alpha_out;
-  const int want_grad = (flags & PGM_FLAG_GRAD) ? 1 : 0;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PGM_DISPATCH(launch_large, A, want_grad, st, 0);
-  return 0;
+  auto A = model_args<pgm::LargeArgs>(x, n_valid, y, fixed_noise, raw, con_kind, con_lb, con_ub,
+                                      B, n_max, Q, flags, info, workspace);
+  A.mll = mll; A.grad = grad_raw; A.alpha_out = alpha_out;
+  return cfg->large(A, (flags & PGM_FLAG_GRAD) ? 1 : 0, static_cast<cudaStream_t>(stream), 0);
 }
 
 size_t pgm_staged_tf32x3_workspace_bytes(int n_max, int B) {
@@ -344,36 +361,20 @@ int pgm_sm_mll_grad_tf32x3_f32(const float* x, const int32_t* n_valid, const flo
                                int B, int n_max, int d, int Q, int kernel_kind, int flags,
                                float* mll, float* grad_raw, int32_t* info, void* workspace,
                                size_t workspace_bytes, void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  if (!check_common(B, n_max, d, Q, kernel_kind)) return -1;
   if (B == 0) return 0;
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !mll || !info || !workspace)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, mll, info, workspace})) return r;
   if ((flags & PGM_FLAG_GRAD) && !grad_raw) return fail("PGM_FLAG_GRAD needs grad_raw");
-  const int P = host_param_count(d, Q, kernel_kind, flags);
-  const bool per_lc = (flags & PGM_FLAG_BOUNDS_PER_LC) != 0;
-  const size_t base = align256(pgm_staged_tf32x3_workspace_bytes(n_max, B));
-  const size_t need = base + pgm_f32_staging_bytes(B, n_max, d, Q, kernel_kind, flags, 0, 0);
-  if (workspace_bytes < need)
-    return fail("workspace too small (pgm_staged_tf32x3_workspace_bytes rounded up to 256 + "
-                "pgm_f32_staging_bytes)");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  Stage32 s = carve32(static_cast<char*>(workspace) + base, B, n_max, d, P, per_lc, 0, false);
-  const size_t Bn = (size_t)B * n_max, BP = (size_t)B * P;
-  widen(x, s.x, Bn * d, st); widen(y, s.y, Bn, st);
-  if (fixed_noise) widen(fixed_noise, s.fn, Bn, st);
-  widen(raw, s.raw, BP, st);
-  widen(con_lb, s.lb, per_lc ? BP : (size_t)P, st);
-  widen(con_ub, s.ub, per_lc ? BP : (size_t)P, st);
-  if (int r = pgm_sm_mll_grad_staged_alpha_f64(
-          s.x, n_valid, s.y, fixed_noise ? s.fn : nullptr, s.raw, con_kind, s.lb, s.ub, B, n_max, d,
-          Q, kernel_kind, flags | PGM_FLAG_JITTER_F32 | PGM_FLAG_TF32X3 | PGM_FLAG_TF32X3_CHOL, s.mll,
-          (flags & PGM_FLAG_GRAD) ? s.grad : nullptr, nullptr, info, workspace, base, stream))
-    return r;
-  narrow(s.mll, mll, (size_t)B, st);
-  if (flags & PGM_FLAG_GRAD) narrow(s.grad, grad_raw, BP, st);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail("f32 staging", e);
-  return 0;
+  const Io32 io{x, y, fixed_noise, raw, con_lb, con_ub, mll,
+                (flags & PGM_FLAG_GRAD) ? grad_raw : nullptr, nullptr, nullptr, nullptr};
+  return stage_f32(io, B, n_max, d, Q, kernel_kind, flags, 0,
+                   pgm_staged_tf32x3_workspace_bytes(n_max, B), "pgm_staged_tf32x3_workspace_bytes",
+                   workspace, workspace_bytes, stream, [&](const Stage32& s, size_t f64_bytes) {
+    return pgm_sm_mll_grad_staged_alpha_f64(
+        s.x, n_valid, s.y, s.fn, s.raw, con_kind, s.lb, s.ub, B, n_max, d, Q, kernel_kind,
+        flags | PGM_FLAG_JITTER_F32 | PGM_FLAG_TF32X3 | PGM_FLAG_TF32X3_CHOL, s.mll, s.grad,
+        nullptr, info, workspace, f64_bytes, stream);
+  });
 }
 
 size_t pgm_predict_workspace_bytes(int n_max, int B, int device) {
@@ -393,32 +394,25 @@ int pgm_sm_predict_f64(const double* x, const int32_t* n_valid, const double* y,
                        int kernel_kind, int flags, const double* xstar, int m, double* mean,
                        double* var, int32_t* info, void* workspace, size_t workspace_bytes,
                        void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  const Config* cfg = check_common(B, n_max, d, Q, kernel_kind);
+  if (!cfg) return -1;
   if (B == 0 || m == 0) return 0;
   if (m < 0) return fail("m must be >= 0");
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !xstar || !mean || !var || !info ||
-      !workspace)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, xstar, mean, var, info, workspace}))
+    return r;
   if (workspace_bytes < pgm_predict_workspace_bytes(n_max, B, -1))
     return fail("workspace too small (see pgm_predict_workspace_bytes)");
-  pgm::PredictArgs PA;
-  pgm::LargeArgs& A = PA.a;
-  A.x = x; A.n_valid = n_valid; A.y = y; A.fixed_noise = fixed_noise; A.raw = raw;
-  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
-  A.B = B; A.n_max = n_max; A.Q = Q; A.flags = flags & ~PGM_FLAG_GRAD;
-  A.mll = nullptr; A.grad = nullptr; A.info = info;
-  A.ws = static_cast<double*>(workspace);
-  A.alpha_out = nullptr;
+  pgm::PredictArgs PA{};
+  PA.a = model_args<pgm::LargeArgs>(x, n_valid, y, fixed_noise, raw, con_kind, con_lb, con_ub, B,
+                                    n_max, Q, flags & ~PGM_FLAG_GRAD, info, workspace);
   PA.xstar = xstar; PA.m = m; PA.mean = mean; PA.var = var;
-  const size_t staged = (pgm::large_ws_bytes(n_max, B) + 255) & ~(size_t)255;
-  PA.kscratch = reinterpret_cast<double*>(static_cast<char*>(workspace) + staged);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PGM_DISPATCH(launch_predict, PA, st);
-  return 0;
+  PA.kscratch = reinterpret_cast<double*>(static_cast<char*>(workspace) +
+                                          align256(pgm::large_ws_bytes(n_max, B)));
+  return cfg->predict(PA, static_cast<cudaStream_t>(stream));
 }
 
 size_t pgm_fisher_workspace_bytes(int n_max, int B, int d, int Q, int kernel_kind, int flags) {
-  if (n_max < 1 || B < 1 || check_common(B, n_max, d, Q, kernel_kind)) return 0;
+  if (n_max < 1 || B < 1 || !check_common(B, n_max, d, Q, kernel_kind)) return 0;
   return pgm::fisher_ws_bytes(n_max, B, host_param_count(d, Q, kernel_kind, flags) - 1);
 }
 
@@ -427,10 +421,10 @@ int pgm_sm_fisher_f64(const double* x, const int32_t* n_valid, const double* y,
                       const double* con_lb, const double* con_ub, int B, int n_max, int d, int Q,
                       int kernel_kind, int flags, double* fisher, int32_t* info, void* workspace,
                       size_t workspace_bytes, void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  const Config* cfg = check_common(B, n_max, d, Q, kernel_kind);
+  if (!cfg) return -1;
   if (B == 0) return 0;
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !fisher || !info || !workspace)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, fisher, info, workspace})) return r;
   if (B > 65535) return fail("pgm_sm_fisher_f64: B > 65535 (split the batch)");
   const int nc = host_param_count(d, Q, kernel_kind, flags) - 1;
   if (nc < 1 || nc > pgm::FS_NC_MAX) return fail("pgm_sm_fisher_f64: unsupported parameter count");
@@ -438,38 +432,27 @@ int pgm_sm_fisher_f64(const double* x, const int32_t* n_valid, const double* y,
   if (ntri * nc > 2147483647LL) return fail("pgm_sm_fisher_f64: n_max too large (tiles x carriers)");
   if (workspace_bytes < pgm_fisher_workspace_bytes(n_max, B, d, Q, kernel_kind, flags))
     return fail("workspace too small (see pgm_fisher_workspace_bytes)");
-  pgm::LargeArgs A;
-  A.x = x; A.n_valid = n_valid; A.y = y; A.fixed_noise = fixed_noise; A.raw = raw;
-  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
-  A.B = B; A.n_max = n_max; A.Q = Q;
-  A.flags = flags & (PGM_FLAG_LEARN_NOISE | PGM_FLAG_BOUNDS_PER_LC | PGM_FLAG_JITTER_F32);
-  A.mll = nullptr; A.grad = nullptr; A.info = info;
-  A.ws = static_cast<double*>(workspace);
-  A.alpha_out = nullptr;
+  const int fs_flags = flags & (PGM_FLAG_LEARN_NOISE | PGM_FLAG_BOUNDS_PER_LC | PGM_FLAG_JITTER_F32);
+  auto A = model_args<pgm::LargeArgs>(x, n_valid, y, fixed_noise, raw, con_kind, con_lb, con_ub,
+                                      B, n_max, Q, fs_flags, info, workspace);
   pgm::FisherArgs F;
   F.nc = nc;
   F.fisher = fisher;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PGM_DISPATCH(launch_fisher, A, F, st);
-  return 0;
+  return cfg->fisher(A, F, static_cast<cudaStream_t>(stream));
 }
 
 int pgm_sm_kernel_dense_f64(const double* x, const int32_t* n_valid, const double* fixed_noise,
                             const double* raw, const int32_t* con_kind, const double* con_lb,
                             const double* con_ub, int B, int n_max, int d, int Q,
                             int kernel_kind, int flags, double* K_out, void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  const Config* cfg = check_common(B, n_max, d, Q, kernel_kind);
+  if (!cfg) return -1;
   if (B == 0) return 0;
-  if (!x || !raw || !con_kind || !con_lb || !con_ub || !K_out) return fail("null pointer argument");
+  if (int r = check_ptrs({x, raw, con_kind, con_lb, con_ub, K_out})) return r;
   if (B > 65535) return fail("B > 65535 not supported by the dense builder");
-  pgm::EvalArgs A;
-  memset(&A, 0, sizeof(A));
-  A.x = x; A.n_valid = n_valid; A.fixed_noise = fixed_noise; A.raw = raw;
-  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
-  A.B = B; A.n_max = n_max; A.Q = Q; A.flags = flags;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PGM_DISPATCH(launch_dense, A, K_out, st);
-  return 0;
+  const auto A = model_args<pgm::EvalArgs>(x, n_valid, nullptr, fixed_noise, raw, con_kind,
+                                           con_lb, con_ub, B, n_max, Q, flags, nullptr, nullptr);
+  return cfg->dense(A, K_out, static_cast<cudaStream_t>(stream));
 }
 
 int pgm_optim_step_f64(double* raw, const double* grad_mll, double* exp_avg, double* exp_avg_sq,
@@ -478,7 +461,7 @@ int pgm_optim_step_f64(double* raw, const double* grad_mll, double* exp_avg, dou
                        void* stream) {
   if (B < 0 || P < 1) return fail("bad B / P");
   if (B == 0) return 0;
-  if (!raw || !grad_mll) return fail("null pointer argument");
+  if (int r = check_ptrs({raw, grad_mll})) return r;
   if (optim_kind != PGM_OPT_SGD && (!exp_avg || !exp_avg_sq))
     return fail("Adam / AdamW need exp_avg and exp_avg_sq");
   if (optim_kind < 0 || optim_kind > 2) return fail("unknown optim_kind");
@@ -506,35 +489,23 @@ int pgm_sm_fit_f64(const double* x, const int32_t* n_valid, const double* y,
                    int32_t* n_iter, int32_t* info, double* opt_state, void* workspace,
                    size_t workspace_bytes, void* stream) {
   (void)opt_state;  // optimiser state lives in shared memory for the whole loop
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  const Config* cfg = check_common(B, n_max, d, Q, kernel_kind);
+  if (!cfg) return -1;
   if (B == 0) return 0;
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !loss_hist || !n_iter || !info ||
-      !workspace)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, loss_hist, n_iter, info, workspace}))
+    return r;
   if (maxiter < 1) return fail("maxiter must be >= 1");
   if (optim_kind < 0 || optim_kind > 2) return fail("unknown optim_kind");
   if (stopavg < 1) stopavg = 1;
-  const size_t per_block = pgm::scratch_elems(n_max, nf_for(d, Q));
-  if (workspace_bytes < pgm_workspace_bytes(8, n_max, d, Q, -1))
-    return fail("workspace too small (see pgm_workspace_bytes)");
-  pgm::FitArgs F;
-  pgm::EvalArgs& A = F.e;
-  A.x = x; A.n_valid = n_valid; A.y = y; A.fixed_noise = fixed_noise; A.raw = raw;
-  A.con_kind = con_kind; A.con_lb = con_lb; A.con_ub = con_ub;
-  A.B = B; A.n_max = n_max; A.Q = Q; A.flags = flags | PGM_FLAG_GRAD;
-  A.mll = nullptr; A.grad = nullptr; A.info = info;
-  A.ws = static_cast<double*>(workspace); A.ws_per_block = per_block;
-  A.alpha_out = nullptr;
-  A.sched = reinterpret_cast<int*>(static_cast<char*>(workspace) + pgm_workspace_bytes(8, n_max, d, Q, -1)
-                                   - pgm::PGM_SCHED_INTS * sizeof(int));
-  A.sms = 0;
+  pgm::FitArgs F{};
+  F.e = model_args<pgm::EvalArgs>(x, n_valid, y, fixed_noise, raw, con_kind, con_lb, con_ub, B,
+                                  n_max, Q, flags | PGM_FLAG_GRAD, info, workspace);
+  if (int r = fused_ws(F.e, d, workspace_bytes)) return r;
   F.raw_io = raw; F.optim_kind = optim_kind; F.lr = lr; F.beta1 = beta1; F.beta2 = beta2;
   F.eps = eps; F.weight_decay = weight_decay; F.stop = stop; F.maxiter = maxiter;
   F.miniter = miniter; F.stopavg = stopavg; F.loss_hist = loss_hist; F.raw_hist = raw_hist;
   F.n_iter = n_iter;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PGM_DISPATCH(launch_fit, F, st);
-  return 0;
+  return cfg->fit(F, static_cast<cudaStream_t>(stream));
 }
 
 size_t pgm_f32_staging_bytes(int B, int n_max, int d, int Q, int kernel_kind, int flags,
@@ -550,36 +521,19 @@ int pgm_sm_mll_grad_f32(const float* x, const int32_t* n_valid, const float* y,
                         const float* con_lb, const float* con_ub, int B, int n_max, int d, int Q,
                         int kernel_kind, int flags, float* mll, float* grad_raw, int32_t* info,
                         void* workspace, size_t workspace_bytes, void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  if (!check_common(B, n_max, d, Q, kernel_kind)) return -1;
   if (B == 0) return 0;
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !mll || !info || !workspace)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, mll, info, workspace})) return r;
   if ((flags & PGM_FLAG_GRAD) && !grad_raw) return fail("PGM_FLAG_GRAD needs grad_raw");
-  const int P = host_param_count(d, Q, kernel_kind, flags);
-  const bool per_lc = (flags & PGM_FLAG_BOUNDS_PER_LC) != 0;
-  const size_t base = align256(pgm_workspace_bytes(8, n_max, d, Q, -1));
-  const size_t need = base + pgm_f32_staging_bytes(B, n_max, d, Q, kernel_kind, flags, 0, 0);
-  if (workspace_bytes < need)
-    return fail("workspace too small (pgm_workspace_bytes rounded up to 256 + pgm_f32_staging_bytes)");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  Stage32 s = carve32(static_cast<char*>(workspace) + base, B, n_max, d, P, per_lc, 0, false);
-  const size_t Bn = (size_t)B * n_max, BP = (size_t)B * P;
-  widen(x, s.x, Bn * d, st); widen(y, s.y, Bn, st);
-  if (fixed_noise) widen(fixed_noise, s.fn, Bn, st);
-  widen(raw, s.raw, BP, st);
-  widen(con_lb, s.lb, per_lc ? BP : (size_t)P, st);
-  widen(con_ub, s.ub, per_lc ? BP : (size_t)P, st);
-  if (int r = pgm_sm_mll_grad_f64(s.x, n_valid, s.y, fixed_noise ? s.fn : nullptr, s.raw, con_kind,
-                                  s.lb, s.ub, B, n_max, d, Q, kernel_kind,
-                                  flags | PGM_FLAG_JITTER_F32, s.mll,
-                                  (flags & PGM_FLAG_GRAD) ? s.grad : nullptr, info, workspace,
-                                  base, stream))
-    return r;
-  narrow(s.mll, mll, (size_t)B, st);
-  if (flags & PGM_FLAG_GRAD) narrow(s.grad, grad_raw, BP, st);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail("f32 staging", e);
-  return 0;
+  const Io32 io{x, y, fixed_noise, raw, con_lb, con_ub, mll,
+                (flags & PGM_FLAG_GRAD) ? grad_raw : nullptr, nullptr, nullptr, nullptr};
+  return stage_f32(io, B, n_max, d, Q, kernel_kind, flags, 0,
+                   pgm_workspace_bytes(8, n_max, d, Q, -1), "pgm_workspace_bytes", workspace,
+                   workspace_bytes, stream, [&](const Stage32& s, size_t f64_bytes) {
+    return pgm_sm_mll_grad_f64(s.x, n_valid, s.y, s.fn, s.raw, con_kind, s.lb, s.ub, B, n_max, d,
+                               Q, kernel_kind, flags | PGM_FLAG_JITTER_F32, s.mll, s.grad, info,
+                               workspace, f64_bytes, stream);
+  });
 }
 
 int pgm_sm_fit_f32(const float* x, const int32_t* n_valid, const float* y,
@@ -589,41 +543,21 @@ int pgm_sm_fit_f32(const float* x, const int32_t* n_valid, const float* y,
                    double beta2, double eps, double weight_decay, int maxiter, int miniter,
                    double stop, int stopavg, float* loss_hist, float* raw_hist, int32_t* n_iter,
                    int32_t* info, void* workspace, size_t workspace_bytes, void* stream) {
-  if (int r = check_common(B, n_max, d, Q, kernel_kind)) return r;
+  if (!check_common(B, n_max, d, Q, kernel_kind)) return -1;
   if (B == 0) return 0;
-  if (!x || !y || !raw || !con_kind || !con_lb || !con_ub || !loss_hist || !n_iter || !info ||
-      !workspace)
-    return fail("null pointer argument");
-  if (maxiter < 1) return fail("maxiter must be >= 1");
-  const int P = host_param_count(d, Q, kernel_kind, flags);
-  const bool per_lc = (flags & PGM_FLAG_BOUNDS_PER_LC) != 0;
-  const size_t base = align256(pgm_workspace_bytes(8, n_max, d, Q, -1));
-  const size_t need = base + pgm_f32_staging_bytes(B, n_max, d, Q, kernel_kind, flags, maxiter,
-                                                   raw_hist != nullptr);
-  if (workspace_bytes < need)
-    return fail("workspace too small (pgm_workspace_bytes rounded up to 256 + pgm_f32_staging_bytes)");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  Stage32 s = carve32(static_cast<char*>(workspace) + base, B, n_max, d, P, per_lc, maxiter,
-                      raw_hist != nullptr);
-  const size_t Bn = (size_t)B * n_max, BP = (size_t)B * P;
-  widen(x, s.x, Bn * d, st); widen(y, s.y, Bn, st);
-  if (fixed_noise) widen(fixed_noise, s.fn, Bn, st);
-  widen(raw, s.raw, BP, st);
-  widen(con_lb, s.lb, per_lc ? BP : (size_t)P, st);
-  widen(con_ub, s.ub, per_lc ? BP : (size_t)P, st);
-  if (int r = pgm_sm_fit_f64(s.x, n_valid, s.y, fixed_noise ? s.fn : nullptr, s.raw, con_kind, s.lb,
-                             s.ub, B, n_max, d, Q, kernel_kind, flags | PGM_FLAG_JITTER_F32,
-                             optim_kind, lr, beta1, beta2,
-                             eps, weight_decay, maxiter, miniter, stop, stopavg, s.loss,
-                             raw_hist ? s.hist : nullptr, n_iter, info, nullptr, workspace, base,
-                             stream))
+  if (int r = check_ptrs({x, y, raw, con_kind, con_lb, con_ub, loss_hist, n_iter, info, workspace}))
     return r;
-  narrow(s.raw, raw, BP, st);
-  narrow(s.loss, loss_hist, (size_t)maxiter * B, st);
-  if (raw_hist) narrow(s.hist, raw_hist, (size_t)(maxiter + 1) * BP, st);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail("f32 staging", e);
-  return 0;
+  if (maxiter < 1) return fail("maxiter must be >= 1");
+  const Io32 io{x, y, fixed_noise, raw, con_lb, con_ub, nullptr, nullptr, raw, loss_hist,
+                raw_hist};
+  return stage_f32(io, B, n_max, d, Q, kernel_kind, flags, maxiter,
+                   pgm_workspace_bytes(8, n_max, d, Q, -1), "pgm_workspace_bytes", workspace,
+                   workspace_bytes, stream, [&](const Stage32& s, size_t f64_bytes) {
+    return pgm_sm_fit_f64(s.x, n_valid, s.y, s.fn, s.raw, con_kind, s.lb, s.ub, B, n_max, d, Q,
+                          kernel_kind, flags | PGM_FLAG_JITTER_F32, optim_kind, lr, beta1, beta2,
+                          eps, weight_decay, maxiter, miniter, stop, stopavg, s.loss, s.hist,
+                          n_iter, info, nullptr, workspace, f64_bytes, stream);
+  });
 }
 
 int pgm_lombscargle_f64(const double* t, const int32_t* n_valid, const double* y, const double* dy,
@@ -632,7 +566,7 @@ int pgm_lombscargle_f64(const double* t, const int32_t* n_valid, const double* y
   if (B < 0 || n_max < 1 || nf_max < 1) return fail("B >= 0, n_max >= 1, nf_max >= 1 required");
   if (B == 0) return 0;
   if (B > 65535) return fail("B > 65535 (split the batch)");
-  if (!t || !y || !f0 || !df || !nf || !power) return fail("null pointer argument");
+  if (int r = check_ptrs({t, y, f0, df, nf, power})) return r;
   pgm::LsArgs A;
   A.t = t; A.n_valid = n_valid; A.y = y; A.dy = dy; A.f0 = f0; A.df = df; A.nf = nf;
   A.B = B; A.n_max = n_max; A.nf_max = nf_max; A.flags = flags; A.power = power;
@@ -649,7 +583,7 @@ int pgm_ls_peaks_f64(const double* power, const int32_t* nf, int B, int nf_max, 
   if (B < 0 || nf_max < 1 || num_peaks < 1) return fail("bad B / nf_max / num_peaks");
   if (B == 0) return 0;
   if (distance < 1) return fail("distance must be >= 1 (scipy.signal.find_peaks)");
-  if (!power || !nf || !peak_idx || !peak_power || !scratch) return fail("null pointer argument");
+  if (int r = check_ptrs({power, nf, peak_idx, peak_power, scratch})) return r;
   if (scratch_bytes < (size_t)B * nf_max) return fail("scratch too small (B * nf_max bytes)");
   pgm::LsPeakArgs A;
   A.power = power; A.nf = nf; A.B = B; A.nf_max = nf_max; A.distance = distance;
@@ -667,9 +601,9 @@ int pgm_sm_psd_peak_f64(const double* freq, const double* fscale, const double* 
                         double* dom_height, int32_t* n_peaks, void* stream) {
   if (B < 0 || Q < 1 || Q > 8 || n_grid < 3) return fail("bad B / Q (1..8) / n_grid (>= 3)");
   if (B == 0) return 0;
-  if (!freq || !fscale || !weight || !fmin || !fmax || !psd || !dom_idx || !dom_freq ||
-      !dom_height || !n_peaks)
-    return fail("null pointer argument");
+  if (int r = check_ptrs({freq, fscale, weight, fmin, fmax, psd, dom_idx, dom_freq, dom_height,
+                          n_peaks}))
+    return r;
   pgm::PsdArgs A;
   A.freq = freq; A.fscale = fscale; A.weight = weight; A.fmin = fmin; A.fmax = fmax;
   A.B = B; A.Q = Q; A.n_grid = n_grid; A.grid = grid; A.psd = psd; A.dom_idx = dom_idx;

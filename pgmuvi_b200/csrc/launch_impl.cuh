@@ -93,14 +93,19 @@ int launch_large(const pgm::LargeArgs& A, int want_grad, cudaStream_t st, int pr
   e = cudaFuncSetAttribute(k_upd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UPD_SMEM);
   if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute(lg_update)", e);
   constexpr size_t CHOL_SMEM = CholAllSmem<KIND, QT, D>::BYTES;
-  cudaFuncSetAttribute(k_chol, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CHOL_SMEM);
+  e = cudaFuncSetAttribute(k_chol, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CHOL_SMEM);
+  if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute(lg_chol_all)", e);
   constexpr size_t GRAD_SMEM = GradSmem<KIND, QT, D>::BYTES;
   e = cudaFuncSetAttribute(k_grad, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GRAD_SMEM);
   if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute(lg_grad)", e);
-  cudaFuncSetAttribute(lg_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_DIAG_SMEM);
-  cudaFuncSetAttribute(lg_trsm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_TRSM_SMEM);
-  cudaFuncSetAttribute(lg_inv_row, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_INV_SMEM);
-  cudaFuncSetAttribute(lg_inv_all, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_INV_SMEM);
+  e = cudaFuncSetAttribute(lg_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_DIAG_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(lg_trsm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_TRSM_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(lg_inv_row, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_INV_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(lg_inv_all, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_INV_SMEM);
+  if (e != cudaSuccess) return cuda_fail("cudaFuncSetAttribute(staged engine kernels)", e);
   BatchState bs = make_batch_state(A.ws, n, B);
   cudaMemsetAsync(bs.state, 0, (size_t)(4 * B + 4) * sizeof(int), st);
   const dim3 blk(NTHREADS);

@@ -12,20 +12,11 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import (FLAG_BOUNDS_PER_LC, FLAG_GRAD, FLAG_LEARN_NOISE, KIND_SM1D,
-                   KIND_SM_ARD_PRODSUM, KIND_SM_ARD_SUMPROD, KIND_STAT_BASE, NUM_LAM, SEP_KINDS,
-                   check, is_stat, ptr, stat_num_lam)
+                   KIND_SM_ARD_PRODSUM, KIND_SM_ARD_SUMPROD, KIND_STAT_BASE, check, is_stat,
+                   param_count, ptr)
 
 _workspaces = {}
 _staged_ws = {}
-
-
-def param_count(Q: int, d: int, learn_noise: bool, kind: int = -1) -> int:
-    """P of the packed layout ``[mean | w | mu | sigma | (noise) | lam]`` (pgmuvi_b200.h)."""
-    if is_stat(kind):            # stationary time kernels: no mixtures (Q = 0)
-        return 1 + (1 if learn_noise else 0) + stat_num_lam(kind)
-    if kind in SEP_KINDS:
-        return 1 + 3 * Q + (1 if learn_noise else 0) + NUM_LAM[kind]
-    return 1 + Q + 2 * Q * d + (1 if learn_noise else 0)
 
 
 def _require_cuda(*ts):
@@ -34,18 +25,30 @@ def _require_cuda(*ts):
             raise RuntimeError("pgmuvi_b200 ops need CUDA tensors (there is no CPU fallback)")
 
 
+def _cached_ws(cache, device, need):
+    """A workspace of at least `need` bytes, kept per device and grown on demand."""
+    ws = cache.get(device.index)
+    if ws is None or ws.numel() < need:
+        cache.pop(device.index, None)   # free the old one before the larger allocation
+        ws = None
+        ws = torch.empty(need, dtype=torch.uint8, device=device)
+        cache[device.index] = ws
+    return ws
+
+
+def _device_index(device):
+    return device.index if device.index is not None else torch.cuda.current_device()
+
+
 def _workspace(device, n_max, d, Q, extra=0):
-    lib = _lib.load()
-    need = lib.pgm_workspace_bytes(8, n_max, d, Q, device.index if device.index is not None
-                                   else torch.cuda.current_device())
+    need = _lib.load().pgm_workspace_bytes(8, n_max, d, Q, _device_index(device))
     if extra:   # fp32 entry points: fp64 staging area behind the (256-aligned) base workspace
         need = ((need + 255) & ~255) + extra
-    key = (device.index, )
-    ws = _workspaces.get(key)
-    if ws is None or ws.numel() < need:
-        ws = torch.empty(need, dtype=torch.uint8, device=device)
-        _workspaces[key] = ws
-    return ws, need
+    return _cached_ws(_workspaces, device, need)
+
+
+def _n_valid(n_valid):
+    return None if n_valid is None else n_valid.to(torch.int32).contiguous()
 
 
 def _stream():
@@ -91,17 +94,16 @@ def sm_mll_grad(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor
     """Per-datum exact MLL, d MLL / d raw and Cholesky info for B light curves."""
     (x, y, fixed_noise, raw, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
         x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    n_valid = _n_valid(n_valid)
     if want_grad:
         flags |= FLAG_GRAD
     mll = torch.empty(B, dtype=x.dtype, device=x.device)
     grad = torch.zeros(B, P, dtype=x.dtype, device=x.device)
     info = torch.zeros(B, dtype=torch.int32, device=x.device)
-    if n_valid is not None:
-        n_valid = n_valid.to(torch.int32).contiguous()
     lib = _lib.load()
     f32 = x.dtype == torch.float32
     extra = lib.pgm_f32_staging_bytes(B, n, d, Q, kind, flags, 0, 0) if f32 else 0
-    ws, nbytes = _workspace(x.device, n, d, Q, extra)
+    ws = _workspace(x.device, n, d, Q, extra)
     entry = lib.pgm_sm_mll_grad_f32 if f32 else lib.pgm_sm_mll_grad_f64
     with torch.cuda.device(x.device):
         check(entry(
@@ -128,6 +130,7 @@ def sm_mll_grad_alpha(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: 
     mean functions).  ``staged`` selects the whole-device engine (long light curves)."""
     (x, y, fixed_noise, raw, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
         x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    n_valid = _n_valid(n_valid)
     if x.dtype != torch.float64:
         raise RuntimeError("sm_mll_grad_alpha takes float64 tensors")
     flags |= FLAG_GRAD
@@ -135,21 +138,12 @@ def sm_mll_grad_alpha(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: 
     grad = torch.zeros(B, P, dtype=x.dtype, device=x.device)
     alpha = torch.zeros(B, n, dtype=x.dtype, device=x.device)
     info = torch.zeros(B, dtype=torch.int32, device=x.device)
-    if n_valid is not None:
-        n_valid = n_valid.to(torch.int32).contiguous()
     lib = _lib.load()
     if staged:
-        need = lib.pgm_staged_workspace_bytes(n, B)
-        key = (x.device.index,)
-        ws = _staged_ws.get(key)
-        if ws is None or ws.numel() < need:
-            _staged_ws.pop(key, None)
-            ws = None
-            ws = torch.empty(need, dtype=torch.uint8, device=x.device)
-            _staged_ws[key] = ws
+        ws = _cached_ws(_staged_ws, x.device, lib.pgm_staged_workspace_bytes(n, B))
         entry = lib.pgm_sm_mll_grad_staged_alpha_f64
     else:
-        ws, _ = _workspace(x.device, n, d, Q)
+        ws = _workspace(x.device, n, d, Q)
         entry = lib.pgm_sm_mll_grad_alpha_f64
     with torch.cuda.device(x.device):
         check(entry(ptr(x), ptr(n_valid), ptr(y), ptr(fixed_noise), ptr(raw), ptr(con_kind),
@@ -174,11 +168,10 @@ def sm_kernel_dense(x: Tensor, fixed_noise: Optional[Tensor], raw: Tensor, con_k
     y = x.new_empty(B, n)
     (x, _, fixed_noise, raw, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
         x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    n_valid = _n_valid(n_valid)
     if x.dtype != torch.float64:
         raise RuntimeError("sm_kernel_dense takes float64 tensors")
     K = torch.zeros(B, n, n, dtype=x.dtype, device=x.device)
-    if n_valid is not None:
-        n_valid = n_valid.to(torch.int32).contiguous()
     with torch.cuda.device(x.device):
         check(_lib.load().pgm_sm_kernel_dense_f64(
             ptr(x), ptr(n_valid), ptr(fixed_noise), ptr(raw), ptr(con_kind), ptr(con_lb),
@@ -224,6 +217,7 @@ def sm_fit(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor, con
     raw_hist [maxiter+1,B,P] or empty, n_iter [B], info [B]); ``raw`` is updated in place."""
     (x, y, fixed_noise, raw_c, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
         x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    n_valid = _n_valid(n_valid)
     if not raw.is_contiguous():
         raise RuntimeError("raw must be contiguous (updated in place)")
     loss_hist = torch.empty(maxiter, B, dtype=x.dtype, device=x.device)
@@ -231,12 +225,10 @@ def sm_fit(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor, con
                            device=x.device)
     n_iter = torch.zeros(B, dtype=torch.int32, device=x.device)
     info = torch.zeros(B, dtype=torch.int32, device=x.device)
-    if n_valid is not None:
-        n_valid = n_valid.to(torch.int32).contiguous()
     lib = _lib.load()
     if x.dtype == torch.float32:
         extra = lib.pgm_f32_staging_bytes(B, n, d, Q, kind, flags, maxiter, int(keep_history))
-        ws, _ = _workspace(x.device, n, d, Q, extra)
+        ws = _workspace(x.device, n, d, Q, extra)
         with torch.cuda.device(x.device):
             check(lib.pgm_sm_fit_f32(
                 ptr(x), ptr(n_valid), ptr(y), ptr(fixed_noise), ptr(raw), ptr(con_kind),
@@ -245,7 +237,7 @@ def sm_fit(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor, con
                 ptr(raw_hist) if keep_history else None, ptr(n_iter), ptr(info), ptr(ws),
                 ws.numel(), _stream()))
         return loss_hist, raw_hist, n_iter, info
-    ws, _ = _workspace(x.device, n, d, Q)
+    ws = _workspace(x.device, n, d, Q)
     with torch.cuda.device(x.device):
         check(lib.pgm_sm_fit_f64(
             ptr(x), ptr(n_valid), ptr(y), ptr(fixed_noise), ptr(raw), ptr(con_kind), ptr(con_lb),
@@ -283,6 +275,7 @@ def sm_mll_grad_staged(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw:
     batches): ``info`` is final once the stream has drained."""
     (x, y, fixed_noise, raw, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
         x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    n_valid = _n_valid(n_valid)
     f32 = x.dtype == torch.float32
     if f32 and not tf32x3:
         raise RuntimeError("the staged engine takes float64 tensors (float32: tf32x3=True)")
@@ -301,18 +294,10 @@ def sm_mll_grad_staged(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw:
             need = ((need + 255) & ~255) + lib.pgm_f32_staging_bytes(B, n, d, Q, kind, flags, 0, 0)
     else:
         need = lib.pgm_staged_workspace_bytes(n, B)
-    key = (x.device.index,)
-    ws = _staged_ws.get(key)
-    if ws is None or ws.numel() < need:
-        _staged_ws.pop(key, None)
-        ws = None
-        ws = torch.empty(need, dtype=torch.uint8, device=x.device)
-        _staged_ws[key] = ws
+    ws = _cached_ws(_staged_ws, x.device, need)
     mll = torch.empty(B, dtype=x.dtype, device=x.device)
     grad = torch.zeros(B, P, dtype=x.dtype, device=x.device)
     info = torch.zeros(B, dtype=torch.int32, device=x.device)
-    if n_valid is not None:
-        n_valid = n_valid.to(torch.int32).contiguous()
     entry = (lib.pgm_sm_mll_grad_tf32x3_f32 if f32 else lib.pgm_sm_mll_grad_staged_tf32x3_f64
              if tf32x3 else lib.pgm_sm_mll_grad_staged_f64)
     with torch.cuda.device(x.device):
@@ -331,6 +316,7 @@ def sm_predict(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor,
     (``pgm_sm_predict_f64``).  Returns (mean [B, m], var [B, m], info [B]); blocking."""
     (x, y, fixed_noise, raw, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
         x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    n_valid = _n_valid(n_valid)
     _require_cuda(xstar)
     if xstar.dim() == 2:
         xstar = xstar.unsqueeze(-1)
@@ -339,20 +325,11 @@ def sm_predict(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor,
     xstar = xstar.contiguous()
     m = xstar.shape[1]
     lib = _lib.load()
-    need = lib.pgm_predict_workspace_bytes(n, B, x.device.index if x.device.index is not None
-                                           else torch.cuda.current_device())
-    key = (x.device.index,)
-    ws = _staged_ws.get(key)
-    if ws is None or ws.numel() < need:
-        _staged_ws.pop(key, None)
-        ws = None
-        ws = torch.empty(need, dtype=torch.uint8, device=x.device)
-        _staged_ws[key] = ws
+    ws = _cached_ws(_staged_ws, x.device,
+                    lib.pgm_predict_workspace_bytes(n, B, _device_index(x.device)))
     mean = torch.empty(B, m, dtype=x.dtype, device=x.device)
     var = torch.empty(B, m, dtype=x.dtype, device=x.device)
     info = torch.zeros(B, dtype=torch.int32, device=x.device)
-    if n_valid is not None:
-        n_valid = n_valid.to(torch.int32).contiguous()
     with torch.cuda.device(x.device):
         check(lib.pgm_sm_predict_f64(
             ptr(x), ptr(n_valid), ptr(y), ptr(fixed_noise), ptr(raw), ptr(con_kind), ptr(con_lb),
@@ -387,12 +364,11 @@ def sm_fisher(x: Tensor, y: Tensor, fixed_noise: Optional[Tensor], raw: Tensor, 
     ``info < 0`` are NaN.  float64 only; blocking."""
     (x, y, fixed_noise, raw, con_kind, con_lb, con_ub, B, n, d, P, flags) = _prep(
         x, y, fixed_noise, raw, con_kind, con_lb, con_ub, kind, Q, learn_noise)
+    n_valid = _n_valid(n_valid)
     if x.dtype != torch.float64:
         raise RuntimeError("sm_fisher takes float64 tensors")
     fisher = torch.empty(B, P, P, dtype=x.dtype, device=x.device)
     info = torch.zeros(B, dtype=torch.int32, device=x.device)
-    if n_valid is not None:
-        n_valid = n_valid.to(torch.int32).contiguous()
     lib = _lib.load()
     # not cached between calls: a batch's workspace can take most of the device memory
     ws = torch.empty(lib.pgm_fisher_workspace_bytes(n, B, d, Q, kind, flags), dtype=torch.uint8,

@@ -14,6 +14,8 @@ import math
 
 import numpy as np
 
+from ._lib import KIND_STAT_BASE, NUM_LAM, param_count, stat_num_lam
+
 # constraint kinds - must match include/pgmuvi_b200.h
 CON_NONE, CON_SOFTPLUS, CON_INTERVAL = 0, 1, 2
 
@@ -33,16 +35,6 @@ def fixed_noise_variance(yerr):
     (lightcurve.py:2780-2784), clamped to GPyTorch's fp64 ``min_fixed_noise`` 1e-6."""
     v = (np.asarray(yerr, dtype=np.float32) ** 2).astype(np.float64)
     return np.maximum(v, 1e-6)
-
-
-NUM_LAM = {3: 2, 4: 2, 5: 3, 6: 1}   # wavelength-kernel parameters of the separable kinds
-
-
-def param_count(Q, d, learn_noise, kind=None):
-    """P of the packed layout (include/pgmuvi_b200.h); ``kind`` >= 3: separable models."""
-    if kind is not None and kind >= 3:
-        return 1 + Q + 2 * Q + (1 if learn_noise else 0) + NUM_LAM[kind]
-    return 1 + Q + 2 * Q * d + (1 if learn_noise else 0)
 
 
 def default_constraints(x, y, yerr, Q, d, learn_noise):
@@ -265,11 +257,10 @@ def make_batch_stat(B, kind, n=None, n_bands=None, n_per_band=None, learn_noise=
     wavelength kernel; pgmuvi/gps.py:985-990, 1131-1184, 1316-1319) on the 1-D / 2-D synthetic
     light curves.  kind = 8 + 5 * TK + WK, Q = 0; packed [mean | (noise) | os_t, l_t | wavelength
     parameters]; GPyTorch's default Positive constraints, mean / learned noise Interval."""
-    from ._lib import KIND_STAT_BASE, stat_num_lam
     tk, wk = divmod(kind - KIND_STAT_BASE, 5)
     d = 1 if wk == 0 else 2
     NL = stat_num_lam(kind)
-    P = 1 + (1 if learn_noise else 0) + NL
+    P = param_count(0, d, learn_noise, kind)
     o_noise = 1
     o_lam = 1 + (1 if learn_noise else 0)
     npts = n if d == 1 else n_bands * n_per_band

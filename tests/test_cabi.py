@@ -63,6 +63,33 @@ def test_bad_arguments_are_rejected_before_any_launch():
                                    0, 0, None, None, None, None, 0, None) == 0
 
 
+def test_model_validation_matches_the_compiled_configurations():
+    """A (kind, d, Q) model is accepted exactly when build.CONFIGS has a row of its kind and d with
+    QT >= max(Q, 1) (stationary kinds take Q == 0, the others 1 <= Q <= 8); no launch happens here
+    (workspace_bytes = 0)."""
+    from pgmuvi_b200.build import CONFIGS
+    rejections = (b"stationary kinds have no mixtures", b"time kernels 3..5", b"stationary kind / d",
+                  b"Q (num_mixtures)", b"d == 1", b"d == 2", b"unknown kernel_kind")
+    lib = _lib.load()
+    one = 8
+    for kind in range(-1, 41):
+        for d in range(0, 4):
+            for Q in range(-1, 10):
+                q_ok = Q == 0 if _lib.is_stat(kind) else 1 <= Q <= 8
+                accepted = q_ok and any(c[0] == kind and c[2] == d and c[1] >= max(Q, 1)
+                                        for c in CONFIGS)
+                rc = lib.pgm_sm_mll_grad_f64(one, None, one, None, one, one, one, one, 1, 64, d, Q,
+                                             kind, 0, one, None, one, one, 0, None)
+                err = lib.pgm_last_error()
+                case = (kind, d, Q, err)
+                assert rc == -1, case
+                if accepted:
+                    assert b"workspace" in err, case
+                else:
+                    assert any(r in err for r in rejections), case
+                assert (lib.pgm_fisher_workspace_bytes(64, 1, d, Q, kind, 0) == 0) != accepted, case
+
+
 def test_workspace_is_per_block_not_per_lightcurve():
     lib = _lib.load()
     w512 = lib.pgm_workspace_bytes(8, 512, 1, 4, -1)
